@@ -4,6 +4,7 @@
 Contract (one JSON line on stdout, printed by rank 0):
   python bench.py --gpus N --steps K --warmup W [--impl reference]
                   [--workload c5|c2w|c1|c2|c3|c4] [--format csr|hll] [--kernel ID] [--wpb W]
+                  [--dump-outputs DIR]
 
   metric   GFLOP/s = 2*nnz / t  (BASELINE.json), with achieved HBM GB/s on the
            minimum-traffic byte count B_min = 12 nnz + 4 (M+1) + 8 M + 8 N.
@@ -13,20 +14,29 @@ Contract (one JSON line on stdout, printed by rank 0):
            STRONG scaling.  --workload c2w is round 1's weak-scaling proxy (one 128^3 slab per
            GPU); c1..c4 time one single-GPU config (N = 1 only).
   step     one SpMV pass over the whole (distributed) matrix.
-  value    whole-job GFLOP/s with inputs resident in HBM: median of --regions (5) timed regions
-           of exactly K steps each, every region bracketed by barrier + synchronize on both
+  value    whole-job GFLOP/s with inputs resident in HBM over exactly K timed steps, cut into
+           --regions (1) regions, every region bracketed by barrier + synchronize on both
            sides, timed with CUDA events on the stepping stream, max over ranks.
+  outputs  --dump-outputs DIR: y of the last timed step as DIR/y.npy, float64, at most 2^21 rows
+           (dump_rows()).  c5/c2w: the iterate after the last region, x_{w+k} = A^(w+k) x_0 with
+           w = config.warmup_steps_per_region and k = region_steps[-1], gathered over ranks.
+           --impl reference: y of the headline variant's last pass.
+           Inputs are generated from fixed seeds, so equal arguments give equal inputs.
   e2e      same metric through the host-buffer C ABI call (spmv_b200_csr_spmv_host): HOST x
            slice in, HOST y slice out, copies inside the timed region.  Headline = PAGEABLE
            caller buffers (what the reference's compute_benchmark_csr hands over); "pinned" =
            page-locked buffers as a sub-key.
   configs  (N = 1 default run) one sub-record per single-GPU BASELINE config -- C1 (L2-flushed),
            C2, C3, C4 -- with GFLOP/s, roofline fraction, parity against the oracle and the
-           reference's CPU paths on that very matrix.
+           reference's CPU paths on that very matrix; each times K steps per format.
   roofline dominant kernel: B_min / mean CUDA-event launch time vs the measured
            HBM copy bandwidth in MEASURED_PEAKS.json.
-  cpu_baseline / --impl reference: the reference's own CPU code (oracle/_ref,
-           compiled from /root/reference/src) on this box's host cores.
+  cpu_baseline / --impl reference: the reference's own CPU code (oracle/_ref, compiled from
+           the original project's src/) on the machine's host cores.  --impl reference times
+           exactly K passes of every variant and reports the median pass.
+  side legs  K does not govern these; each reports its own count: the e2e legs (min(K, 20)
+           calls, at least 3), the stand-alone kernel of c5/c2w before and after the run (20
+           reps, 8 above 10^9 entries) and the cpu_baseline sub-records of the B200 line.
 """
 import argparse
 import json
@@ -75,6 +85,24 @@ def ncu_traffic(workload, kernel_symbol):
 
 def roofline_bytes(n_rows, n_cols, nnz):
     return 12 * nnz + 4 * (n_rows + 1) + 8 * n_rows + 8 * n_cols
+
+
+DUMP_MAX_ROWS = 1 << 21     # 16 MB of float64 per dumped vector
+
+
+def dump_rows(n):
+    """Rows of an n-row result that --dump-outputs writes: all of them up to DUMP_MAX_ROWS, else the
+    same seeded sample in every run and every build, in ascending order."""
+    if n <= DUMP_MAX_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ROWS, replace=False))
+
+
+def dump_outputs(directory, arrays):
+    """arrays: name -> float64 vector; written as <directory>/<name>.npy."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 DESCR = {
@@ -159,9 +187,11 @@ class ClockSampler:
 
 
 # ---------------------------------------------------------- reference (CPU) --
-def cpu_reference_run(O, A_arrays, x, steps, warmup, threads=None, hll=True):
+def cpu_reference_run(O, A_arrays, x, steps, warmup, threads=None, hll=True, serial_steps=None, ys=None):
     """Times the reference's own CPU CSR SpMV on this box.  Returns the best variant (GFLOP/s) and
-    every variant measured.  oracle/_ref when present ("reference"), else the oracle port ("port")."""
+    every variant measured.  oracle/_ref when present ("reference"), else the oracle port ("port").
+    Every OpenMP variant times `steps` passes, the serial one `serial_steps` (default min(steps, 2));
+    each variant reports its count as "steps".  ys: a dict that receives each variant's last y."""
     M, N, IRP, JA, AS = A_arrays
     nnz = len(JA)
     nthreads = threads or O.max_threads()
@@ -172,9 +202,9 @@ def cpu_reference_run(O, A_arrays, x, steps, warmup, threads=None, hll=True):
 
         def run(name):
             if name == "serial":
-                return O.ref_csr_serial(R, x)[0]
+                return O.ref_csr_serial(R, x)
             sched = "guided" if name == "omp_guided" else "nnz"
-            return O.ref_csr_omp(R, x, nthreads, sched)[0]
+            return O.ref_csr_omp(R, x, nthreads, sched)[:2]
 
         names = ["serial", "omp_guided", "omp_nnz"]
     else:
@@ -183,17 +213,23 @@ def cpu_reference_run(O, A_arrays, x, steps, warmup, threads=None, hll=True):
                           np.ascontiguousarray(AS, np.float64))
 
         def run(name):
-            return O.csr_spmv_timed(M, IRPc, JAc, ASc, x, 1 if name == "serial" else nthreads)[0]
+            return O.csr_spmv_timed(M, IRPc, JAc, ASc, x, 1 if name == "serial" else nthreads)
 
         names = ["serial", "omp_guided"]
     for name in names:
-        n_w, n_s = (min(warmup, 1), min(steps, 2)) if name == "serial" else (warmup, steps)
+        n_w, n_s = ((min(warmup, 1), min(steps, 2) if serial_steps is None else serial_steps) if name == "serial"
+                    else (warmup, steps))
         for _ in range(n_w):
             run(name)
-        ms = [run(name) for _ in range(n_s)]
+        ms = []
+        for _ in range(n_s):
+            t, y = run(name)
+            ms.append(t)
+        if ys is not None:
+            ys[name] = y
         variants[name] = {"ms_per_step": statistics.median(ms),
                           "gflops": 2.0 * nnz / (statistics.median(ms) * 1e6),
-                          "cores": 1 if name == "serial" else nthreads}
+                          "cores": 1 if name == "serial" else nthreads, "steps": n_s}
     best = max(variants, key=lambda k: variants[k]["gflops"])
     if hll and kind == "reference" and nnz <= 100_000_000:
         # the reference's HLL CPU paths too (row-major hacks, its own packer); reported beside
@@ -250,13 +286,17 @@ def run_reference_arm(args):
     arrays, sample = reference_sample(O, args.workload, args.gpus)
     M, N, IRP, JA, AS = arrays
     x = np.random.default_rng(0).uniform(0, 1, N)
-    steps = max(1, min(args.steps, 10))
+    steps = max(1, args.steps)
+    ys = {}
     kind, best, variants, nthreads = cpu_reference_run(O, arrays, x, steps, max(min(args.warmup, 2), 1),
-                                                       threads=max(O.max_threads(), 1), hll=False)
+                                                       threads=max(O.max_threads(), 1), hll=False,
+                                                       serial_steps=steps, ys=ys)
     v = variants[best]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"y": ys[best][dump_rows(M)]})
     line = {
         "impl": "reference", "metric": "fp64_spmv_gflops", "value": v["gflops"], "unit": "GFLOP/s",
-        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": v["ms_per_step"],
+        "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup, "ms_per_step": v["ms_per_step"],
         "higher_is_better": True, "scaling": "strong" if args.workload == "c5" else "weak",
         "vs_baseline": None, "dtype": "f64", "data": "synthetic", "gpu_launches": 0,
         "config": {"workload": f"{args.workload}: {DESCR[args.workload]}", "format": "csr", "rows": M,
@@ -264,7 +304,7 @@ def run_reference_arm(args):
                    "note": "GFLOP/s of the sample; SpMV throughput of the stencil does not depend on "
                            "how many planes are timed"},
         "cpu_baseline": {"value": v["gflops"], "unit": "GFLOP/s", "cores": v["cores"], "kind": kind,
-                         "sample": f"{sample}, {steps} SpMV passes per OpenMP variant (2 serial), median",
+                         "sample": f"{sample}, {steps} SpMV passes per variant, median",
                          "variants": variants, "host_threads": nthreads, "host_cores": cores,
                          "build": O.ref_kind() if kind == "reference" else "port"},
         "e2e": {"value": v["gflops"], "unit": "GFLOP/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -287,9 +327,11 @@ DOMINANT_KERNEL = {("c1", "csr"): "csr_pipe_kernel", ("c1", "hll"): "hll_pipe_ke
                    ("c3", "csr"): "sell_kernel", ("c3", "hll"): "sell_kernel", ("c4", "csr"): "sell_kernel"}
 
 
-def single_config(sp, O, torch, workload, steps, warmup, wpb, with_cpu=True, with_e2e=True, kernels=None):
+def single_config(sp, O, torch, workload, steps, warmup, wpb, with_cpu=True, with_e2e=True, kernels=None,
+                  keep_y=None):
     """One BASELINE single-GPU config: parity gate, then device-timed CSR and HLL, the e2e entry
-    points and the reference's CPU paths on the same matrix."""
+    points and the reference's CPU paths on the same matrix.  keep_y: a format; the dump_rows()
+    of the y its last timed step computed go to rec["y"]."""
     t_start = time.time()
     A = host_matrix(sp, workload)
     nnz, M, N = A.NZ, A.M, A.N
@@ -345,6 +387,8 @@ def single_config(sp, O, torch, workload, steps, warmup, wpb, with_cpu=True, wit
             b.record(stream)
         e_all.record(stream)
         torch.cuda.synchronize()
+        if name == keep_y:
+            y_last = y.cpu().numpy()[dump_rows(M)]
         per = [a.elapsed_time(b) for a, b in ev]
         total_ms = sum(per) if small else s_all.elapsed_time(e_all)
         ms_step, kern_ms = total_ms / steps, statistics.mean(per)
@@ -444,6 +488,8 @@ def single_config(sp, O, torch, workload, steps, warmup, wpb, with_cpu=True, wit
                          if small else "inputs larger than L2"),
            "parity": parity, "formats": results, "e2e": e2e, "cpu_baseline": cpu,
            "wall_s": time.time() - t_start}
+    if keep_y is not None:
+        rec["y"] = y_last
     del A
     progress(f"config {workload} done in {rec['wall_s']:.1f} s")
     return rec
@@ -476,7 +522,8 @@ def run_single(args):
     kernels = {"csr": args.kernel if args.kernel is not None and args.format == "csr" else 2,
                "hll": args.kernel if args.kernel is not None and args.format == "hll" else 2}
     rec = single_config(sp, O, torch, args.workload, args.steps, args.warmup, args.wpb,
-                        with_cpu=not args.no_cpu, kernels=kernels)
+                        with_cpu=not args.no_cpu, kernels=kernels,
+                        keep_y=args.format if args.dump_outputs else None)
     clocks = sampler.stop(t0, time.time())
     head = rec["formats"][args.format]
     e2e = rec["e2e"].get(args.format, {})
@@ -493,6 +540,8 @@ def run_single(args):
         "gpu_launches": head["launches_per_step"] * args.steps, "clocks": clocks,
         "formats": rec["formats"], "e2e_formats": rec["e2e"], "device": sp.device_info()["name"],
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"y": rec["y"]})
     emit(line)
     return 0
 
@@ -524,10 +573,14 @@ def main():
     ap.add_argument("--format", default="csr", choices=["csr", "hll"])
     ap.add_argument("--kernel", type=int, default=None)
     ap.add_argument("--wpb", type=int, default=4)
-    ap.add_argument("--regions", type=int, default=5, help="timed regions of K steps; the median is reported")
+    ap.add_argument("--regions", type=int, default=1,
+                    help="c5/c2w: the K timed steps are cut into this many regions, each after a reset of x")
     ap.add_argument("--configs", default="auto", choices=["auto", "all", "none"],
                     help="single-GPU BASELINE configs as sub-records of the N=1 line (auto: at N=1)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/y.npy (float64; all rows, or the "
+                         "same seeded sample of 2^21 rows when there are more)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 

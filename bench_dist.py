@@ -51,8 +51,8 @@ def gather_lists(dist, torch, device, values):
 def run(args):
     import torch
     import torch.distributed as dist
-    from bench import (ClockSampler, DESCR, emit, host_cores, measured_peak, ncu_traffic, progress, roofline_bytes,
-                       reference_gpu_rows, single_config, cpu_reference_run)
+    from bench import (ClockSampler, DESCR, dump_outputs, dump_rows, emit, host_cores, measured_peak, ncu_traffic,
+                       progress, roofline_bytes, reference_gpu_rows, single_config, cpu_reference_run)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -121,11 +121,12 @@ def run(args):
     bmin_total = roofline_bytes(n_total, n_total, nnz_total)
 
     # ---- timed regions ----
-    # Every region: x reset to x_0 (the iteration multiplies magnitudes by up to 52 per step, so a
-    # region starts from bounded values), W warm-up steps queued on the rank's stream, a
-    # stream-ordered rendezvous (one-word all-reduce the stepping stream waits for: ranks leave the
-    # host barrier milliseconds apart, and in push mode a rank may run one step ahead per hop),
-    # then exactly K steps between two CUDA events on that stream.  ms of a region = max over ranks.
+    # The K timed steps are cut into R regions of K/R steps.  Every region: x reset to x_0 (the
+    # iteration multiplies magnitudes by up to 52 per step, so a region starts from bounded values),
+    # W warm-up steps queued on the rank's stream, a stream-ordered rendezvous (one-word all-reduce
+    # the stepping stream waits for: ranks leave the host barrier milliseconds apart, and in push
+    # mode a rank may run one step ahead per hop), then its steps between two CUDA events on that
+    # stream.  ms of a region = max over ranks.
     sampler = None
     if rank == 0:
         sampler = ClockSampler(local)
@@ -136,13 +137,15 @@ def run(args):
     warm += warm % 2
     sync_word = torch.zeros(1, device=device)
     launches0 = sp.counters()["launches"]
+    n_regions = max(1, min(args.regions, args.steps))
+    region_steps = [args.steps * (i + 1) // n_regions - args.steps * i // n_regions for i in range(n_regions)]
     region_ms_mine = []
-    for _ in range(max(1, args.regions)):
+    for k in region_steps:
         it.set_x(x0_own)                       # sync + barrier inside
         it.iterate(warm)
         with torch.cuda.stream(it.stream):
             dist.all_reduce(sync_word)
-        region_ms_mine.append(it.time(args.steps, 1)[0])
+        region_ms_mine.append(it.time(k, 1)[0])
         torch.cuda.synchronize()
         dist.barrier()
     launches = sp.counters()["launches"] - launches0
@@ -151,8 +154,16 @@ def run(args):
         progress(f"{args.workload}: {len(region_ms_mine)} timed regions done")
     by_rank = gather_lists(dist, torch, device, region_ms_mine)          # [rank][region]
     region_ms = [max(by_rank[r][i] for r in range(world)) for i in range(len(region_ms_mine))]
-    total_ms = statistics.median(region_ms)
-    finite = bool(np.isfinite(it.result_own()).all())
+    total_ms = sum(region_ms)
+    x_last = it.result_own()                   # x after the last region's warm-up and timed steps: rows [r0, r1)
+    finite = bool(np.isfinite(x_last).all())
+    y_dump = None
+    if args.dump_outputs:
+        rows = dump_rows(n_total)
+        parts = [None] * world
+        dist.all_gather_object(parts, x_last[rows[(rows >= r0) & (rows < r1)] - r0])
+        y_dump = np.concatenate(parts)         # slabs are in rank order
+    del x_last
     launches_per_step = len(plan.segments) + (2 if it.mode == "push" and world > 1 else 0)
 
     # ---- stand-alone kernel again, after the peers are mapped and the job has run ----
@@ -216,13 +227,15 @@ def run(args):
                        "exchange": it.mode, "cuda_graph": it.has_graph,
                        "halo_bytes_per_rank_per_step": plan.halo_bytes(),
                        "l2_policy": "inputs larger than L2 (>= 0.7 GB streamed per GPU per step)",
-                       "timing": f"median of {len(region_ms)} regions of exactly {args.steps} steps, each after a reset "
-                                 f"of x and {warm} warm-up steps; CUDA events on the stepping stream; max over ranks",
+                       "timing": f"{args.steps} steps in {len(region_ms)} region(s) of {region_steps} steps, each after a "
+                                 f"reset of x and {warm} warm-up steps; CUDA events on the stepping stream; max over ranks",
+                       "warmup_steps_per_region": warm,
                        "shard_build_s": t_build, "finite": finite,
                        "e2e_path": "per rank: host x[c0,c1) in, host y slice out through spmv_b200_csr_spmv_host "
                                    "(x upload, row-chunk kernels, y download pipelined on 3 streams)"},
             "hbm_gbs": bmin_total / (ms_step * 1e6),
             "regions_ms": region_ms,
+            "region_steps": region_steps,
             "region_ms_by_rank": {"min": [min(r) for r in by_rank], "median": [statistics.median(r) for r in by_rank],
                                   "max": [max(r) for r in by_rank]},
             "roofline": {"bound": "hbm", "achieved": bmin_local / (kern_ms * 1e6), "peak": peak, "unit": "GB/s",
@@ -237,7 +250,7 @@ def run(args):
             "standalone_kernel_ms_by_rank": {"before_peer_mapping_mean": [a[0] for a in alone],
                                              "before_peer_mapping_min": [a[1] for a in alone],
                                              "after_run_mean": [a[2] for a in alone],
-                                             "after_run_min": [a[3] for a in alone]},
+                                             "after_run_min": [a[3] for a in alone], "reps": reps_alone},
             "cpu_baseline": None,
             "e2e": dict(e2e_rec("pageable"), pinned=e2e_rec("pinned")),
             "gpu_launches": launches_per_step * args.steps,
@@ -276,8 +289,8 @@ def run(args):
             line["configs"] = {}
             for wl in ("c2", "c1", "c3", "c4"):
                 try:
-                    line["configs"][wl] = single_config(sp, O, torch, wl, steps=20, warmup=3, wpb=args.wpb,
-                                                        with_cpu=not args.no_cpu)
+                    line["configs"][wl] = single_config(sp, O, torch, wl, steps=args.steps, warmup=args.warmup,
+                                                        wpb=args.wpb, with_cpu=not args.no_cpu)
                 except SystemExit as e:     # a failed parity gate is reported, never hidden
                     line["configs"][wl] = {"error": str(e)}
                 torch.cuda.empty_cache()
@@ -288,6 +301,8 @@ def run(args):
                             "on this GPU, C2 (128^3 stencil), one launch per call as the reference times it",
                     "rows": ref_gpu}
     if rank == 0:
+        if y_dump is not None:
+            dump_outputs(args.dump_outputs, {"y": y_dump})
         emit(line)
     dist.barrier()
     dist.destroy_process_group()

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -34,9 +35,26 @@ def test_reference_arm_line():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_reference_arm_times_every_step(tmp_path):
+    """--steps K times exactly K passes of every variant (no cap), and --dump-outputs writes y of
+    the headline variant: A x for x as bench.py draws it."""
+    d = run_bench("--impl", "reference", "--workload", "tiny", "--steps", "12", "--warmup", "1",
+                  "--dump-outputs", str(tmp_path))
+    assert d["steps"] == 12
+    variants = d["cpu_baseline"]["variants"]
+    assert {"serial", "omp_guided"} <= set(variants)
+    assert all(v["steps"] == 12 for v in variants.values())
+    from oracle import oracle as O
+    M, N, IRP, JA, AS = O.gen_stencil27(32, 32, 32)
+    x = np.random.default_rng(0).uniform(0, 1, N)
+    y = np.load(tmp_path / "y.npy")
+    assert y.dtype == np.float64 and y.shape == (M,)
+    assert O.check_tolerance(y, O.csr_spmv(M, IRP, JA, AS, x), O.csr_abs_bound(M, IRP, JA, AS, x), 1e-12)[0]
+
+
 @pytest.mark.gpu
-def test_b200_arm_line():
-    d = run_bench("--workload", "tiny", "--steps", "5", "--warmup", "3")
+def test_b200_arm_line(tmp_path):
+    d = run_bench("--workload", "tiny", "--steps", "5", "--warmup", "3", "--dump-outputs", str(tmp_path))
     assert BASE_KEYS | {"roofline", "gpu_launches", "clocks"} <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 5 and d["value"] > 0
     rf = d["roofline"]
@@ -50,22 +68,43 @@ def test_b200_arm_line():
     assert d["cpu_baseline"]["value"] > 0
     assert d["config"]["parity"]["csr"]["ok"] and d["config"]["parity"]["hll"]["ok"]
     assert "sm_mhz" in d["clocks"] and isinstance(d["clocks"]["reasons"], list)
+    # --dump-outputs: y = A x of the last timed step, every row (32^3 < 2^21), x as bench.py draws it
+    from oracle import oracle as O
+    M, N, IRP, JA, AS = O.gen_stencil27(32, 32, 32)
+    x = np.random.default_rng(0).uniform(0, 1, N)
+    y = np.load(tmp_path / "y.npy")
+    assert y.dtype == np.float64 and y.shape == (M,)
+    assert O.check_tolerance(y, O.csr_spmv(M, IRP, JA, AS, x), O.csr_abs_bound(M, IRP, JA, AS, x), 1e-12)[0]
 
 
 @pytest.mark.gpu
-def test_b200_default_path_line():
+def test_b200_default_path_line(tmp_path):
     """The default path (bench_dist, one rank = one GPU) on the small slab workload: strong/weak
-    flag, repeated timed regions, stand-alone kernel before and after, both e2e variants."""
+    flag, K timed steps cut into regions, stand-alone kernel before and after, both e2e variants."""
     d = run_bench("--workload", "c2w", "--steps", "4", "--warmup", "3", "--regions", "3", "--configs", "none",
-                  "--no-cpu")
+                  "--no-cpu", "--dump-outputs", str(tmp_path))
     assert BASE_KEYS | {"roofline", "gpu_launches", "clocks", "regions_ms"} <= set(d)
     assert d["n_gpus"] == 1 and d["scaling"] == "weak" and len(d["regions_ms"]) == 3
     assert d["config"]["nnz"] == 55742968 and d["config"]["cuda_graph"] is True and d["config"]["finite"]
-    assert abs(d["ms_per_step"] * 4 - sorted(d["regions_ms"])[1]) < 1e-9
+    assert d["region_steps"] == [1, 1, 2]
+    assert abs(d["ms_per_step"] * 4 - sum(d["regions_ms"])) < 1e-9
     assert 0.3 < d["roofline"]["frac"] < 1.2
     assert d["e2e"]["value"] > 0 and d["e2e"]["pinned"]["value"] >= 0.5 * d["e2e"]["value"]
     assert d["parity"]["step1_vs_oracle"] is True
     assert len(d["standalone_kernel_ms_by_rank"]["after_run_mean"]) == 1
+    # --dump-outputs: x after the last region = A^(w+2) x_0 (w warm-up steps after the reset, then its
+    # 2 timed steps), every row (128^3 = 2^21)
+    from bench_dist import x0_slice
+    from oracle import oracle as O
+    M, N, IRP, JA, AS = O.gen_stencil27(128, 128, 128)
+    steps = d["config"]["warmup_steps_per_region"] + 2
+    x = x0_slice(0, N)
+    for _ in range(steps):
+        bound = O.csr_abs_bound(M, IRP, JA, AS, np.abs(x))
+        x = O.csr_spmv(M, IRP, JA, AS, x)
+    y = np.load(tmp_path / "y.npy")
+    assert y.dtype == np.float64 and y.shape == (M,)
+    assert O.check_tolerance(y, x, steps * bound, 1e-12)[0]
 
 
 def test_reference_arm_under_torchrun_env():
