@@ -16,10 +16,9 @@
  *                                      (row-major input transposed on upload)
  *   1 hll_spmv_cuda_threads_col_major  thread per row, scalar loads
  *   2 hll_spmv_cuda_warp_block         warp per hack, lane = row, 64-bit value / 32-bit
- *                                      index loads (the 128- and 256-bit variants measured
- *                                      slower and stay behind the "hll_vec" knob); narrow
- *                                      hacks (width <= 8) through per-warp cp.async.bulk
- *                                      rings; column panels (SELL-P) when x is larger than
+ *                                      index loads (128- and 256-bit loads measured
+ *                                      slower); narrow hacks (width <= 8) through
+ *                                      per-warp cp.async.bulk rings; column panels (SELL-P) when x is larger than
  *                                      the L2 and the columns scatter
  *   3 hll_spmv_cuda_halfwarp_row       warp per hack, streams staged in shared
  *                                      memory by cp.async.bulk (TMA)

@@ -173,9 +173,9 @@ int spmv_b200_csr_spmv_fused(spmv_b200_csr *h, int kernel, int warps_per_block,
 int spmv_b200_csr_spmv_host(spmv_b200_csr *h, int kernel, int warps_per_block, const double *x,
                             double *y, double *kernel_ms);
 /* SELL-P plan of this matrix (column-panelled, window-sorted slices; csrc/sell_kernels.cuh):
- * out[0..13) = {state (1 built), panels, sigma, slices, padded slots, entries in slices, rows
+ * out[0..11) = {state (1 built), panels, sigma, slices, padded slots, entries in slices, rows
  * handled by the long-row kernels, gather span * 1e6, virtual-row chunk (0: none), rows split into
- * pieces, pieces, columns in the shared-memory hot table, share of the gathers they serve * 1e6}.
+ * pieces, pieces}.
  * build != 0 builds the plan first. */
 int spmv_b200_csr_sell_info(spmv_b200_csr *h, int build, int64_t *out, int n_out);
 /* Device SELL-P arrays back to the host for bit-compare (any output may be NULL):
@@ -256,11 +256,10 @@ void spmv_b200_set_timing(int warmup, int reps);
 void spmv_b200_counters(int64_t *launches, int64_t *h2d_bytes,
                         int64_t *d2h_bytes);
 
-/* Experiment knobs used by bin/kbench sweeps and tests ("csr_stream_cfg", "hll_vec",
- * "hll_stream_cfg", "regular_lpr", "adaptive_direct", "force_wide", "pipeline", "pipe_chunks",
- * "csr_pipe", "hll_pipe" (short rows / narrow hacks through per-warp bulk-copy rings: -1 auto, 0 off,
- * 1 whenever they fit), "sell", "sell_panels", "sell_sigma", "sell_panel_mb", "sell_max_row",
- * "sell_unroll", "sell_chunk", "sell_hot", "sell_hot_mode", "cache", "l2_fetch_granularity").
+/* Experiment knobs used by bin/kbench sweeps and tests ("csr_stream_cfg", "hll_stream_cfg",
+ * "force_wide", "pipeline", "pipe_chunks", "csr_pipe", "hll_pipe" (short rows / narrow hacks
+ * through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit), "sell", "sell_panels",
+ * "sell_sigma", "sell_panel_mb", "sell_max_row", "sell_chunk", "cache").
  * 0 or -EINVAL.  Knobs that change planning must be set before a handle is created. */
 int spmv_b200_set_knob(const char *key, int value);
 

@@ -450,10 +450,10 @@ class CsrDevice:
         return ms.value
 
     def sell_info(self, build=False):
-        out = (C.c_int64 * 13)()
-        self._check(L.b200.spmv_b200_csr_sell_info(self._h, int(build), out, 13))
+        out = (C.c_int64 * 11)()
+        self._check(L.b200.spmv_b200_csr_sell_info(self._h, int(build), out, 11))
         keys = ("state", "panels", "sigma", "slices", "slots", "nnz_in_slices", "long_rows", "gather_span_ppm",
-                "chunk", "split_rows", "pieces", "hot_columns", "hot_coverage_ppm")
+                "chunk", "split_rows", "pieces")
         return dict(zip(keys, list(out)))
 
     def sell_download(self):

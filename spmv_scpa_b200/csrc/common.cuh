@@ -89,27 +89,6 @@ __device__ __forceinline__ int ld_stream_s32(const int *p, uint64_t pol) {
                    : "l"(p), "l"(pol));
       return v;
 }
-__device__ __forceinline__ double2 ld_stream_f64x2(const double *p, uint64_t pol) {
-      double2 v;
-      asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.f64 {%0,%1}, [%2], %3;"
-                   : "=d"(v.x), "=d"(v.y)
-                   : "l"(p), "l"(pol));
-      return v;
-}
-__device__ __forceinline__ int2 ld_stream_s32x2(const int *p, uint64_t pol) {
-      int2 v;
-      asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.s32 {%0,%1}, [%2], %3;"
-                   : "=r"(v.x), "=r"(v.y)
-                   : "l"(p), "l"(pol));
-      return v;
-}
-__device__ __forceinline__ int4 ld_stream_s32x4(const int *p, uint64_t pol) {
-      int4 v;
-      asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.s32 {%0,%1,%2,%3}, [%4], %5;"
-                   : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-                   : "l"(p), "l"(pol));
-      return v;
-}
 // Same L2 priority but allowed to live in L1: sub-warp row groups re-touch the
 // tail of a 32-byte sector on their next step.
 __device__ __forceinline__ double ld_stream_l1_f64(const double *p, uint64_t pol) {
@@ -120,17 +99,6 @@ __device__ __forceinline__ double ld_stream_l1_f64(const double *p, uint64_t pol
 __device__ __forceinline__ int ld_stream_l1_s32(const int *p, uint64_t pol) {
       int v;
       asm("ld.global.nc.L2::cache_hint.s32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-      return v;
-}
-// 256-bit load (sm_100+): four doubles per lane, 1 KiB per warp instruction.
-struct double4_t {
-      double a, b, c, d;
-};
-__device__ __forceinline__ double4_t ld_stream_f64x4(const double *p) {
-      double4_t v;
-      asm("ld.global.nc.L1::no_allocate.L2::evict_first.v4.f64 {%0,%1,%2,%3}, [%4];"
-                   : "=d"(v.a), "=d"(v.b), "=d"(v.c), "=d"(v.d)
-                   : "l"(p));
       return v;
 }
 

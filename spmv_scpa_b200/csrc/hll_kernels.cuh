@@ -12,13 +12,8 @@
 // boundary and a warp reads whole 256-byte lines.
 //
 // Kernels (reference counterparts: src/cuda_hll.cu:19-152):
-//   hll_warp_kernel<VEC>  warp per hack.  VEC=1: lane = row, 64-bit value and
-//                         32-bit index loads.  VEC=2: 128-bit value / 64-bit
-//                         index loads, a lane owns 2 rows of every other slot
-//                         column.  VEC=4: 256-bit value / 128-bit index loads,
-//                         a lane owns 4 rows of every 4th slot column.  The
-//                         partial sums of lanes that share rows are combined
-//                         with shuffles.
+//   hll_warp_kernel       warp per hack, lane = row, 64-bit value and 32-bit
+//                         index loads.
 //   hll_stream_kernel     persistent CTAs; groups of consecutive hacks are
 //                         staged in shared memory by cp.async.bulk (TMA)
 //                         through an mbarrier ring; warp per hack, lane = row.
@@ -28,12 +23,12 @@
 
 namespace b200 {
 
-template <int VEC, int EPI>
+template <int EPI>
 __global__ void __launch_bounds__(1024)
     hll_warp_kernel(const long long *__restrict__ hoff, const int *__restrict__ ja,
                     const double *__restrict__ as, long long hack0, long long n_hacks, long long M,
                     const double *__restrict__ x, double *__restrict__ y, EpiArgs epi) {
-      static_assert(EPI == EPI_PLAIN || (EPI == EPI_FUSED && VEC == 1), "HLL epilogues");
+      static_assert(EPI == EPI_PLAIN || EPI == EPI_FUSED, "HLL epilogues");
       const long long wslot = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
       const long long h = hack0 + wslot;
       if (h >= n_hacks)
@@ -48,88 +43,33 @@ __global__ void __launch_bounds__(1024)
       const int *hja = ja + base;
       const long long row_base = h * kHack;
 
-      if (VEC == 1) {
-            constexpr int U = 4;
-            double acc0 = 0.0, acc1 = 0.0;
-            for (int j = 0; j < width; j += U) {
-                  double a[U], xv[U];
-                  int c[U];
-                  bool okm[U];
+      constexpr int U = 4;
+      double acc0 = 0.0, acc1 = 0.0;
+      for (int j = 0; j < width; j += U) {
+            double a[U], xv[U];
+            int c[U];
+            bool okm[U];
 #pragma unroll
-                  for (int u = 0; u < U; ++u) {
-                        const int s = (j + u) * 32 + lane;
-                        const bool ok = j + u < width;
-                        okm[u] = ok;
-                        a[u] = ok ? ld_stream_f64(has + s, pol_s) : 0.0;
-                        c[u] = ok ? ld_stream_s32(hja + s, pol_s) : 0;
-                  }
-#pragma unroll
-                  for (int u = 0; u < U; ++u)
-                        xv[u] = okm[u] ? ld_x(x + c[u], pol_x) : 0.0;
-#pragma unroll
-                  for (int u = 0; u < U; u += 2) {
-                        acc0 = fma(a[u], xv[u], acc0);
-                        acc1 = fma(a[u + 1], xv[u + 1], acc1);
-                  }
-            }
-            const double acc = acc0 + acc1;
-            if (row_base + lane < M)
-                  store_y<EPI>(y, row_base + lane, acc, epi, dot_acc);
-            epi_finish_warp<EPI>(epi, dot_acc, wslot);
-      } else if (VEC == 2) {
-            // lane L: rows 2*(L&15), +1 ; slot columns j + (L>>4), step 2
-            const int sub = lane & 15, half = lane >> 4;
-            double acc0 = 0.0, acc1 = 0.0;
-#pragma unroll 4
-            for (int j = half; j < width; j += 2) {
-                  const int s = j * 32 + 2 * sub;
-                  const double2 a = ld_stream_f64x2(has + s, pol_s);
-                  const int2 c = ld_stream_s32x2(hja + s, pol_s);
-                  acc0 = fma(a.x, ld_x(x + c.x, pol_x), acc0);
-                  acc1 = fma(a.y, ld_x(x + c.y, pol_x), acc1);
-            }
-            acc0 += __shfl_xor_sync(0xffffffffu, acc0, 16);
-            acc1 += __shfl_xor_sync(0xffffffffu, acc1, 16);
-            if (half == 0) {
-                  const long long r = row_base + 2 * sub;
-                  if (r < M)
-                        store_y<EPI>(y, r, acc0, epi, dot_acc);
-                  if (r + 1 < M)
-                        store_y<EPI>(y, r + 1, acc1, epi, dot_acc);
-            }
-      } else {
-            // lane L: rows 4*(L&7) .. +3 ; slot columns j + (L>>3), step 4
-            const int sub = lane & 7, quarter = lane >> 3;
-            double acc0 = 0.0, acc1 = 0.0, acc2 = 0.0, acc3 = 0.0;
-#pragma unroll 2
-            for (int j = quarter; j < width; j += 4) {
-                  const int s = j * 32 + 4 * sub;
-                  const double4_t a = ld_stream_f64x4(has + s);
-                  const int4 c = ld_stream_s32x4(hja + s, pol_s);
-                  acc0 = fma(a.a, ld_x(x + c.x, pol_x), acc0);
-                  acc1 = fma(a.b, ld_x(x + c.y, pol_x), acc1);
-                  acc2 = fma(a.c, ld_x(x + c.z, pol_x), acc2);
-                  acc3 = fma(a.d, ld_x(x + c.w, pol_x), acc3);
+            for (int u = 0; u < U; ++u) {
+                  const int s = (j + u) * 32 + lane;
+                  const bool ok = j + u < width;
+                  okm[u] = ok;
+                  a[u] = ok ? ld_stream_f64(has + s, pol_s) : 0.0;
+                  c[u] = ok ? ld_stream_s32(hja + s, pol_s) : 0;
             }
 #pragma unroll
-            for (int o = 8; o <= 16; o <<= 1) {
-                  acc0 += __shfl_xor_sync(0xffffffffu, acc0, o);
-                  acc1 += __shfl_xor_sync(0xffffffffu, acc1, o);
-                  acc2 += __shfl_xor_sync(0xffffffffu, acc2, o);
-                  acc3 += __shfl_xor_sync(0xffffffffu, acc3, o);
-            }
-            if (quarter == 0) {
-                  const long long r = row_base + 4 * sub;
-                  if (r < M)
-                        store_y<EPI>(y, r, acc0, epi, dot_acc);
-                  if (r + 1 < M)
-                        store_y<EPI>(y, r + 1, acc1, epi, dot_acc);
-                  if (r + 2 < M)
-                        store_y<EPI>(y, r + 2, acc2, epi, dot_acc);
-                  if (r + 3 < M)
-                        store_y<EPI>(y, r + 3, acc3, epi, dot_acc);
+            for (int u = 0; u < U; ++u)
+                  xv[u] = okm[u] ? ld_x(x + c[u], pol_x) : 0.0;
+#pragma unroll
+            for (int u = 0; u < U; u += 2) {
+                  acc0 = fma(a[u], xv[u], acc0);
+                  acc1 = fma(a[u + 1], xv[u + 1], acc1);
             }
       }
+      const double acc = acc0 + acc1;
+      if (row_base + lane < M)
+            store_y<EPI>(y, row_base + lane, acc, epi, dot_acc);
+      epi_finish_warp<EPI>(epi, dot_acc, wslot);
 }
 
 // ------------------------------------------------------------------------

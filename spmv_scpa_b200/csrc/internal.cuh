@@ -32,25 +32,19 @@ extern Counters g_counters;
 
 struct Knobs {
       int csr_stream_cfg = -1; // -1: pick from warps_per_block and the row-length profile
-      int hll_vec = -1;        // vector width of the HLL headline kernel; -1 = 1
       int csr_pipe = -1;       // short regular CSR rows through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit
       int hll_pipe = -1;       // narrow hacks through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit
       int hll_stream_cfg = -1;
-      int regular_lpr = -1;    // force lanes-per-row (log2) of the adaptive base launch
       int force_wide = 0;      // use 64-bit row offsets even when NZ < 2^31 (tests)
-      int adaptive_direct = 0; // 1: the adaptive path uses the direct binned kernels only
       int pipeline = 1;        // host-buffer pipeline in the host-pointer entry points
       int pipe_chunks = 0;     // 0: by size
       int sell = -1;           // -1 auto, 0 never, 1 always route ids 2/4 (CSR) and 2 (HLL) to SELL-P
       int sell_panels = 0;     // 0: by size of x
       int sell_sigma = 16384;  // rows per sorting window
       int sell_panel_mb = 64;  // target size of a panel's x slice (C3 sweep: 64 MB beats 43 / 32 MB)
-      int sell_unroll = 4;     // slot columns a lane keeps in flight (4 or 8)
       int sell_max_row = 4096; // longer rows go to the CSR long-row kernels (panel mode)
       int sell_chunk = 256;    // ragged matrices: rows are cut into virtual rows of this many entries
                                // (C4 sweep: 32/64/128/256/512/1024 -> 34/42/45/46/44/39 %); 0 = off
-      int sell_hot = 0;        // ragged matrices: size of the hot-column table (0 = off)
-      int sell_hot_mode = 0;   // home of the table: 0 shared memory (persistent CTAs), 1 compact global array kept in the L1
       int cache = 1;           // entry-point matrix cache: 0 off, 1 full content hash, 2 trust pointers
       int warmup = 1, reps = 3;
 };
@@ -147,11 +141,6 @@ struct SellPlan {
       int *d_split_row = nullptr, *d_split_first = nullptr;
       double *d_partial = nullptr;
       double *d_partial_mm = nullptr; // 4 partial sums per piece (SpMM), allocated on first use
-      // hot-column table (virtual-row form only): columns served from shared memory
-      int n_hot = 0;
-      int *d_hot_cols = nullptr;
-      double *d_xhot = nullptr; // x[hot_cols[..]], refreshed before every launch (L1 mode)
-      double hot_coverage = 0.0;
       // rows too long for a slice (CSR source only): warp-per-row, CTA-per-row and split lists
       RowList long_warp;
       RowList long_block;

@@ -38,9 +38,9 @@
 
 namespace b200 {
 
-// One warp per slice, lane = row (the mapping of hll_warp_kernel<1>, which measured best
+// One warp per slice, lane = row (the mapping of hll_warp_kernel, which measured best
 // whenever the gather is the limiter).  Slices [slice0, slice0 + n) of one panel.
-template <int EPI, int U, bool VROWS = false>
+template <int EPI, bool VROWS = false>
 __global__ void __launch_bounds__(1024)
     sell_kernel(const long long *__restrict__ soff, const int *__restrict__ perm,
                 const int *__restrict__ ja, const double *__restrict__ as, long long n_slices,
@@ -59,6 +59,7 @@ __global__ void __launch_bounds__(1024)
       const uint64_t pol_x = policy_evict_last();
       const double *sas = as + base;
       const int *sja = ja + base;
+      constexpr int U = 4;
 
       double acc0 = 0.0, acc1 = 0.0;
       for (int j = 0; j < width; j += U) {
@@ -143,152 +144,6 @@ __global__ void __launch_bounds__(512)
 #pragma unroll
             for (int k = 0; k < K; ++k)
                   out[k] = (EPI == EPI_ACC && row >= 0) ? out[k] + acc[k] : acc[k];
-      }
-}
-
-// Hot-column variant (ragged matrices, one panel).  Power-law matrices are as skewed in their
-// columns as in their rows: on R-MAT scale 24 the 12 288 most referenced columns (0.07 % of x)
-// take 27 % of all gathers, the top 24 576 take 34 %.  Every gather that goes to the L2 moves a
-// 32-byte sector for 8 useful bytes, and the L2's sector throughput is what bounds the kernel
-// (profiles/r2_c4_ncu_summary.md), so those columns are served from a compact table instead: at
-// build time the H hottest columns get the codes ~0 .. ~(H-1) in the slices' index array
-// (negative = "slot of the hot table").  Two homes for the table:
-//   HOT_SMEM  shared memory; each persistent CTA first copies x[hot_cols[0..H)] into it;
-//   HOT_L1    a compact global array (filled by hot_gather_kernel before the launch) that the
-//             hot gathers keep in the L1 (L1::evict_last) while every other load bypasses it
-//             (L1::no_allocate): the L1 tags 128-byte lines, so the SCATTERED hot columns of x
-//             cannot live there (2 048 lines), but 16 packed ones per line can.
-// A gather is TWO predicated loads (hot / cold), never a branch and never a generic load: the
-// round-2 version picked the address with a select and issued one generic load, which the LSU
-// splits and replays when a warp mixes shared and global lanes (measured 2-3x slower,
-// profiles/r2_kbench_c4_chunks_and_hot_table.txt).
-constexpr int HOT_SMEM = 0;
-constexpr int HOT_L1 = 1;
-
-template <int MODE>
-__device__ __forceinline__ double ld_x_hot(const double *x, const double *xhot, uint32_t s_hot, int c,
-                                           uint64_t pol) {
-      double v;
-      if (MODE == HOT_SMEM) {
-            asm("{\n\t"
-                ".reg .pred p;\n\t"
-                ".reg .b32 sa;\n\t"
-                ".reg .b64 ga;\n\t"
-                "setp.lt.s32 p, %1, 0;\n\t"
-                "not.b32 sa, %1;\n\t"
-                "shl.b32 sa, sa, 3;\n\t"
-                "add.u32 sa, sa, %2;\n\t"
-                "mul.wide.s32 ga, %1, 8;\n\t"
-                "add.u64 ga, ga, %3;\n\t"
-                "@p ld.shared.f64 %0, [sa];\n\t"
-                "@!p ld.global.nc.L2::cache_hint.f64 %0, [ga], %4;\n\t"
-                "}"
-                : "=d"(v)
-                : "r"(c), "r"(s_hot), "l"(x), "l"(pol));
-      } else {
-            asm("{\n\t"
-                ".reg .pred p;\n\t"
-                ".reg .b32 hi;\n\t"
-                ".reg .b64 ha, ga;\n\t"
-                "setp.lt.s32 p, %1, 0;\n\t"
-                "not.b32 hi, %1;\n\t"
-                "mul.wide.s32 ha, hi, 8;\n\t"
-                "add.u64 ha, ha, %2;\n\t"
-                "mul.wide.s32 ga, %1, 8;\n\t"
-                "add.u64 ga, ga, %3;\n\t"
-                "@p ld.global.nc.L1::evict_last.f64 %0, [ha];\n\t"
-                "@!p ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [ga], %4;\n\t"
-                "}"
-                : "=d"(v)
-                : "r"(c), "l"(xhot), "l"(x), "l"(pol));
-      }
-      return v;
-}
-
-// xhot[i] = x[hot_cols[i]]
-static __global__ void hot_gather_kernel(const double *__restrict__ x, const int *__restrict__ hot_cols,
-                                         int n_hot, double *__restrict__ xhot) {
-      const int i = blockIdx.x * blockDim.x + threadIdx.x;
-      if (i < n_hot)
-            xhot[i] = x[hot_cols[i]];
-}
-
-// Warps walk slices s, s + (warps of the grid), ...: with a grid that covers every slice this is
-// one slice per warp (HOT_L1), with one or two CTAs per SM it is a persistent kernel (HOT_SMEM).
-template <int EPI, int U, int THREADS, int MIN_CTAS, int MODE>
-__global__ void __launch_bounds__(THREADS, MIN_CTAS)
-    sell_hot_kernel(const long long *__restrict__ soff, const int *__restrict__ perm,
-                    const int *__restrict__ ja, const double *__restrict__ as, long long n_slices,
-                    const double *__restrict__ x, double *__restrict__ y,
-                    double *__restrict__ partial, const int *__restrict__ hot_cols,
-                    const double *__restrict__ xhot, int n_hot, EpiArgs epi) {
-      extern __shared__ double s_hot[];
-      if (MODE == HOT_SMEM) {
-            for (int i = threadIdx.x; i < n_hot; i += blockDim.x)
-                  s_hot[i] = x[hot_cols[i]];
-            __syncthreads();
-      }
-      const uint32_t s_hot_addr = MODE == HOT_SMEM ? smem_u32(s_hot) : 0u;
-      const int lane = threadIdx.x & 31;
-      const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
-      const uint64_t pol_s = policy_evict_first();
-      const uint64_t pol_x = policy_evict_last();
-      for (long long s = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); s < n_slices;
-           s += warps) {
-            const long long base = soff[s];
-            const int width = (int)((soff[s + 1] - base) >> 5);
-            const int row = perm[s * 32 + lane];
-            const double *sas = as + base;
-            const int *sja = ja + base;
-            double acc0 = 0.0, acc1 = 0.0;
-#pragma unroll 1
-            for (int j = 0; j < width; j += U) {
-                  double a[U], xv[U];
-                  int c[U];
-                  bool okm[U];
-#pragma unroll
-                  for (int u = 0; u < U; ++u) {
-                        const int k = (j + u) * 32 + lane;
-                        const bool ok = j + u < width;
-                        okm[u] = ok;
-                        a[u] = ok ? ld_stream_f64(sas + k, pol_s) : 0.0;
-                        c[u] = ok ? ld_stream_s32(sja + k, pol_s) : 0;
-                  }
-#pragma unroll
-                  for (int u = 0; u < U; ++u) {
-                        const double v = ld_x_hot<MODE>(x, xhot, s_hot_addr, c[u], pol_x);
-                        xv[u] = okm[u] ? v : 0.0; // beyond the slice: x[0] was read, not used
-                  }
-#pragma unroll
-                  for (int u = 0; u < U; u += 2) {
-                        acc0 = fma(a[u], xv[u], acc0);
-                        acc1 = fma(a[u + 1], xv[u + 1], acc1);
-                  }
-            }
-            double dot_acc = 0.0;
-            if (row >= 0)
-                  store_y<EPI>(y, row, acc0 + acc1, epi, dot_acc);
-            else if (row < -1)
-                  partial[-2 - row] = acc0 + acc1;
-            epi_finish_warp<EPI>(epi, dot_acc, s);
-      }
-}
-
-// counts[c] += 1 for every stored entry with column c (hot-column selection)
-static __global__ void col_hist_kernel(const int *__restrict__ ja, long long n, int *__restrict__ counts) {
-      for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n;
-           k += (long long)gridDim.x * blockDim.x)
-            atomicAdd(&counts[ja[k]], 1);
-}
-
-// ja[k] = ~hot_idx[ja[k]] where the column is hot
-static __global__ void sell_mark_hot_kernel(int *__restrict__ ja, long long n,
-                                            const int *__restrict__ hot_idx) {
-      for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n;
-           k += (long long)gridDim.x * blockDim.x) {
-            const int h = hot_idx[ja[k]];
-            if (h >= 0)
-                  ja[k] = ~h;
       }
 }
 

@@ -93,7 +93,6 @@ void free_sell(SellPlan &sp) {
       free_list(sp.long_block);
       free_split(sp.long_split);
       cudaFree(sp.d_split_row), cudaFree(sp.d_split_first), cudaFree(sp.d_partial), cudaFree(sp.d_partial_mm);
-      cudaFree(sp.d_hot_cols), cudaFree(sp.d_xhot);
       sp = SellPlan();
 }
 void free_segment(Segment &sg) {
@@ -160,10 +159,6 @@ int build_adaptive(spmv_b200_csr *h, Segment &sg) {
             below += sg.kind_rows[k];
       sg.regular = rows > 0 && below * 10 >= rows * 9;
       sg.base_kind = dom;
-      if (g_knobs.regular_lpr >= 0 && g_knobs.regular_lpr <= 5) {
-            sg.regular = true;
-            sg.base_kind = g_knobs.regular_lpr;
-      }
       return 0;
 }
 
@@ -653,60 +648,6 @@ void sell_virtual_rows(const std::vector<long long> &irp, long long M, int chunk
       split_first.push_back((int)p);
 }
 
-// Hot-column table of a built virtual-row plan: the H most referenced columns (by a device
-// histogram over the CSR's index array) get negative codes in the slices' index array.  Skipped
-// when they would serve less than a tenth of the gathers (uniform columns).
-int sell_pick_hot_columns(const int *d_csr_ja, long long nnz, long long N, SellPlan &sp) {
-      const int H = (int)std::min<long long>(std::min(g_knobs.sell_hot, 28000), N);
-      if (H < 32 || nnz <= 0)
-            return 0;
-      int *d_cnt = nullptr;
-      B200_CUDA(cudaMalloc(&d_cnt, (size_t)N * sizeof(int)));
-      B200_CUDA(cudaMemset(d_cnt, 0, (size_t)N * sizeof(int)));
-      col_hist_kernel<<<1184, 256>>>(d_csr_ja, nnz, d_cnt);
-      std::vector<int> cnt((size_t)N);
-      cudaError_t e = cudaMemcpy(cnt.data(), d_cnt, (size_t)N * sizeof(int), cudaMemcpyDeviceToHost);
-      cudaFree(d_cnt);
-      if (e != cudaSuccess)
-            return fail(-EIO, "column histogram failed: %s", cudaGetErrorString(e));
-      std::vector<int> order((size_t)N);
-      std::iota(order.begin(), order.end(), 0);
-      std::nth_element(order.begin(), order.begin() + H, order.end(), [&](int a, int b) {
-            return cnt[a] != cnt[b] ? cnt[a] > cnt[b] : a < b;
-      });
-      order.resize((size_t)H);
-      std::sort(order.begin(), order.end());
-      long long covered = 0;
-      for (int c : order)
-            covered += cnt[c];
-      sp.hot_coverage = (double)covered / (double)nnz;
-      if (sp.hot_coverage < 0.10)
-            return 0;
-      std::vector<int> hot_idx((size_t)N, -1);
-      for (int i = 0; i < H; ++i)
-            hot_idx[order[i]] = i;
-      int *d_idx = nullptr;
-      int rc = upload(&d_idx, hot_idx);
-      rc = rc ? rc : upload(&sp.d_hot_cols, order);
-      if (!rc && cudaMalloc(&sp.d_xhot, (size_t)H * sizeof(double)) != cudaSuccess)
-            rc = fail(-ENOMEM, "hot-column table: out of device memory");
-      if (!rc) {
-            sell_mark_hot_kernel<<<1184, 256>>>(sp.d_ja, sp.slots, d_idx);
-            e = cudaDeviceSynchronize();
-            if (e != cudaSuccess)
-                  rc = fail(-EIO, "hot-column marking failed: %s", cudaGetErrorString(e));
-      }
-      cudaFree(d_idx);
-      if (rc) {
-            cudaFree(sp.d_hot_cols), cudaFree(sp.d_xhot);
-            sp.d_hot_cols = nullptr, sp.d_xhot = nullptr;
-            return rc;
-      }
-      sp.n_hot = H;
-      g_counters.launches += 2;
-      return 0;
-}
-
 template <typename Src>
 int sell_build_vrows(const Src &src, const std::vector<long long> &irp, long long M, long long N,
                      int chunk, SellPlan &sp) {
@@ -755,83 +696,21 @@ int sell_build_vrows(const Src &src, const std::vector<long long> &irp, long lon
       if (rc)
             return rc;
       sp.state = 1;
-      if (g_knobs.sell_hot > 0 && sell_pick_hot_columns(src.ja, irp[M], N, sp))
-            cudaGetLastError(); // the table is an optimisation: without it the plain kernel runs
       return 0;
 }
 
 // y = A x through the panels: panel 0 stores, later panels accumulate (stream order).
-template <int EPI, int U, int THREADS, int MIN_CTAS, int MODE>
-int launch_sell_hot(const SellPlan &sp, const double *d_x, double *d_y, const EpiArgs &epi, cudaStream_t st) {
-      auto kern = sell_hot_kernel<EPI, U, THREADS, MIN_CTAS, MODE>;
-      if (MODE == HOT_L1) { // one slice per warp; the table is a global array the L1 keeps
-            hot_gather_kernel<<<blocks_for(sp.n_hot, 256), 256, 0, st>>>(d_x, sp.d_hot_cols, sp.n_hot, sp.d_xhot);
-            ++g_counters.launches;
-            kern<<<blocks_for(sp.n_slices * 32, THREADS), THREADS, 0, st>>>(
-                sp.d_soff, sp.d_perm, sp.d_ja, sp.d_as, sp.n_slices, d_x, d_y, sp.d_partial, sp.d_hot_cols,
-                sp.d_xhot, sp.n_hot, epi);
-            return 0;
-      }
-      const size_t smem = (size_t)sp.n_hot * sizeof(double);
-      static int occ_by_dev[kMaxDevices] = {0};
-      static size_t smem_set[kMaxDevices] = {0};
-      int dev = 0;
-      cudaGetDevice(&dev);
-      int &occ = occ_by_dev[dev % kMaxDevices];
-      if (!occ || smem_set[dev % kMaxDevices] != smem) {
-            B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, THREADS, smem));
-            smem_set[dev % kMaxDevices] = smem;
-            if (occ < 1)
-                  return fail(-EINVAL, "hot-column kernel does not fit on an SM (%zu bytes)", smem);
-      }
-      const int grid = (int)std::min<long long>(blocks_for(sp.n_slices * 32, THREADS), (long long)occ * g_sm_count);
-      kern<<<grid, THREADS, smem, st>>>(sp.d_soff, sp.d_perm, sp.d_ja, sp.d_as, sp.n_slices, d_x, d_y,
-                                        sp.d_partial, sp.d_hot_cols, sp.d_xhot, sp.n_hot, epi);
-      return 0;
-}
-
-template <int EPI>
-int launch_sell_hot_any(const SellPlan &sp, const double *d_x, double *d_y, const EpiArgs &epi, cudaStream_t st) {
-      const bool u8 = g_knobs.sell_unroll == 8;
-      if (g_knobs.sell_hot_mode == 1) // 48 warps x 4 or 32 warps x 8 gathers in flight per SM
-            return u8 ? launch_sell_hot<EPI, 8, 512, 2, HOT_L1>(sp, d_x, d_y, epi, st)
-                      : launch_sell_hot<EPI, 4, 512, 3, HOT_L1>(sp, d_x, d_y, epi, st);
-      // two CTAs of 768 threads per SM (42 registers) while two tables fit, else one of 1 024 with
-      // twice the loads in flight per lane
-      const bool two = 2 * ((size_t)sp.n_hot * sizeof(double) + 1024) <= 227u * 1024 && !u8;
-      return two ? launch_sell_hot<EPI, 4, 768, 2, HOT_SMEM>(sp, d_x, d_y, epi, st)
-                 : launch_sell_hot<EPI, 8, 1024, 1, HOT_SMEM>(sp, d_x, d_y, epi, st);
-}
-
 int sell_run(const SellPlan &sp, int wpb, const double *d_x, double *d_y, int epi_mode,
              const EpiArgs &epi, cudaStream_t st, int blocks = 0,
              const std::function<void(long long, long long)> *block_done = nullptr) {
       const int threads = 32 * wpb;
       const int grid = blocks_for(sp.n_slices * 32, threads);
-      const bool u8 = g_knobs.sell_unroll == 8;
-      if (sp.chunk > 0 && sp.n_hot > 0) { // hot columns from a compact table (the index array holds their codes)
-            int rc = epi_mode == EPI_FUSED ? launch_sell_hot_any<EPI_FUSED>(sp, d_x, d_y, epi, st)
-                                           : launch_sell_hot_any<EPI_PLAIN>(sp, d_x, d_y, epi, st);
-            if (rc)
-                  return rc;
-            ++g_counters.launches;
-            if (sp.n_split_rows) {
-                  csr_combine_kernel<EPI_PLAIN><<<blocks_for(sp.n_split_rows, 128), 128, 0, st>>>(
-                      sp.d_split_row, sp.d_split_first, (int)sp.n_split_rows, sp.d_partial, d_y, EpiArgs{});
-                  ++g_counters.launches;
-            }
-            return 0;
-      }
       if (sp.chunk > 0) { // virtual rows: one panel, pieces of split rows go to partial sums
             if (epi_mode == EPI_FUSED)
-                  sell_kernel<EPI_FUSED, 4, true><<<grid, threads, 0, st>>>(
-                      sp.d_soff, sp.d_perm, sp.d_ja, sp.d_as, sp.n_slices, d_x, d_y, sp.d_partial, epi);
-            else if (u8)
-                  sell_kernel<EPI_PLAIN, 8, true><<<grid, threads, 0, st>>>(
+                  sell_kernel<EPI_FUSED, true><<<grid, threads, 0, st>>>(
                       sp.d_soff, sp.d_perm, sp.d_ja, sp.d_as, sp.n_slices, d_x, d_y, sp.d_partial, epi);
             else
-                  sell_kernel<EPI_PLAIN, 4, true><<<grid, threads, 0, st>>>(
+                  sell_kernel<EPI_PLAIN, true><<<grid, threads, 0, st>>>(
                       sp.d_soff, sp.d_perm, sp.d_ja, sp.d_as, sp.n_slices, d_x, d_y, sp.d_partial, epi);
             ++g_counters.launches;
             if (sp.n_split_rows) {
@@ -859,22 +738,18 @@ int sell_run(const SellPlan &sp, int wpb, const double *d_x, double *d_y, int ep
             const long long ns = s1 - s0;
             const int grid = blocks_for(ns * 32, threads);
             const bool push = epi_mode == EPI_PUSH && last; // finished sums also go to the peers
-#define SELL_LAUNCH(E, U)                                                                          \
-      sell_kernel<E, U><<<grid, threads, 0, st>>>(soff, perm, sp.d_ja, sp.d_as, ns, d_x, d_y, nullptr, epi)
+#define SELL_LAUNCH(E)                                                                             \
+      sell_kernel<E><<<grid, threads, 0, st>>>(soff, perm, sp.d_ja, sp.d_as, ns, d_x, d_y, nullptr, epi)
             if (push && p > 0)
-                  SELL_LAUNCH(EPI_ACC_PUSH, 4);
+                  SELL_LAUNCH(EPI_ACC_PUSH);
             else if (push)
-                  SELL_LAUNCH(EPI_PUSH, 4);
-            else if (p > 0 && u8)
-                  SELL_LAUNCH(EPI_ACC, 8);
+                  SELL_LAUNCH(EPI_PUSH);
             else if (p > 0)
-                  SELL_LAUNCH(EPI_ACC, 4);
+                  SELL_LAUNCH(EPI_ACC);
             else if (epi_mode == EPI_FUSED)
-                  SELL_LAUNCH(EPI_FUSED, 4);
-            else if (u8)
-                  SELL_LAUNCH(EPI_PLAIN, 8);
+                  SELL_LAUNCH(EPI_FUSED);
             else
-                  SELL_LAUNCH(EPI_PLAIN, 4);
+                  SELL_LAUNCH(EPI_PLAIN);
 #undef SELL_LAUNCH
             ++g_counters.launches;
             if (last && block_done && blocks)
@@ -885,7 +760,7 @@ int sell_run(const SellPlan &sp, int wpb, const double *d_x, double *d_y, int ep
 
 // Should ids 2 / 4 of this CSR go through SELL-P?  (whole-matrix calls on single-segment handles)
 bool csr_wants_sell(spmv_b200_csr *h) {
-      if (g_knobs.sell == 0 || g_knobs.adaptive_direct || h->segs.size() != 1 || h->M < 64)
+      if (g_knobs.sell == 0 || h->segs.size() != 1 || h->M < 64)
             return false;
       if (g_knobs.sell == 1)
             return true;
@@ -1003,7 +878,7 @@ static int run_kernel(spmv_b200_csr *h, int kernel, int wpb, Segment &sg, const 
             // through the TMA-staged tile kernel, which also bins its own long rows; an
             // irregular one goes through the direct binned kernels (whole irregular matrices
             // never get here: csr_run routes them to the sorted slices of SELL-P).
-            if (a.epi_mode != EPI_FUSED && (!sg.regular || g_knobs.adaptive_direct)) {
+            if (a.epi_mode != EPI_FUSED && !sg.regular) {
                   int rc = build_bin_lists(h, sg);
                   if (rc)
                         return rc;
@@ -1462,10 +1337,10 @@ extern "C" int spmv_b200_csr_sell_info(spmv_b200_csr *h, int build, int64_t *out
       if (build && h->sell.state == 0 && h->segs.size() == 1)
             csr_ensure_sell(h);
       const SellPlan &sp = h->sell;
-      const int64_t v[13] = {sp.state, sp.K, sp.sigma, sp.n_slices, sp.slots, sp.nnz_in_slices,
+      const int64_t v[11] = {sp.state, sp.K, sp.sigma, sp.n_slices, sp.slots, sp.nnz_in_slices,
                              sp.n_long, (int64_t)(h->gather_span * 1e6), sp.chunk, sp.n_split_rows,
-                             sp.n_partials, sp.n_hot, (int64_t)(sp.hot_coverage * 1e6)};
-      for (int i = 0; i < n_out && i < 13; ++i)
+                             sp.n_partials};
+      for (int i = 0; i < n_out && i < 11; ++i)
             out[i] = v[i];
       return 0;
 }
@@ -1617,8 +1492,6 @@ int csr_spmm_k(spmv_b200_csr *h, const double *X, double *Y, cudaStream_t st) {
                   }
                   return 0;
             }
-            if (sp.n_hot > 0)
-                  return fail(-ENOTSUP, "SpMM: not available with the hot-column table (sell_hot knob)");
             for (int p = 0; p < sp.K; ++p) {
                   const long long *soff = sp.d_soff + (size_t)p * (sp.n_slices + 1);
                   const int *perm = sp.d_perm + (size_t)p * sp.n_slices * 32;
@@ -1687,8 +1560,7 @@ extern "C" int spmv_b200_csr_launches(const spmv_b200_csr *h, int kernel) {
             if (sg.r1 == sg.r0)
                   continue;
             const bool streamed = kernel == SPMV_B200_CSR_STREAM ||
-                                  (kernel == SPMV_B200_CSR_ADAPTIVE && sg.regular &&
-                                   !g_knobs.adaptive_direct);
+                                  (kernel == SPMV_B200_CSR_ADAPTIVE && sg.regular);
             if (streamed) {
                   n += 1;
                   for (auto &kv : sg.stream) {
@@ -1879,8 +1751,8 @@ int hll_run_range(spmv_b200_hll *h, int kernel, int wpb, long long hack0, long l
       switch (kernel) {
       case SPMV_B200_HLL_THREAD_ROW_RM:
       case SPMV_B200_HLL_THREAD_ROW:
-            hll_warp_kernel<1, EPI_PLAIN><<<grid, threads, 0, st>>>(h->d_hoff, h->d_ja, h->d_as, hack0,
-                                                                    hack1, h->M, d_x, d_y, epi);
+            hll_warp_kernel<EPI_PLAIN><<<grid, threads, 0, st>>>(h->d_hoff, h->d_ja, h->d_as, hack0,
+                                                                 hack1, h->M, d_x, d_y, epi);
             break;
       case SPMV_B200_HLL_WARP_HACK: {
             // x larger than the L2 and scattered columns: column panels (sell_kernels.cuh); the
@@ -1892,12 +1764,10 @@ int hll_run_range(spmv_b200_hll *h, int kernel, int wpb, long long hack0, long l
                   break;
             }
             // Measured (profiles/r1_kbench_c2_sweep.txt): lane = row with 64/32-bit loads wins
-            // whenever the gather is cache friendly (C2: 99 % vs 97 % / 88 % for the 256/128-bit
-            // and 128/64-bit variants, whose lanes share rows and split their gathers); the wide
-            // variants stay selectable with the hll_vec knob.
-            const int vec = g_knobs.hll_vec;
+            // whenever the gather is cache friendly (C2: 99 % vs 97 % / 88 % for 256/128-bit and
+            // 128/64-bit loads, whose lanes share rows and split their gathers).
             // narrow hacks: persistent warps, each with its own ring of bulk-copied hacks (hll_pipe_kernel)
-            if (vec <= 1 && g_knobs.hll_pipe != 0 && h->max_width > 0 && h->max_width <= kHllPipeMaxWidth &&
+            if (g_knobs.hll_pipe != 0 && h->max_width > 0 && h->max_width <= kHllPipeMaxWidth &&
                 (g_knobs.hll_pipe > 0 || n >= 4ll * g_sm_count * 8)) {
                   constexpr int kStages = 2, kWarps = 8;
                   const int capw = 32 * h->max_width; // 3.8 KB per warp for width 5: 48 warps per SM
@@ -1930,16 +1800,10 @@ int hll_run_range(spmv_b200_hll *h, int kernel, int wpb, long long hack0, long l
                   break;
             }
             if (epi_mode == EPI_FUSED)
-                  hll_warp_kernel<1, EPI_FUSED><<<grid, threads, 0, st>>>(
-                      h->d_hoff, h->d_ja, h->d_as, hack0, hack1, h->M, d_x, d_y, epi);
-            else if (vec == 2)
-                  hll_warp_kernel<2, EPI_PLAIN><<<grid, threads, 0, st>>>(
-                      h->d_hoff, h->d_ja, h->d_as, hack0, hack1, h->M, d_x, d_y, epi);
-            else if (vec == 4)
-                  hll_warp_kernel<4, EPI_PLAIN><<<grid, threads, 0, st>>>(
+                  hll_warp_kernel<EPI_FUSED><<<grid, threads, 0, st>>>(
                       h->d_hoff, h->d_ja, h->d_as, hack0, hack1, h->M, d_x, d_y, epi);
             else
-                  hll_warp_kernel<1, EPI_PLAIN><<<grid, threads, 0, st>>>(
+                  hll_warp_kernel<EPI_PLAIN><<<grid, threads, 0, st>>>(
                       h->d_hoff, h->d_ja, h->d_as, hack0, hack1, h->M, d_x, d_y, epi);
             break;
       }
@@ -2344,23 +2208,17 @@ extern "C" int spmv_b200_set_knob(const char *key, int value) {
             const char *name;
             int *slot;
       } table[] = {{"csr_stream_cfg", &g_knobs.csr_stream_cfg},
-                   {"hll_vec", &g_knobs.hll_vec},
                    {"hll_pipe", &g_knobs.hll_pipe},
                    {"csr_pipe", &g_knobs.csr_pipe},
                    {"hll_stream_cfg", &g_knobs.hll_stream_cfg},
-                   {"regular_lpr", &g_knobs.regular_lpr},
                    {"force_wide", &g_knobs.force_wide},
-                   {"adaptive_direct", &g_knobs.adaptive_direct},
                    {"pipeline", &g_knobs.pipeline},
                    {"pipe_chunks", &g_knobs.pipe_chunks},
                    {"sell", &g_knobs.sell},
                    {"sell_panels", &g_knobs.sell_panels},
                    {"sell_sigma", &g_knobs.sell_sigma},
                    {"sell_panel_mb", &g_knobs.sell_panel_mb},
-                   {"sell_unroll", &g_knobs.sell_unroll},
                    {"sell_chunk", &g_knobs.sell_chunk},
-                   {"sell_hot", &g_knobs.sell_hot},
-                   {"sell_hot_mode", &g_knobs.sell_hot_mode},
                    {"sell_max_row", &g_knobs.sell_max_row},
                    {"cache", &g_knobs.cache}};
       for (auto &t : table)
@@ -2368,12 +2226,5 @@ extern "C" int spmv_b200_set_knob(const char *key, int value) {
                   *t.slot = value;
                   return 0;
             }
-      if (!strcmp(key, "l2_fetch_granularity")) {
-            // device-wide hint: bytes fetched from HBM on an L2 miss (32, 64 or 128)
-            if (ensure_device())
-                  return -ENODEV;
-            B200_CUDA(cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)value));
-            return 0;
-      }
       return fail(-EINVAL, "unknown knob %s", key);
 }

@@ -310,51 +310,6 @@ def test_sell_virtual_rows_bit_exact_and_parity(sp, O, torch, name):
         sp.set_knob("sell_sigma", 16384)
 
 
-def test_sell_hot_column_table(sp, O, torch):
-    """Power-law matrices: the most referenced columns are served from shared memory (codes ~i in
-    the slices' index array).  Same y within tolerance for several table sizes and both unroll
-    depths; a matrix with uniform columns gets no table (it would serve < 10 % of the gathers)."""
-    A = sp.gen_rmat(15, 16)
-    IRP, JA, AS = A.IRP.copy(), A.JA.copy(), A.AS.copy()
-    x = np.random.default_rng(9).uniform(-1, 1, A.N)
-    y_ref = O.csr_spmv(A.M, IRP, JA, AS, x)
-    bound = O.csr_abs_bound(A.M, IRP, JA, AS, x)
-    xd = dev(torch, x)
-    y = torch.zeros(A.M, dtype=torch.float64, device="cuda")
-    try:
-        for hot in (64, 1000, 12288, 24576):
-            sp.set_knob("sell_hot", hot)
-            h = sp.CsrDevice.from_host(A)
-            info = h.sell_info(build=True)
-            assert info["state"] == 1 and info["hot_columns"] == min(hot, 28000) and info["hot_coverage_ppm"] > 100000
-            _, _, ja, _ = h.sell_download()
-            cnt = np.bincount(JA, minlength=A.N)
-            top = np.sort(cnt)[::-1][:info["hot_columns"]].sum() / A.NZ
-            assert abs(info["hot_coverage_ppm"] * 1e-6 - top) < 1e-6
-            assert (ja < 0).any() and ja.min() >= -info["hot_columns"]
-            for mode in (0, 1):                   # table in shared memory / compact global array kept in the L1
-                sp.set_knob("sell_hot_mode", mode)
-                for unroll in (4, 8):
-                    sp.set_knob("sell_unroll", unroll)
-                    y.fill_(float("nan"))
-                    h.spmv(xd, y, kernel=2, warps_per_block=4)
-                    ok, worst = O.check_tolerance(y.cpu().numpy(), y_ref, bound, TOL)
-                    assert ok, (hot, mode, unroll, worst)
-            h.close()
-        U = sp.gen_ragged(5000, 300)             # banded, no hub columns
-        sp.set_knob("sell_hot", 64)
-        sp.set_knob("sell", 1)
-        h = sp.CsrDevice.from_host(U)
-        info = h.sell_info(build=True)
-        assert info["chunk"] > 0 and info["hot_columns"] == 0
-        h.close()
-    finally:
-        sp.set_knob("sell", -1)
-        sp.set_knob("sell_hot", 0)
-        sp.set_knob("sell_hot_mode", 0)
-        sp.set_knob("sell_unroll", 4)
-
-
 def test_sell_auto_routing(sp, O, torch):
     """Who goes through SELL-P without a knob: ragged / power-law CSR (one panel while x fits
     the L2); regular rows stay on the staged kernel; and the host half of the plan (row order and

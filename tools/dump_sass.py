@@ -10,10 +10,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 rnd = sys.argv[1] if len(sys.argv) > 1 else "r1"
 WANT = [r"csr_stream_kernelILi512ELi4ELi2ELi4096ELi1ELb1ELb0ELi0EiE",   # C2 / C5 headline: row-wise staged tiles, plain epilogue
         r"csr_stream_kernelILi512ELi4ELi2ELi4096ELi1ELb1ELb0ELi1ExE",   # ... push epilogue, 64-bit offsets (C5 boundary rows)
-        r"hll_warp_kernelILi1ELi0EE",                                    # HLL headline (C2)
+        r"hll_warp_kernelILi0EE",                                        # HLL headline (C2)
         r"hll_pipe_kernelILi2ELi0EE", r"csr_pipe_kernelILi2ELi176EiE",   # short rows (C1): per-warp bulk-copy rings
-        r"sell_kernelILi0ELi4ELb0EE", r"sell_kernelILi2ELi4ELb0EE",      # C3 column panels: first / later panels
-        r"sell_kernelILi0ELi4ELb1EE",                                    # C4 virtual rows
+        r"sell_kernelILi0ELb0EE", r"sell_kernelILi2ELb0EE",              # C3 column panels: first / later panels
+        r"sell_kernelILi0ELb1EE",                                        # C4 virtual rows
         r"sell_mm_kernelILi2ELi0ELb1EE"]                                 # SpMM, 2 right-hand sides, virtual rows
 txt = subprocess.run(["cuobjdump", "-sass", os.path.join(ROOT, "spmv_scpa_b200/lib/libspmv_b200.so")],
                      capture_output=True, text=True).stdout

@@ -28,7 +28,6 @@ static int g_reps = 20, g_warmup = 3, g_flush = 0, g_quick = 0, g_profile = 0, g
 static int g_sell = 0, g_spmm = 0;
 static int g_panels[16] = {1, 2, 3, 4, 6, 8, 16}, g_n_panels = 7;
 static int g_chunks[16], g_n_chunks = 0, g_auto = 0;
-static int g_hots[16] = {0}, g_n_hots = 1;
 static double g_peak = 6559.7; /* MEASURED_PEAKS.json hbm_gbs of this pool */
 static const char *g_only = "";
 
@@ -162,11 +161,7 @@ int main(int argc, char **argv) {
                   g_spmm = 1; /* SpMM: 1 (id 2), 2 and 4 right-hand sides in one pass */
             else if (!strcmp(argv[i], "--auto"))
                   g_auto = 1; /* only what the library picks on its own: CSR id 2, HLL id 2 (ncu captures) */
-            else if (!strcmp(argv[i], "--hot") && i + 1 < argc) {
-                  g_n_hots = 0;
-                  for (char *tok = strtok(argv[++i], ","); tok && g_n_hots < 16; tok = strtok(NULL, ","))
-                        g_hots[g_n_hots++] = atoi(tok);
-            } else if (!strcmp(argv[i], "--chunks") && i + 1 < argc) {
+            else if (!strcmp(argv[i], "--chunks") && i + 1 < argc) {
                   for (char *tok = strtok(argv[++i], ","); tok && g_n_chunks < 16; tok = strtok(NULL, ","))
                         g_chunks[g_n_chunks++] = atoi(tok);
             } else if (!strcmp(argv[i], "--panels") && i + 1 < argc) {
@@ -304,36 +299,23 @@ int main(int argc, char **argv) {
       }
 
       if (g_n_chunks) {
-            /* ragged matrices: virtual-row chunk size x unroll x warps/block */
-            int64_t info[13];
-            for (int ic = 0; ic < g_n_chunks * g_n_hots; ++ic) {
-                  const int hot = g_hots[ic / g_n_chunks];
-                  spmv_b200_set_knob("sell_hot", hot);
-                  spmv_b200_set_knob("sell_chunk", g_chunks[ic % g_n_chunks]);
+            /* ragged matrices: virtual-row chunk size x warps/block */
+            int64_t info[11];
+            for (int ic = 0; ic < g_n_chunks; ++ic) {
+                  spmv_b200_set_knob("sell_chunk", g_chunks[ic]);
                   spmv_b200_csr *h = spmv_b200_csr_create(A);
-                  if (!h || spmv_b200_csr_sell_info(h, 1, info, 13) || info[0] != 1) {
-                        printf("CSR  sell chunk=%d BUILD FAILED: %s\n", g_chunks[ic % g_n_chunks], spmv_b200_last_error());
+                  if (!h || spmv_b200_csr_sell_info(h, 1, info, 11) || info[0] != 1) {
+                        printf("CSR  sell chunk=%d BUILD FAILED: %s\n", g_chunks[ic], spmv_b200_last_error());
                         spmv_b200_csr_destroy(h);
                         continue;
                   }
-                  /* hot table: both homes (0 shared memory, persistent CTAs: warps/block is
-                   * ignored; 1 compact global array kept in the L1) */
-                  for (int mode = 0; mode < (info[11] ? 2 : 1); ++mode)
-                        for (int u = 4; u <= 8; u += 4) {
-                              spmv_b200_set_knob("sell_hot_mode", mode);
-                              spmv_b200_set_knob("sell_unroll", u);
-                              snprintf(knob, sizeof knob, "C=%d U=%d pad=%.1f%% H=%lld(%.0f%%)%s", g_chunks[ic % g_n_chunks], u,
-                                       info[5] ? 100.0 * (info[4] - (double)info[5]) / info[5] : 0.0,
-                                       (long long)info[11], info[12] * 1e-4, !info[11] ? "" : mode ? " L1" : " smem");
-                              for (int w = (info[11] && !mode) ? 3 : 1; w < 4; ++w)
-                                    run_csr(&c, h, 2, wpbs[w], knob);
-                        }
+                  snprintf(knob, sizeof knob, "C=%d pad=%.1f%%", g_chunks[ic],
+                           info[5] ? 100.0 * (info[4] - (double)info[5]) / info[5] : 0.0);
+                  for (int w = 1; w < 4; ++w)
+                        run_csr(&c, h, 2, wpbs[w], knob);
                   spmv_b200_csr_destroy(h);
             }
-            spmv_b200_set_knob("sell_unroll", 4);
             spmv_b200_set_knob("sell_chunk", 256);
-            spmv_b200_set_knob("sell_hot", 0);
-            spmv_b200_set_knob("sell_hot_mode", 0);
             return 0;
       }
 
@@ -397,11 +379,6 @@ int main(int argc, char **argv) {
                         else
                               snprintf(knob, sizeof knob, "K=%d", panels[ip]);
                         run_hll(&c, hh, 2, 8, knob);
-                        if (ip < 0) {
-                              spmv_b200_set_knob("hll_vec", 4);
-                              run_hll(&c, hh, 2, 16, "sell=0 vec=4");
-                              spmv_b200_set_knob("hll_vec", -1);
-                        }
                         spmv_b200_hll_destroy(hh);
                   }
                   spmv_b200_csr_destroy(hc);
@@ -418,20 +395,12 @@ int main(int argc, char **argv) {
                   return 1;
             }
             run_csr(&c, h, 4, 4, "auto");
-            spmv_b200_set_knob("adaptive_direct", 1);
-            run_csr(&c, h, 2, 4, "direct-binned");
-            spmv_b200_set_knob("adaptive_direct", 0);
             if (strcmp(g_only, "csr")) {
                   spmv_b200_hll *hh = spmv_b200_hll_from_csr(h);
                   if (!hh) {
                         fprintf(stderr, "kbench: %s\n", spmv_b200_last_error());
                         return 1;
                   }
-                  spmv_b200_set_knob("hll_vec", 1);
-                  run_hll(&c, hh, 2, 4, "vec=1");
-                  spmv_b200_set_knob("hll_vec", 4);
-                  run_hll(&c, hh, 2, 4, "vec=4");
-                  spmv_b200_set_knob("hll_vec", -1);
                   run_hll(&c, hh, 2, 16, "auto");
                   run_hll(&c, hh, 3, 8, "auto");
                   spmv_b200_hll_destroy(hh);
@@ -466,10 +435,6 @@ int main(int argc, char **argv) {
             spmv_b200_set_knob("csr_pipe", 1);
             run_csr(&c, h, 2, 4, "pipe=1");
             spmv_b200_set_knob("csr_pipe", -1);
-            spmv_b200_set_knob("adaptive_direct", 1);
-            for (int w = 0; w < 3; ++w)
-                  run_csr(&c, h, 2, wpbs[w], "direct-binned");
-            spmv_b200_set_knob("adaptive_direct", 0);
             for (int w = 0; w < 3; ++w)
                   run_csr(&c, h, 4, wpbs[w], "auto");
             static const int cfgs[] = {10, 12, 13, 24, 25, 26, 33};
@@ -484,20 +449,6 @@ int main(int argc, char **argv) {
             spmv_b200_set_knob("sell", -1);
             spmv_b200_set_knob("csr_stream_cfg", -1);
             spmv_b200_csr_destroy(h);
-            if (!g_quick) {
-                  /* forced lanes-per-row of the regular base launch */
-                  spmv_b200_set_knob("adaptive_direct", 1);
-                  for (int lg = 0; lg <= 5; ++lg) {
-                        spmv_b200_set_knob("regular_lpr", lg);
-                        h = spmv_b200_csr_create(A);
-                        snprintf(knob, sizeof knob, "lanes/row=%d", 1 << lg);
-                        run_csr(&c, h, 2, 8, knob);
-                        run_csr(&c, h, 2, 4, knob);
-                        spmv_b200_csr_destroy(h);
-                  }
-                  spmv_b200_set_knob("regular_lpr", -1);
-                  spmv_b200_set_knob("adaptive_direct", 0);
-            }
       }
 
       if (strcmp(g_only, "csr")) {
@@ -515,13 +466,8 @@ int main(int argc, char **argv) {
             for (int w = 0; w < 4; ++w)
                   run_hll(&c, hh, 1, wpbs[w], "-");
             spmv_b200_set_knob("hll_pipe", 0); /* warp per hack, whatever the width */
-            for (int v = 1; v <= 4; v *= 2) {
-                  spmv_b200_set_knob("hll_vec", v);
-                  snprintf(knob, sizeof knob, "vec=%d", v);
-                  for (int w = 0; w < 4; ++w)
-                        run_hll(&c, hh, 2, wpbs[w], knob);
-            }
-            spmv_b200_set_knob("hll_vec", -1);
+            for (int w = 0; w < 4; ++w)
+                  run_hll(&c, hh, 2, wpbs[w], "pipe=0");
             /* narrow hacks: persistent warps with private bulk-copy rings (what id 2 picks for them) */
             spmv_b200_set_knob("hll_pipe", -1);
             run_hll(&c, hh, 2, 4, "pipe=auto");
