@@ -123,6 +123,13 @@ spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, int z0,
                                            int64_t n_local,
                                            const int64_t *cuts, int n_cuts);
 
+/* Aᵀ of a resident CSR as a new resident CSR, built on A's device: row j lists column j of A in
+ * increasing row order (entries of one row with equal columns keep their order; values are copied,
+ * never summed).  A shard transposes its local block (n_local rows, M columns, col_offset 0, no
+ * cuts).  Synchronous; A is unchanged; destroy both handles separately.  NULL + last_error on
+ * failure; -ENOTSUP for 2^31 or more entries. */
+spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A);
+
 int64_t spmv_b200_csr_rows(const spmv_b200_csr *h);
 int64_t spmv_b200_csr_cols(const spmv_b200_csr *h);
 int64_t spmv_b200_csr_nnz(const spmv_b200_csr *h);

@@ -496,6 +496,12 @@ class CsrDevice:
     def to_hll(self):
         return HllDevice(L.b200.spmv_b200_hll_from_csr(self._h))
 
+    def transpose(self):
+        """Aᵀ as a new resident CSR built on the GPU (spmv_b200_csr_transpose): row j lists column j
+        of A in increasing row order, duplicates kept.  A shard gives the transpose of its local
+        block.  Both handles are independent."""
+        return CsrDevice(L.b200.spmv_b200_csr_transpose(self._h))
+
     def close(self):
         if self._h:
             L.b200.spmv_b200_csr_destroy(self._h)

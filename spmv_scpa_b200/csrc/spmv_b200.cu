@@ -8,10 +8,13 @@
 // fails loudly.
 #include "internal.cuh"
 
+#include <cub/cub.cuh>
+
 #include "csr_kernels.cuh"
 #include "gen_kernels.cuh"
 #include "hll_kernels.cuh"
 #include "sell_kernels.cuh"
+#include "transpose_kernels.cuh"
 
 using namespace b200;
 
@@ -1279,6 +1282,121 @@ extern "C" spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, in
             return nullptr;
       }
       csr_measure_span(h);
+      return h;
+}
+
+// A^T on the current device.  Memory while the sort runs, besides A and the new handle:
+//   sort keys   the two key buffers of the radix sort live in the new handle's value array
+//               (8 bytes per entry = two int32 arrays), which the fill overwrites afterwards;
+//   sort values one buffer is the new handle's column array, the other is temporary (4 B/entry);
+//   row_of      row of every entry of A (temporary, 4 B/entry);
+//   count       entries per column of A (temporary, 4 B per column + 4);
+//   scratch     CUB's temporary storage (histograms and tile state, independent of the entry count
+//               up to a few bytes per tile).
+// Peak temporary memory is therefore 8 bytes per entry + 4 bytes per column + CUB's scratch.
+template <typename InOffT, typename OutOffT>
+static int csr_transpose_fill(const spmv_b200_csr *A, spmv_b200_csr *h) {
+      const long long NZ = A->NZ, NT = A->N; // NT: rows of A^T
+      int *d_count = nullptr, *d_row_of = nullptr, *d_idx = nullptr;
+      void *d_scratch = nullptr;
+      size_t scan_bytes = 0, sort_bytes = 0;
+      int *key0 = reinterpret_cast<int *>(h->d_as);
+      int *key1 = key0 + ((NZ + 3) & ~3ll); // 16-byte aligned second half of the value array
+      cub::DoubleBuffer<int> keys(key0, key1), vals(nullptr, h->d_ja);
+      int end_bit = 1; // column bits that can be non-zero
+      while (end_bit < 31 && (1ll << end_bit) < NT)
+            ++end_bit;
+      OutOffT *t_irp = static_cast<OutOffT *>(h->d_irp);
+      cudaError_t e = cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_count, t_irp, (int)(NT + 1));
+      if (e == cudaSuccess && NZ > 0)
+            e = cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
+      if (e != cudaSuccess)
+            return fail(-EIO, "transpose: CUB size query failed: %s", cudaGetErrorString(e));
+      const size_t scratch_bytes = std::max(scan_bytes, sort_bytes);
+      if (cudaMalloc(&d_count, (size_t)(NT + 1) * sizeof(int)) != cudaSuccess ||
+          cudaMalloc(&d_scratch, std::max<size_t>(scratch_bytes, 1)) != cudaSuccess ||
+          (NZ > 0 && (cudaMalloc(&d_row_of, (size_t)NZ * sizeof(int)) != cudaSuccess ||
+                      cudaMalloc(&d_idx, (size_t)NZ * sizeof(int)) != cudaSuccess))) {
+            cudaGetLastError(); // clear the allocation error
+            cudaFree(d_count), cudaFree(d_scratch), cudaFree(d_row_of), cudaFree(d_idx);
+            return fail(-ENOMEM, "transpose: cudaMalloc of %lld bytes of temporaries failed",
+                        (long long)((NT + 1) * 4 + NZ * 8 + (long long)scratch_bytes));
+      }
+      e = cudaMemsetAsync(d_count, 0, (size_t)(NT + 1) * sizeof(int));
+      if (e == cudaSuccess && NZ > 0) {
+            const int grid = (int)std::min<long long>(blocks_for(A->M * 32, 256), 65535ll * 8);
+            transpose_prep_kernel<InOffT><<<grid, 256>>>(static_cast<const InOffT *>(A->d_irp), A->d_ja,
+                                                         A->M, d_row_of, key0, d_idx, d_count);
+            ++g_counters.launches;
+            e = cudaGetLastError();
+      }
+      if (e == cudaSuccess)
+            e = cub::DeviceScan::ExclusiveSum(d_scratch, scan_bytes, d_count, t_irp, (int)(NT + 1));
+      if (e == cudaSuccess && NZ > 0) {
+            vals = cub::DoubleBuffer<int>(d_idx, h->d_ja);
+            e = cub::DeviceRadixSort::SortPairs(d_scratch, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
+      }
+      if (e == cudaSuccess && NZ > 0) {
+            const int grid = (int)std::min<long long>(blocks_for(NZ, 256), (long long)g_sm_count * 64);
+            transpose_fill_kernel<<<grid, 256>>>(vals.Current(), d_row_of, A->d_as, NZ, h->d_ja, h->d_as);
+            ++g_counters.launches;
+            e = cudaGetLastError();
+      }
+      // the second key buffer may have reached into the 16 zero entries after the values
+      if (e == cudaSuccess)
+            e = cudaMemsetAsync(h->d_as + NZ, 0, 16 * sizeof(double));
+      if (e == cudaSuccess)
+            e = cudaDeviceSynchronize();
+      cudaFree(d_count), cudaFree(d_scratch), cudaFree(d_row_of), cudaFree(d_idx);
+      if (e != cudaSuccess)
+            return fail(-EIO, "transpose failed: %s", cudaGetErrorString(e));
+      // planning needs the row offsets on the host
+      h->h_irp.resize((size_t)NT + 1);
+      std::vector<OutOffT> tmp((size_t)NT + 1);
+      e = cudaMemcpy(tmp.data(), t_irp, (size_t)(NT + 1) * sizeof(OutOffT), cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess)
+            return fail(-EIO, "transpose: row offsets download failed: %s", cudaGetErrorString(e));
+      std::copy(tmp.begin(), tmp.end(), h->h_irp.begin());
+      return 0;
+}
+
+static spmv_b200_csr *csr_transpose_here(const spmv_b200_csr *A) {
+      spmv_b200_csr *h = csr_alloc_shell(A->N, A->M, A->NZ, 0);
+      if (!h)
+            return nullptr;
+      int rc;
+      if (A->wide)
+            rc = h->wide ? csr_transpose_fill<long long, long long>(A, h)
+                         : csr_transpose_fill<long long, int>(A, h);
+      else
+            rc = h->wide ? csr_transpose_fill<int, long long>(A, h) : csr_transpose_fill<int, int>(A, h);
+      if (rc || finish_create(h, nullptr, 0)) {
+            spmv_b200_csr_destroy(h);
+            return nullptr;
+      }
+      csr_measure_span(h);
+      return h;
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A) {
+      if (!A) {
+            fail(-EINVAL, "null CSR handle");
+            return nullptr;
+      }
+      if (A->NZ >= (1ll << 31) - 64) {
+            fail(-ENOTSUP, "transpose of handles with 2^31 or more entries is not supported (NZ=%lld)",
+                 A->NZ);
+            return nullptr;
+      }
+      if (ensure_device())
+            return nullptr;
+      int prev = 0;
+      if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(A->device) != cudaSuccess) {
+            fail(-EIO, "transpose: cannot select device %d", A->device);
+            return nullptr;
+      }
+      spmv_b200_csr *h = csr_transpose_here(A);
+      cudaSetDevice(prev);
       return h;
 }
 
