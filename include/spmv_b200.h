@@ -130,6 +130,21 @@ spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, int z0,
  * failure; -ENOTSUP for 2^31 or more entries. */
 spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A);
 
+#define SPMV_B200_COO_SUM_DUPLICATES 1
+/* Resident CSR from n entries (d_row[k], d_col[k], d_val[k]) in device memory of the current
+ * device.  idx_bytes = 4 or 8 (both index arrays; torch indices are int64).  Row r of the result
+ * lists the entries of row r in increasing column order.  Entries with equal (row, col) keep
+ * their input order, or, with SPMV_B200_COO_SUM_DUPLICATES, become one entry whose value is
+ * their left-to-right sum in input order, starting from the first value.  Nothing is dropped for
+ * being zero.  The build is ordered after earlier work on `stream` and is synchronous.  The
+ * caller's arrays are not retained.  NULL + last_error on failure: -EINVAL for a bad shape, index
+ * width or flag, a null array, an array that is not device memory of the current device, or an
+ * index out of range (the message names the first such entry); -ENOTSUP for 2^31 - 64 or more
+ * entries; -ENOMEM when the temporaries do not fit. */
+spmv_b200_csr *spmv_b200_csr_from_coo(int64_t M, int64_t N, int64_t n, const void *d_row,
+                                      const void *d_col, int idx_bytes, const double *d_val,
+                                      int flags, void *stream);
+
 int64_t spmv_b200_csr_rows(const spmv_b200_csr *h);
 int64_t spmv_b200_csr_cols(const spmv_b200_csr *h);
 int64_t spmv_b200_csr_nnz(const spmv_b200_csr *h);

@@ -394,6 +394,59 @@ class CsrDevice:
         return cls(L.b200.spmv_b200_csr_gen_stencil27(nx, ny, nz, z0, z1, col_offset, n_local,
                                                       cuts_a.ctypes.data_as(L.c_i64p), len(cuts_a)))
 
+    @classmethod
+    def from_coo(cls, M, N, row, col, val, sum_duplicates=False, stream=None):
+        """CSR built on the GPU from COO triplets already in device memory
+        (spmv_b200_csr_from_coo).  `row` and `col`: contiguous 1-D CUDA tensors of equal length,
+        both int32 or both int64; `val`: contiguous float64 CUDA tensor of the same length.  Row r
+        lists its entries in increasing column order; entries with equal (row, col) keep their
+        input order, or with `sum_duplicates` become one entry holding their left-to-right sum.
+        Ordered after earlier work on `stream` (default: torch's current stream); synchronous.
+        The tensors are not retained."""
+        import torch
+        for name, t in (("row", row), ("col", col), ("val", val)):
+            if not isinstance(t, torch.Tensor):
+                raise TypeError(f"{name} must be a torch.Tensor, got {type(t).__name__}")
+            if not t.is_cuda or t.layout != torch.strided or t.dim() != 1 or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous 1-D CUDA tensor")
+        if row.dtype != col.dtype or row.dtype not in (torch.int32, torch.int64):
+            raise TypeError(f"row and col must both be int32 or both int64, got {row.dtype} and {col.dtype}")
+        if val.dtype != torch.float64:
+            raise TypeError(f"val must be float64, got {val.dtype}")
+        n = row.numel()
+        if col.numel() != n or val.numel() != n:
+            raise ValueError(f"row, col and val have {n}, {col.numel()} and {val.numel()} entries")
+        return cls(L.b200.spmv_b200_csr_from_coo(
+            int(M), int(N), n, row.data_ptr(), col.data_ptr(), row.element_size(), val.data_ptr(),
+            int(bool(sum_duplicates)), _stream_ptr(stream)))
+
+    @classmethod
+    def from_torch(cls, t, sum_duplicates=False, stream=None):
+        """CSR built on the GPU from a 2-D float64 CUDA tensor in torch.sparse_coo (coalesced or
+        not) or torch.sparse_csr layout; see from_coo.  A CSR tensor's row offsets are expanded
+        to row indices on the device first."""
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"expected a torch.Tensor, got {type(t).__name__}")
+        if t.layout not in (torch.sparse_coo, torch.sparse_csr):
+            raise TypeError(f"layout {t.layout} is not torch.sparse_coo or torch.sparse_csr")
+        if t.dtype != torch.float64:
+            raise TypeError(f"dtype {t.dtype} is not torch.float64")
+        if not t.is_cuda:
+            raise ValueError(f"tensor is on {t.device}, not on a CUDA device")
+        if t.dim() != 2 or t.sparse_dim() != 2 or t.dense_dim() != 0:
+            raise ValueError(f"need a 2-D sparse matrix without batch or dense dimensions, got shape "
+                             f"{tuple(t.shape)} with {t.sparse_dim()} sparse and {t.dense_dim()} dense dimensions")
+        M, N = t.shape
+        if t.layout == torch.sparse_coo:
+            idx = t._indices()
+            return cls.from_coo(M, N, idx[0].contiguous(), idx[1].contiguous(), t._values().contiguous(),
+                                sum_duplicates, stream)
+        crow, col = t.crow_indices(), t.col_indices()
+        with torch.cuda.stream(stream if stream is not None else torch.cuda.current_stream()):
+            row = torch.repeat_interleave(crow.diff(), output_size=col.numel())
+        return cls.from_coo(M, N, row, col.contiguous(), t.values().contiguous(), sum_duplicates, stream)
+
     def _check(self, rc):
         if rc:
             raise RuntimeError(f"libspmv_b200: {L.last_error()} (rc={rc})")

@@ -10,6 +10,7 @@
 
 #include <cub/cub.cuh>
 
+#include "coo_kernels.cuh"
 #include "csr_kernels.cuh"
 #include "gen_kernels.cuh"
 #include "hll_kernels.cuh"
@@ -1285,6 +1286,35 @@ extern "C" spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, in
       return h;
 }
 
+// Bits that can be non-zero in an index below n (at least 1, at most 31): the end bit of a radix
+// sort over such indices.
+static int index_bits(long long n) {
+      int b = 1;
+      while (b < 31 && (1ll << b) < n)
+            ++b;
+      return b;
+}
+
+// Row offsets from entries per row: irp[0..rows] = exclusive scan of count[0..rows] (count[rows] is
+// 0, so irp[rows] is the total).  d_scratch == nullptr only sets `bytes`.
+template <typename OffT>
+static cudaError_t scan_row_offsets(void *d_scratch, size_t &bytes, const int *count, OffT *irp,
+                                    long long rows, cudaStream_t st = 0) {
+      return cub::DeviceScan::ExclusiveSum(d_scratch, bytes, count, irp, (int)(rows + 1), st);
+}
+
+// Planning needs the row offsets on the host: h_irp = the M + 1 offsets of d_irp (the device work
+// that wrote them has finished).
+template <typename OffT>
+static int download_row_offsets(spmv_b200_csr *h, const char *what) {
+      std::vector<OffT> tmp((size_t)h->M + 1);
+      cudaError_t e = cudaMemcpy(tmp.data(), h->d_irp, tmp.size() * sizeof(OffT), cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess)
+            return fail(-EIO, "%s: row offsets download failed: %s", what, cudaGetErrorString(e));
+      h->h_irp.assign(tmp.begin(), tmp.end());
+      return 0;
+}
+
 // A^T on the current device.  Memory while the sort runs, besides A and the new handle:
 //   sort keys   the two key buffers of the radix sort live in the new handle's value array
 //               (8 bytes per entry = two int32 arrays), which the fill overwrites afterwards;
@@ -1303,11 +1333,9 @@ static int csr_transpose_fill(const spmv_b200_csr *A, spmv_b200_csr *h) {
       int *key0 = reinterpret_cast<int *>(h->d_as);
       int *key1 = key0 + ((NZ + 3) & ~3ll); // 16-byte aligned second half of the value array
       cub::DoubleBuffer<int> keys(key0, key1), vals(nullptr, h->d_ja);
-      int end_bit = 1; // column bits that can be non-zero
-      while (end_bit < 31 && (1ll << end_bit) < NT)
-            ++end_bit;
+      const int end_bit = index_bits(NT); // column bits that can be non-zero
       OutOffT *t_irp = static_cast<OutOffT *>(h->d_irp);
-      cudaError_t e = cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_count, t_irp, (int)(NT + 1));
+      cudaError_t e = scan_row_offsets(nullptr, scan_bytes, d_count, t_irp, NT);
       if (e == cudaSuccess && NZ > 0)
             e = cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
       if (e != cudaSuccess)
@@ -1331,7 +1359,7 @@ static int csr_transpose_fill(const spmv_b200_csr *A, spmv_b200_csr *h) {
             e = cudaGetLastError();
       }
       if (e == cudaSuccess)
-            e = cub::DeviceScan::ExclusiveSum(d_scratch, scan_bytes, d_count, t_irp, (int)(NT + 1));
+            e = scan_row_offsets(d_scratch, scan_bytes, d_count, t_irp, NT);
       if (e == cudaSuccess && NZ > 0) {
             vals = cub::DoubleBuffer<int>(d_idx, h->d_ja);
             e = cub::DeviceRadixSort::SortPairs(d_scratch, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
@@ -1350,14 +1378,7 @@ static int csr_transpose_fill(const spmv_b200_csr *A, spmv_b200_csr *h) {
       cudaFree(d_count), cudaFree(d_scratch), cudaFree(d_row_of), cudaFree(d_idx);
       if (e != cudaSuccess)
             return fail(-EIO, "transpose failed: %s", cudaGetErrorString(e));
-      // planning needs the row offsets on the host
-      h->h_irp.resize((size_t)NT + 1);
-      std::vector<OutOffT> tmp((size_t)NT + 1);
-      e = cudaMemcpy(tmp.data(), t_irp, (size_t)(NT + 1) * sizeof(OutOffT), cudaMemcpyDeviceToHost);
-      if (e != cudaSuccess)
-            return fail(-EIO, "transpose: row offsets download failed: %s", cudaGetErrorString(e));
-      std::copy(tmp.begin(), tmp.end(), h->h_irp.begin());
-      return 0;
+      return download_row_offsets<OutOffT>(h, "transpose");
 }
 
 static spmv_b200_csr *csr_transpose_here(const spmv_b200_csr *A) {
@@ -1398,6 +1419,266 @@ extern "C" spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A) {
       spmv_b200_csr *h = csr_transpose_here(A);
       cudaSetDevice(prev);
       return h;
+}
+
+// ------------------------------------------------------------- from COO --
+namespace {
+
+// Device temporaries of one build, freed on every way out.
+struct DeviceTemps {
+      std::vector<void *> ptrs;
+      long long bytes = 0; // requested so far, for the -ENOMEM message
+      ~DeviceTemps() { release_all(); }
+      template <typename T>
+      int alloc(T **out, size_t n_bytes, const char *what) {
+            bytes += (long long)n_bytes;
+            void *p = nullptr;
+            if (cudaMalloc(&p, std::max<size_t>(n_bytes, 1)) != cudaSuccess) {
+                  cudaGetLastError(); // clear the allocation error
+                  return fail(-ENOMEM, "%s: cudaMalloc of %lld bytes of temporaries failed", what, bytes);
+            }
+            ptrs.push_back(p);
+            *out = static_cast<T *>(p);
+            return 0;
+      }
+      void release(const void *p) {
+            for (auto &q : ptrs)
+                  if (q == p) {
+                        cudaFree(q);
+                        q = nullptr;
+                  }
+      }
+      void release_all() {
+            for (void *p : ptrs)
+                  cudaFree(p);
+            ptrs.clear();
+      }
+};
+
+} // namespace
+
+// CSR from n COO entries on the current device, all device work on `st`.  Steps:
+//   pack   bounds check, key = row << cb | col (rb row bits, cb column bits; 32-bit keys when
+//          rb + cb <= 32, else 64-bit), and whether the keys are sorted or repeat; 16 bytes read back;
+//   sort   only when some key is smaller than its predecessor: stable radix sort of (key, entry
+//          index) over bits [0, rb + cb), so entries with equal (row, col) keep their input order;
+//   heads  sum mode, when equal keys are possible: run starts, scanned in place into each run's
+//          output position and the output entry count (read back, 4 bytes);
+//   fill   one thread per output entry writes ja and as and counts its row; an exclusive scan of
+//          the counts is the row offsets.  In sum mode the thread of a run adds its L values left to
+//          right: L dependent loads on one thread, so one (row, col) repeated many times is slow.
+// Temporary memory besides the new handle (KB = 4 or 8 bytes per key):
+//   sort   two key buffers and two index buffers: 2*KB + 8 bytes per entry (16 or 24), plus CUB's
+//          scratch (histograms and tile state: a small fraction of a byte per entry); the spare key
+//          and index buffers and the scratch are freed when the sort is done;
+//   fill   sorted keys, the permutation and, in sum mode, the output positions: KB + 8 bytes per entry
+//          (12 or 16) + 4 bytes per row (+ 4) for the counts, plus CUB's scan scratch.
+// Input that is already sorted skips the sort and the permutation: KB bytes per entry, + 4 in sum
+// mode when keys repeat, + 4 per row.
+template <typename IdxT, typename KeyT>
+static spmv_b200_csr *csr_from_coo_here(long long M, long long N, long long n, const IdxT *d_row,
+                                        const IdxT *d_col, const double *d_val, bool sum, cudaStream_t st) {
+      static const char *what = "from_coo";
+      const int rb = index_bits(M), cb = index_bits(N);
+      const int grid = (int)std::max<long long>(
+          1, std::min<long long>(blocks_for(n, 256), (long long)g_sm_count * 64));
+      DeviceTemps tmp;
+      KeyT *key = nullptr;
+      CooStatus *d_st = nullptr, hs{0x7fffffff, 0, 0, 0};
+      if (n > 0 && (tmp.alloc(&d_st, sizeof(CooStatus), what) || tmp.alloc(&key, n * sizeof(KeyT), what)))
+            return nullptr;
+      cudaError_t e = cudaSuccess;
+      if (n > 0) {
+            e = cudaMemcpyAsync(d_st, &hs, sizeof hs, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) {
+                  coo_pack_kernel<IdxT, KeyT><<<grid, 256, 0, st>>>(d_row, d_col, n, M, N, cb, key, d_st);
+                  ++g_counters.launches;
+                  e = cudaGetLastError();
+            }
+            if (e == cudaSuccess)
+                  e = cudaMemcpyAsync(&hs, d_st, sizeof hs, cudaMemcpyDeviceToHost, st);
+            if (e == cudaSuccess)
+                  e = cudaStreamSynchronize(st);
+      }
+      if (e == cudaSuccess && hs.bad != 0x7fffffff) {
+            IdxT r = 0, c = 0;
+            e = cudaMemcpy(&r, d_row + hs.bad, sizeof r, cudaMemcpyDeviceToHost);
+            if (e == cudaSuccess)
+                  e = cudaMemcpy(&c, d_col + hs.bad, sizeof c, cudaMemcpyDeviceToHost);
+            if (e == cudaSuccess) {
+                  fail(-EINVAL, "from_coo: entry %d has row %lld and column %lld, outside [0, %lld) x [0, %lld)",
+                       hs.bad, (long long)r, (long long)c, M, N);
+                  return nullptr;
+            }
+      }
+      const int *perm = nullptr;
+      if (e == cudaSuccess && hs.unsorted) {
+            KeyT *key1 = nullptr;
+            int *idx0 = nullptr, *idx1 = nullptr;
+            void *scratch = nullptr;
+            size_t bytes = 0;
+            cub::DoubleBuffer<KeyT> keys(key, nullptr);
+            cub::DoubleBuffer<int> vals(nullptr, nullptr);
+            e = cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys, vals, (int)n, 0, rb + cb, st);
+            if (e != cudaSuccess) {
+                  fail(-EIO, "from_coo: CUB size query failed: %s", cudaGetErrorString(e));
+                  return nullptr;
+            }
+            if (tmp.alloc(&key1, n * sizeof(KeyT), what) || tmp.alloc(&idx0, n * sizeof(int), what) ||
+                tmp.alloc(&idx1, n * sizeof(int), what) || tmp.alloc(&scratch, bytes, what))
+                  return nullptr;
+            coo_iota_kernel<<<grid, 256, 0, st>>>(idx0, n);
+            ++g_counters.launches;
+            e = cudaGetLastError();
+            keys = cub::DoubleBuffer<KeyT>(key, key1);
+            vals = cub::DoubleBuffer<int>(idx0, idx1);
+            if (e == cudaSuccess) {
+                  e = cub::DeviceRadixSort::SortPairs(scratch, bytes, keys, vals, (int)n, 0, rb + cb, st);
+                  ++g_counters.launches; // one CUB call counts as one launch
+            }
+            if (e == cudaSuccess)
+                  e = cudaStreamSynchronize(st);
+            key = keys.Current();
+            perm = vals.Current();
+            tmp.release(keys.Alternate()), tmp.release(vals.Alternate()), tmp.release(scratch);
+      }
+      long long nz_out = n;
+      int *pos = nullptr;
+      if (e == cudaSuccess && sum && (hs.unsorted || hs.dup)) {
+            void *scratch = nullptr;
+            size_t bytes = 0;
+            e = cub::DeviceScan::ExclusiveSum(nullptr, bytes, pos, (int)(n + 1), st);
+            if (e != cudaSuccess) {
+                  fail(-EIO, "from_coo: CUB size query failed: %s", cudaGetErrorString(e));
+                  return nullptr;
+            }
+            if (tmp.alloc(&pos, (n + 1) * sizeof(int), what) || tmp.alloc(&scratch, bytes, what))
+                  return nullptr;
+            coo_heads_kernel<KeyT><<<grid, 256, 0, st>>>(key, n, pos);
+            ++g_counters.launches;
+            e = cudaGetLastError();
+            if (e == cudaSuccess) {
+                  e = cub::DeviceScan::ExclusiveSum(scratch, bytes, pos, (int)(n + 1), st);
+                  ++g_counters.launches;
+            }
+            int total = 0;
+            if (e == cudaSuccess)
+                  e = cudaMemcpyAsync(&total, pos + n, sizeof total, cudaMemcpyDeviceToHost, st);
+            if (e == cudaSuccess)
+                  e = cudaStreamSynchronize(st);
+            nz_out = total;
+            tmp.release(scratch);
+      }
+      if (e != cudaSuccess) {
+            fail(-EIO, "from_coo failed: %s", cudaGetErrorString(e));
+            return nullptr;
+      }
+
+      spmv_b200_csr *h = csr_alloc_shell(M, N, nz_out, 0);
+      if (!h)
+            return nullptr;
+      int *count = nullptr;
+      void *scratch = nullptr;
+      size_t bytes = 0;
+      // csr_alloc_shell zeroes the arrays on the legacy default stream, which `st` need not wait for
+      e = cudaStreamSynchronize(0);
+      if (e == cudaSuccess)
+            e = h->wide ? scan_row_offsets(nullptr, bytes, count, (long long *)h->d_irp, M, st)
+                        : scan_row_offsets(nullptr, bytes, count, (int *)h->d_irp, M, st);
+      int rc = e == cudaSuccess ? 0 : fail(-EIO, "from_coo: CUB size query failed: %s", cudaGetErrorString(e));
+      if (!rc)
+            rc = tmp.alloc(&count, (M + 1) * sizeof(int), what) || tmp.alloc(&scratch, bytes, what);
+      if (!rc) {
+            e = cudaMemsetAsync(count, 0, (M + 1) * sizeof(int), st);
+            if (e == cudaSuccess && n > 0) {
+                  if (pos)
+                        coo_fill_kernel<KeyT, true><<<grid, 256, 0, st>>>(key, perm, pos, d_val, n, cb, h->d_ja,
+                                                                          h->d_as, count);
+                  else
+                        coo_fill_kernel<KeyT, false><<<grid, 256, 0, st>>>(key, perm, pos, d_val, n, cb, h->d_ja,
+                                                                           h->d_as, count);
+                  ++g_counters.launches;
+                  e = cudaGetLastError();
+            }
+            if (e == cudaSuccess) {
+                  e = h->wide ? scan_row_offsets(scratch, bytes, count, (long long *)h->d_irp, M, st)
+                              : scan_row_offsets(scratch, bytes, count, (int *)h->d_irp, M, st);
+                  ++g_counters.launches;
+            }
+            if (e == cudaSuccess)
+                  e = cudaStreamSynchronize(st);
+            tmp.release_all();
+            if (e != cudaSuccess)
+                  rc = fail(-EIO, "from_coo failed: %s", cudaGetErrorString(e));
+      }
+      if (!rc)
+            rc = h->wide ? download_row_offsets<long long>(h, what) : download_row_offsets<int>(h, what);
+      if (rc || finish_create(h, nullptr, 0)) {
+            spmv_b200_csr_destroy(h);
+            return nullptr;
+      }
+      csr_measure_span(h);
+      return h;
+}
+
+template <typename IdxT>
+static spmv_b200_csr *csr_from_coo_idx(long long M, long long N, long long n, const void *d_row,
+                                       const void *d_col, const double *d_val, bool sum, cudaStream_t st) {
+      const IdxT *r = static_cast<const IdxT *>(d_row), *c = static_cast<const IdxT *>(d_col);
+      if (index_bits(M) + index_bits(N) <= 32)
+            return csr_from_coo_here<IdxT, unsigned>(M, N, n, r, c, d_val, sum, st);
+      return csr_from_coo_here<IdxT, unsigned long long>(M, N, n, r, c, d_val, sum, st);
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_from_coo(int64_t M, int64_t N, int64_t n, const void *d_row,
+                                                 const void *d_col, int idx_bytes, const double *d_val,
+                                                 int flags, void *stream) {
+      const long long lim = (1ll << 31) - 64;
+      if (M < 0 || N < 0 || n < 0 || M >= lim || N >= lim) {
+            fail(-EINVAL, "from_coo: bad shape M=%lld N=%lld n=%lld", (long long)M, (long long)N, (long long)n);
+            return nullptr;
+      }
+      if (idx_bytes != 4 && idx_bytes != 8) {
+            fail(-EINVAL, "from_coo: index width %d bytes (4 or 8)", idx_bytes);
+            return nullptr;
+      }
+      if (flags & ~SPMV_B200_COO_SUM_DUPLICATES) {
+            fail(-EINVAL, "from_coo: unknown flag bits 0x%x", flags);
+            return nullptr;
+      }
+      if (n >= lim) {
+            fail(-ENOTSUP, "from_coo: 2^31 or more entries are not supported (n=%lld)", (long long)n);
+            return nullptr;
+      }
+      if (n > 0 && (!d_row || !d_col || !d_val)) {
+            fail(-EINVAL, "from_coo: null array with n=%lld", (long long)n);
+            return nullptr;
+      }
+      if (ensure_device())
+            return nullptr;
+      int dev = 0;
+      if (cudaGetDevice(&dev) != cudaSuccess) {
+            fail(-EIO, "from_coo: no current device");
+            return nullptr;
+      }
+      const void *arrays[3] = {d_row, d_col, d_val};
+      const char *names[3] = {"row", "col", "val"};
+      for (int i = 0; i < 3 && n > 0; ++i) {
+            cudaPointerAttributes a;
+            if (cudaPointerGetAttributes(&a, arrays[i]) != cudaSuccess) {
+                  cudaGetLastError(); // clear the error of the query
+                  a.type = cudaMemoryTypeUnregistered;
+            }
+            if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != dev) {
+                  fail(-EINVAL, "from_coo: %s array %p is not device or managed memory of device %d", names[i],
+                       arrays[i], dev);
+                  return nullptr;
+            }
+      }
+      const bool sum = flags & SPMV_B200_COO_SUM_DUPLICATES;
+      cudaStream_t st = static_cast<cudaStream_t>(stream);
+      return idx_bytes == 4 ? csr_from_coo_idx<int>(M, N, n, d_row, d_col, d_val, sum, st)
+                            : csr_from_coo_idx<long long>(M, N, n, d_row, d_col, d_val, sum, st);
 }
 
 extern "C" void spmv_b200_csr_destroy(spmv_b200_csr *h) {
