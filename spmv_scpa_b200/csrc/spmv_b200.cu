@@ -1123,306 +1123,14 @@ int hll_max_col(const spmv_b200_hll *h, long long hack0, long long hack1, int *o
 } // namespace b200
 
 // --------------------------------------------------------------- creation --
-static void csr_measure_span(spmv_b200_csr *h) {
-      if (h->wide)
-            h->gather_span = measure_gather_span(
-                CsrSrc<long long>{(const long long *)h->d_irp, h->d_ja, h->d_as}, h->M, h->N);
-      else
-            h->gather_span =
-                measure_gather_span(CsrSrc<int>{(const int *)h->d_irp, h->d_ja, h->d_as}, h->M, h->N);
-}
-
-static spmv_b200_csr *csr_alloc_shell(long long M, long long n_local, long long NZ,
-                                      long long col_offset) {
-      if (ensure_device())
-            return nullptr;
-      if (M < 0 || n_local < 0 || NZ < 0 || M >= (1ll << 31) - 64) {
-            fail(-EINVAL, "bad CSR shape M=%lld N=%lld NZ=%lld", M, n_local, NZ);
-            return nullptr;
-      }
-      auto *h = new spmv_b200_csr();
-      h->M = M, h->N = n_local, h->NZ = NZ, h->col_offset = col_offset;
-      h->wide = g_knobs.force_wide || NZ >= (1ll << 31) - 64;
-      cudaGetDevice(&h->device);
-      // +8 entries of slack: the entry-split kernel bulk-copies row offsets in 16-byte units
-      const size_t irp_bytes = (size_t)(M + 1 + 8) * (h->wide ? 8 : 4);
-      // +16 entries of slack: bulk copies round the entry range out to x4
-      if (cudaMalloc(&h->d_irp, irp_bytes) != cudaSuccess ||
-          cudaMalloc(&h->d_ja, ((size_t)NZ + 16) * sizeof(int)) != cudaSuccess ||
-          cudaMalloc(&h->d_as, ((size_t)NZ + 16) * sizeof(double)) != cudaSuccess) {
-            fail(-ENOMEM, "cudaMalloc failed for CSR M=%lld NZ=%lld: %s", M, NZ,
-                 cudaGetErrorString(cudaGetLastError()));
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      cudaMemset(h->d_irp, 0, irp_bytes);
-      cudaMemset(h->d_ja + NZ, 0, 16 * sizeof(int));
-      cudaMemset(h->d_as + NZ, 0, 16 * sizeof(double));
-      return h;
-}
-
-extern "C" spmv_b200_csr *spmv_b200_csr_create_ex(int64_t M, int64_t n_local, int64_t NZ,
-                                                  const void *irp, int irp_bytes, const int *JA,
-                                                  const double *AS, int64_t col_offset,
-                                                  const int64_t *cuts, int n_cuts) {
-      if (!irp || (NZ > 0 && (!JA || !AS)) || (irp_bytes != 4 && irp_bytes != 8)) {
-            fail(-EINVAL, "spmv_b200_csr_create_ex: bad arguments");
-            return nullptr;
-      }
-      spmv_b200_csr *h = csr_alloc_shell(M, n_local, NZ, col_offset);
-      if (!h)
-            return nullptr;
-
-      h->h_irp.resize((size_t)M + 1);
-      if (irp_bytes == 4) {
-            const int *p = static_cast<const int *>(irp);
-            for (long long r = 0; r <= M; ++r)
-                  h->h_irp[r] = p[r];
-      } else {
-            const long long *p = static_cast<const long long *>(irp);
-            for (long long r = 0; r <= M; ++r)
-                  h->h_irp[r] = p[r];
-      }
-      bool ok = h->h_irp[0] == 0 && h->h_irp[M] == NZ;
-      for (long long r = 0; r < M && ok; ++r)
-            ok = h->h_irp[r + 1] >= h->h_irp[r];
-      if (!ok) {
-            fail(-EINVAL, "row offsets are not a monotone prefix ending at NZ");
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-
-      cudaError_t e;
-      if (h->wide) {
-            e = cudaMemcpy(h->d_irp, h->h_irp.data(), (size_t)(M + 1) * 8, cudaMemcpyHostToDevice);
-      } else {
-            std::vector<int> tmp(h->h_irp.begin(), h->h_irp.end());
-            e = cudaMemcpy(h->d_irp, tmp.data(), (size_t)(M + 1) * 4, cudaMemcpyHostToDevice);
-      }
-      if (e == cudaSuccess && NZ > 0)
-            e = cudaMemcpy(h->d_as, AS, (size_t)NZ * sizeof(double), cudaMemcpyHostToDevice);
-      if (e == cudaSuccess && NZ > 0) {
-            if (col_offset == 0) {
-                  e = cudaMemcpy(h->d_ja, JA, (size_t)NZ * sizeof(int), cudaMemcpyHostToDevice);
-            } else {
-                  std::vector<int> rel((size_t)NZ);
-#pragma omp parallel for schedule(static)
-                  for (long long k = 0; k < NZ; ++k)
-                        rel[k] = (int)((long long)JA[k] - col_offset);
-                  e = cudaMemcpy(h->d_ja, rel.data(), (size_t)NZ * sizeof(int),
-                                 cudaMemcpyHostToDevice);
-            }
-      }
-      if (e != cudaSuccess) {
-            fail(-EIO, "CSR upload failed: %s", cudaGetErrorString(e));
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      g_counters.h2d += (long long)((M + 1) * (h->wide ? 8 : 4) + NZ * 12);
-
-      if (csr_check_columns(h) || finish_create(h, reinterpret_cast<const long long *>(cuts), n_cuts)) {
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      csr_measure_span(h);
-      return h;
-}
-
-extern "C" spmv_b200_csr *spmv_b200_csr_create(const sparse_csr *A) {
-      if (!A) {
-            fail(-EINVAL, "null sparse_csr");
-            return nullptr;
-      }
-      return spmv_b200_csr_create_ex(A->M, A->N, A->NZ, A->IRP, 4, A->JA, A->AS, 0, nullptr, 0);
-}
-
-extern "C" spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, int z0, int z1,
-                                                      int64_t col_offset, int64_t n_local,
-                                                      const int64_t *cuts, int n_cuts) {
-      if (nx < 1 || ny < 1 || nz < 1 || z0 < 0 || z1 > nz || z0 > z1) {
-            fail(-EINVAL, "bad stencil geometry");
-            return nullptr;
-      }
-      const long long plane = (long long)nx * ny, rows = plane * (z1 - z0);
-      auto prefix = [](long long c, long long n) {
-            return c == 0 ? 0ll : (c >= n ? 3 * n - 2 : 3 * c - 1);
-      };
-      const long long nnz = (prefix(z1, nz) - prefix(z0, nz)) * (3ll * ny - 2) * (3ll * nx - 2);
-      spmv_b200_csr *h = csr_alloc_shell(rows, n_local, nnz, col_offset);
-      if (!h)
-            return nullptr;
-      StencilGeom g{nx, ny, nz, z0, col_offset};
-      const int grid = blocks_for(rows + 1, 256);
-      if (h->wide)
-            stencil27_fill_kernel<long long><<<grid, 256>>>(g, rows, (long long *)h->d_irp,
-                                                            h->d_ja, h->d_as);
-      else
-            stencil27_fill_kernel<int><<<grid, 256>>>(g, rows, (int *)h->d_irp, h->d_ja, h->d_as);
-      ++g_counters.launches;
-      cudaError_t e = cudaDeviceSynchronize();
-      // planning needs the row offsets on the host
-      h->h_irp.resize((size_t)rows + 1);
-      if (e == cudaSuccess) {
-            if (h->wide) {
-                  e = cudaMemcpy(h->h_irp.data(), h->d_irp, (size_t)(rows + 1) * 8,
-                                 cudaMemcpyDeviceToHost);
-            } else {
-                  std::vector<int> tmp((size_t)rows + 1);
-                  e = cudaMemcpy(tmp.data(), h->d_irp, (size_t)(rows + 1) * 4,
-                                 cudaMemcpyDeviceToHost);
-                  std::copy(tmp.begin(), tmp.end(), h->h_irp.begin());
-            }
-      }
-      if (e != cudaSuccess) {
-            fail(-EIO, "stencil generation failed: %s", cudaGetErrorString(e));
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      if (finish_create(h, reinterpret_cast<const long long *>(cuts), n_cuts)) {
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      csr_measure_span(h);
-      return h;
-}
-
-// Bits that can be non-zero in an index below n (at least 1, at most 31): the end bit of a radix
-// sort over such indices.
-static int index_bits(long long n) {
-      int b = 1;
-      while (b < 31 && (1ll << b) < n)
-            ++b;
-      return b;
-}
-
-// Row offsets from entries per row: irp[0..rows] = exclusive scan of count[0..rows] (count[rows] is
-// 0, so irp[rows] is the total).  d_scratch == nullptr only sets `bytes`.
-template <typename OffT>
-static cudaError_t scan_row_offsets(void *d_scratch, size_t &bytes, const int *count, OffT *irp,
-                                    long long rows, cudaStream_t st = 0) {
-      return cub::DeviceScan::ExclusiveSum(d_scratch, bytes, count, irp, (int)(rows + 1), st);
-}
-
-// Planning needs the row offsets on the host: h_irp = the M + 1 offsets of d_irp (the device work
-// that wrote them has finished).
-template <typename OffT>
-static int download_row_offsets(spmv_b200_csr *h, const char *what) {
-      std::vector<OffT> tmp((size_t)h->M + 1);
-      cudaError_t e = cudaMemcpy(tmp.data(), h->d_irp, tmp.size() * sizeof(OffT), cudaMemcpyDeviceToHost);
-      if (e != cudaSuccess)
-            return fail(-EIO, "%s: row offsets download failed: %s", what, cudaGetErrorString(e));
-      h->h_irp.assign(tmp.begin(), tmp.end());
-      return 0;
-}
-
-// A^T on the current device.  Memory while the sort runs, besides A and the new handle:
-//   sort keys   the two key buffers of the radix sort live in the new handle's value array
-//               (8 bytes per entry = two int32 arrays), which the fill overwrites afterwards;
-//   sort values one buffer is the new handle's column array, the other is temporary (4 B/entry);
-//   row_of      row of every entry of A (temporary, 4 B/entry);
-//   count       entries per column of A (temporary, 4 B per column + 4);
-//   scratch     CUB's temporary storage (histograms and tile state, independent of the entry count
-//               up to a few bytes per tile).
-// Peak temporary memory is therefore 8 bytes per entry + 4 bytes per column + CUB's scratch.
-template <typename InOffT, typename OutOffT>
-static int csr_transpose_fill(const spmv_b200_csr *A, spmv_b200_csr *h) {
-      const long long NZ = A->NZ, NT = A->N; // NT: rows of A^T
-      int *d_count = nullptr, *d_row_of = nullptr, *d_idx = nullptr;
-      void *d_scratch = nullptr;
-      size_t scan_bytes = 0, sort_bytes = 0;
-      int *key0 = reinterpret_cast<int *>(h->d_as);
-      int *key1 = key0 + ((NZ + 3) & ~3ll); // 16-byte aligned second half of the value array
-      cub::DoubleBuffer<int> keys(key0, key1), vals(nullptr, h->d_ja);
-      const int end_bit = index_bits(NT); // column bits that can be non-zero
-      OutOffT *t_irp = static_cast<OutOffT *>(h->d_irp);
-      cudaError_t e = scan_row_offsets(nullptr, scan_bytes, d_count, t_irp, NT);
-      if (e == cudaSuccess && NZ > 0)
-            e = cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
-      if (e != cudaSuccess)
-            return fail(-EIO, "transpose: CUB size query failed: %s", cudaGetErrorString(e));
-      const size_t scratch_bytes = std::max(scan_bytes, sort_bytes);
-      if (cudaMalloc(&d_count, (size_t)(NT + 1) * sizeof(int)) != cudaSuccess ||
-          cudaMalloc(&d_scratch, std::max<size_t>(scratch_bytes, 1)) != cudaSuccess ||
-          (NZ > 0 && (cudaMalloc(&d_row_of, (size_t)NZ * sizeof(int)) != cudaSuccess ||
-                      cudaMalloc(&d_idx, (size_t)NZ * sizeof(int)) != cudaSuccess))) {
-            cudaGetLastError(); // clear the allocation error
-            cudaFree(d_count), cudaFree(d_scratch), cudaFree(d_row_of), cudaFree(d_idx);
-            return fail(-ENOMEM, "transpose: cudaMalloc of %lld bytes of temporaries failed",
-                        (long long)((NT + 1) * 4 + NZ * 8 + (long long)scratch_bytes));
-      }
-      e = cudaMemsetAsync(d_count, 0, (size_t)(NT + 1) * sizeof(int));
-      if (e == cudaSuccess && NZ > 0) {
-            const int grid = (int)std::min<long long>(blocks_for(A->M * 32, 256), 65535ll * 8);
-            transpose_prep_kernel<InOffT><<<grid, 256>>>(static_cast<const InOffT *>(A->d_irp), A->d_ja,
-                                                         A->M, d_row_of, key0, d_idx, d_count);
-            ++g_counters.launches;
-            e = cudaGetLastError();
-      }
-      if (e == cudaSuccess)
-            e = scan_row_offsets(d_scratch, scan_bytes, d_count, t_irp, NT);
-      if (e == cudaSuccess && NZ > 0) {
-            vals = cub::DoubleBuffer<int>(d_idx, h->d_ja);
-            e = cub::DeviceRadixSort::SortPairs(d_scratch, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
-      }
-      if (e == cudaSuccess && NZ > 0) {
-            const int grid = (int)std::min<long long>(blocks_for(NZ, 256), (long long)g_sm_count * 64);
-            transpose_fill_kernel<<<grid, 256>>>(vals.Current(), d_row_of, A->d_as, NZ, h->d_ja, h->d_as);
-            ++g_counters.launches;
-            e = cudaGetLastError();
-      }
-      // the second key buffer may have reached into the 16 zero entries after the values
-      if (e == cudaSuccess)
-            e = cudaMemsetAsync(h->d_as + NZ, 0, 16 * sizeof(double));
-      if (e == cudaSuccess)
-            e = cudaDeviceSynchronize();
-      cudaFree(d_count), cudaFree(d_scratch), cudaFree(d_row_of), cudaFree(d_idx);
-      if (e != cudaSuccess)
-            return fail(-EIO, "transpose failed: %s", cudaGetErrorString(e));
-      return download_row_offsets<OutOffT>(h, "transpose");
-}
-
-static spmv_b200_csr *csr_transpose_here(const spmv_b200_csr *A) {
-      spmv_b200_csr *h = csr_alloc_shell(A->N, A->M, A->NZ, 0);
-      if (!h)
-            return nullptr;
-      int rc;
-      if (A->wide)
-            rc = h->wide ? csr_transpose_fill<long long, long long>(A, h)
-                         : csr_transpose_fill<long long, int>(A, h);
-      else
-            rc = h->wide ? csr_transpose_fill<int, long long>(A, h) : csr_transpose_fill<int, int>(A, h);
-      if (rc || finish_create(h, nullptr, 0)) {
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      csr_measure_span(h);
-      return h;
-}
-
-extern "C" spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A) {
-      if (!A) {
-            fail(-EINVAL, "null CSR handle");
-            return nullptr;
-      }
-      if (A->NZ >= (1ll << 31) - 64) {
-            fail(-ENOTSUP, "transpose of handles with 2^31 or more entries is not supported (NZ=%lld)",
-                 A->NZ);
-            return nullptr;
-      }
-      if (ensure_device())
-            return nullptr;
-      int prev = 0;
-      if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(A->device) != cudaSuccess) {
-            fail(-EIO, "transpose: cannot select device %d", A->device);
-            return nullptr;
-      }
-      spmv_b200_csr *h = csr_transpose_here(A);
-      cudaSetDevice(prev);
-      return h;
-}
-
-// ------------------------------------------------------------- from COO --
 namespace {
+
+template <typename T> struct OffTag { using type = T; };
+
+// f(OffTag<OffT>{}) with OffT the row offset type of a handle: long long when `wide`, else int.
+template <typename F> auto with_offsets(bool wide, F &&f) {
+      return wide ? f(OffTag<long long>{}) : f(OffTag<int>{});
+}
 
 // Device temporaries of one build, freed on every way out.
 struct DeviceTemps {
@@ -1457,6 +1165,278 @@ struct DeviceTemps {
 
 } // namespace
 
+static void csr_measure_span(spmv_b200_csr *h) {
+      h->gather_span = with_offsets(h->wide, [&](auto t) {
+            using OffT = typename decltype(t)::type;
+            return measure_gather_span(CsrSrc<OffT>{(const OffT *)h->d_irp, h->d_ja, h->d_as}, h->M, h->N);
+      });
+}
+
+// Planning needs the row offsets on the host: h_irp = the M + 1 offsets of d_irp (the device work
+// that wrote them has finished).  64-bit offsets come down in place, 32-bit ones through a copy.
+static int download_row_offsets(spmv_b200_csr *h, const char *what) {
+      h->h_irp.resize((size_t)h->M + 1);
+      std::vector<int> narrow(h->wide ? 0 : h->h_irp.size());
+      void *dst = h->wide ? (void *)h->h_irp.data() : (void *)narrow.data();
+      cudaError_t e = cudaMemcpy(dst, h->d_irp, h->h_irp.size() * (h->wide ? 8 : 4), cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess)
+            return fail(-EIO, "%s: row offsets download failed: %s", what, cudaGetErrorString(e));
+      std::copy(narrow.begin(), narrow.end(), h->h_irp.begin());
+      return 0;
+}
+
+// Every constructor returns through here once its shell exists.  rc != 0: the fill failed (fail()
+// has set the message), so the shell is destroyed.  Otherwise the row offsets come down to the host
+// unless the constructor built them there (h_irp is empty until then), and the handle is planned.
+static spmv_b200_csr *csr_finish(spmv_b200_csr *h, int rc, const int64_t *cuts, int n_cuts,
+                                 const char *what) {
+      if (!rc && h->h_irp.empty())
+            rc = download_row_offsets(h, what);
+      if (rc || finish_create(h, reinterpret_cast<const long long *>(cuts), n_cuts)) {
+            spmv_b200_csr_destroy(h);
+            return nullptr;
+      }
+      csr_measure_span(h);
+      return h;
+}
+
+// A new handle whose row offsets and slack entries are zeroed on `st`, the stream its fill runs on,
+// so the fill is ordered after the zeroing without a synchronisation.
+static spmv_b200_csr *csr_alloc_shell(long long M, long long n_local, long long NZ,
+                                      long long col_offset, cudaStream_t st) {
+      if (ensure_device())
+            return nullptr;
+      if (M < 0 || n_local < 0 || NZ < 0 || M >= (1ll << 31) - 64) {
+            fail(-EINVAL, "bad CSR shape M=%lld N=%lld NZ=%lld", M, n_local, NZ);
+            return nullptr;
+      }
+      auto *h = new spmv_b200_csr();
+      h->M = M, h->N = n_local, h->NZ = NZ, h->col_offset = col_offset;
+      h->wide = g_knobs.force_wide || NZ >= (1ll << 31) - 64;
+      cudaGetDevice(&h->device);
+      // +8 entries of slack: the entry-split kernel bulk-copies row offsets in 16-byte units
+      const size_t irp_bytes = (size_t)(M + 1 + 8) * (h->wide ? 8 : 4);
+      // +16 entries of slack: bulk copies round the entry range out to x4
+      if (cudaMalloc(&h->d_irp, irp_bytes) != cudaSuccess ||
+          cudaMalloc(&h->d_ja, ((size_t)NZ + 16) * sizeof(int)) != cudaSuccess ||
+          cudaMalloc(&h->d_as, ((size_t)NZ + 16) * sizeof(double)) != cudaSuccess) {
+            fail(-ENOMEM, "cudaMalloc failed for CSR M=%lld NZ=%lld: %s", M, NZ,
+                 cudaGetErrorString(cudaGetLastError()));
+            spmv_b200_csr_destroy(h);
+            return nullptr;
+      }
+      cudaError_t e = cudaMemsetAsync(h->d_irp, 0, irp_bytes, st);
+      if (e == cudaSuccess)
+            e = cudaMemsetAsync(h->d_ja + NZ, 0, 16 * sizeof(int), st);
+      if (e == cudaSuccess)
+            e = cudaMemsetAsync(h->d_as + NZ, 0, 16 * sizeof(double), st);
+      if (e != cudaSuccess) {
+            fail(-EIO, "zeroing a new CSR handle failed: %s", cudaGetErrorString(e));
+            spmv_b200_csr_destroy(h);
+            return nullptr;
+      }
+      return h;
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_create_ex(int64_t M, int64_t n_local, int64_t NZ,
+                                                  const void *irp, int irp_bytes, const int *JA,
+                                                  const double *AS, int64_t col_offset,
+                                                  const int64_t *cuts, int n_cuts) {
+      if (!irp || (NZ > 0 && (!JA || !AS)) || (irp_bytes != 4 && irp_bytes != 8)) {
+            fail(-EINVAL, "spmv_b200_csr_create_ex: bad arguments");
+            return nullptr;
+      }
+      static const char *what = "create_ex";
+      spmv_b200_csr *h = csr_alloc_shell(M, n_local, NZ, col_offset, 0);
+      if (!h)
+            return nullptr;
+
+      h->h_irp.resize((size_t)M + 1);
+      if (irp_bytes == 4) {
+            const int *p = static_cast<const int *>(irp);
+            for (long long r = 0; r <= M; ++r)
+                  h->h_irp[r] = p[r];
+      } else {
+            const long long *p = static_cast<const long long *>(irp);
+            for (long long r = 0; r <= M; ++r)
+                  h->h_irp[r] = p[r];
+      }
+      bool ok = h->h_irp[0] == 0 && h->h_irp[M] == NZ;
+      for (long long r = 0; r < M && ok; ++r)
+            ok = h->h_irp[r + 1] >= h->h_irp[r];
+      if (!ok)
+            return csr_finish(h, fail(-EINVAL, "row offsets are not a monotone prefix ending at NZ"),
+                              cuts, n_cuts, what);
+
+      cudaError_t e;
+      if (h->wide) {
+            e = cudaMemcpy(h->d_irp, h->h_irp.data(), (size_t)(M + 1) * 8, cudaMemcpyHostToDevice);
+      } else {
+            std::vector<int> tmp(h->h_irp.begin(), h->h_irp.end());
+            e = cudaMemcpy(h->d_irp, tmp.data(), (size_t)(M + 1) * 4, cudaMemcpyHostToDevice);
+      }
+      if (e == cudaSuccess && NZ > 0)
+            e = cudaMemcpy(h->d_as, AS, (size_t)NZ * sizeof(double), cudaMemcpyHostToDevice);
+      if (e == cudaSuccess && NZ > 0) {
+            if (col_offset == 0) {
+                  e = cudaMemcpy(h->d_ja, JA, (size_t)NZ * sizeof(int), cudaMemcpyHostToDevice);
+            } else {
+                  std::vector<int> rel((size_t)NZ);
+#pragma omp parallel for schedule(static)
+                  for (long long k = 0; k < NZ; ++k)
+                        rel[k] = (int)((long long)JA[k] - col_offset);
+                  e = cudaMemcpy(h->d_ja, rel.data(), (size_t)NZ * sizeof(int),
+                                 cudaMemcpyHostToDevice);
+            }
+      }
+      if (e != cudaSuccess)
+            return csr_finish(h, fail(-EIO, "CSR upload failed: %s", cudaGetErrorString(e)), cuts, n_cuts,
+                              what);
+      g_counters.h2d += (long long)((M + 1) * (h->wide ? 8 : 4) + NZ * 12);
+      return csr_finish(h, csr_check_columns(h), cuts, n_cuts, what);
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_create(const sparse_csr *A) {
+      if (!A) {
+            fail(-EINVAL, "null sparse_csr");
+            return nullptr;
+      }
+      return spmv_b200_csr_create_ex(A->M, A->N, A->NZ, A->IRP, 4, A->JA, A->AS, 0, nullptr, 0);
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, int z0, int z1,
+                                                      int64_t col_offset, int64_t n_local,
+                                                      const int64_t *cuts, int n_cuts) {
+      if (nx < 1 || ny < 1 || nz < 1 || z0 < 0 || z1 > nz || z0 > z1) {
+            fail(-EINVAL, "bad stencil geometry");
+            return nullptr;
+      }
+      const long long plane = (long long)nx * ny, rows = plane * (z1 - z0);
+      auto prefix = [](long long c, long long n) {
+            return c == 0 ? 0ll : (c >= n ? 3 * n - 2 : 3 * c - 1);
+      };
+      const long long nnz = (prefix(z1, nz) - prefix(z0, nz)) * (3ll * ny - 2) * (3ll * nx - 2);
+      spmv_b200_csr *h = csr_alloc_shell(rows, n_local, nnz, col_offset, 0);
+      if (!h)
+            return nullptr;
+      StencilGeom g{nx, ny, nz, z0, col_offset};
+      with_offsets(h->wide, [&](auto t) {
+            using OffT = typename decltype(t)::type;
+            stencil27_fill_kernel<OffT><<<blocks_for(rows + 1, 256), 256>>>(g, rows, (OffT *)h->d_irp,
+                                                                           h->d_ja, h->d_as);
+      });
+      ++g_counters.launches;
+      const cudaError_t e = cudaDeviceSynchronize();
+      const int rc = e == cudaSuccess ? 0 : fail(-EIO, "stencil generation failed: %s", cudaGetErrorString(e));
+      return csr_finish(h, rc, cuts, n_cuts, "stencil generation");
+}
+
+// Bits that can be non-zero in an index below n (at least 1, at most 31): the end bit of a radix
+// sort over such indices.
+static int index_bits(long long n) {
+      int b = 1;
+      while (b < 31 && (1ll << b) < n)
+            ++b;
+      return b;
+}
+
+// Row offsets of h from entries per row: d_irp[0..M] = exclusive scan of count[0..M] (count[M] is 0,
+// so d_irp[M] is the total).  d_scratch == nullptr only sets `bytes`.
+static cudaError_t scan_row_offsets(void *d_scratch, size_t &bytes, const int *count, spmv_b200_csr *h,
+                                    cudaStream_t st = 0) {
+      return with_offsets(h->wide, [&](auto t) {
+            using OffT = typename decltype(t)::type;
+            return cub::DeviceScan::ExclusiveSum(d_scratch, bytes, count, (OffT *)h->d_irp, (int)(h->M + 1), st);
+      });
+}
+
+// A^T on the current device.  Memory while the sort runs, besides A and the new handle:
+//   sort keys   the two key buffers of the radix sort live in the new handle's value array
+//               (8 bytes per entry = two int32 arrays), which the fill overwrites afterwards;
+//   sort values one buffer is the new handle's column array, the other is temporary (4 B/entry);
+//   row_of      row of every entry of A (temporary, 4 B/entry);
+//   count       entries per column of A (temporary, 4 B per column + 4);
+//   scratch     CUB's temporary storage (histograms and tile state, independent of the entry count
+//               up to a few bytes per tile).
+// Peak temporary memory is therefore 8 bytes per entry + 4 bytes per column + CUB's scratch.
+static int csr_transpose_fill(const spmv_b200_csr *A, spmv_b200_csr *h) {
+      static const char *what = "transpose";
+      const long long NZ = A->NZ, NT = A->N; // NT: rows of A^T
+      DeviceTemps tmp;
+      int *d_count = nullptr, *d_row_of = nullptr, *d_idx = nullptr;
+      void *d_scratch = nullptr;
+      size_t scan_bytes = 0, sort_bytes = 0;
+      int *key0 = reinterpret_cast<int *>(h->d_as);
+      int *key1 = key0 + ((NZ + 3) & ~3ll); // 16-byte aligned second half of the value array
+      cub::DoubleBuffer<int> keys(key0, key1), vals(nullptr, h->d_ja);
+      const int end_bit = index_bits(NT); // column bits that can be non-zero
+      cudaError_t e = scan_row_offsets(nullptr, scan_bytes, d_count, h);
+      if (e == cudaSuccess && NZ > 0)
+            e = cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
+      if (e != cudaSuccess)
+            return fail(-EIO, "transpose: CUB size query failed: %s", cudaGetErrorString(e));
+      if (tmp.alloc(&d_count, (NT + 1) * sizeof(int), what) ||
+          tmp.alloc(&d_scratch, std::max(scan_bytes, sort_bytes), what) ||
+          (NZ > 0 && (tmp.alloc(&d_row_of, NZ * sizeof(int), what) || tmp.alloc(&d_idx, NZ * sizeof(int), what))))
+            return -ENOMEM;
+      e = cudaMemsetAsync(d_count, 0, (size_t)(NT + 1) * sizeof(int));
+      if (e == cudaSuccess && NZ > 0) {
+            const int grid = (int)std::min<long long>(blocks_for(A->M * 32, 256), 65535ll * 8);
+            with_offsets(A->wide, [&](auto t) {
+                  using OffT = typename decltype(t)::type;
+                  transpose_prep_kernel<OffT><<<grid, 256>>>((const OffT *)A->d_irp, A->d_ja, A->M, d_row_of,
+                                                             key0, d_idx, d_count);
+            });
+            ++g_counters.launches;
+            e = cudaGetLastError();
+      }
+      if (e == cudaSuccess)
+            e = scan_row_offsets(d_scratch, scan_bytes, d_count, h);
+      if (e == cudaSuccess && NZ > 0) {
+            vals = cub::DoubleBuffer<int>(d_idx, h->d_ja);
+            e = cub::DeviceRadixSort::SortPairs(d_scratch, sort_bytes, keys, vals, (int)NZ, 0, end_bit);
+      }
+      if (e == cudaSuccess && NZ > 0) {
+            const int grid = (int)std::min<long long>(blocks_for(NZ, 256), (long long)g_sm_count * 64);
+            transpose_fill_kernel<<<grid, 256>>>(vals.Current(), d_row_of, A->d_as, NZ, h->d_ja, h->d_as);
+            ++g_counters.launches;
+            e = cudaGetLastError();
+      }
+      // the second key buffer may have reached into the 16 zero entries after the values
+      if (e == cudaSuccess)
+            e = cudaMemsetAsync(h->d_as + NZ, 0, 16 * sizeof(double));
+      if (e == cudaSuccess)
+            e = cudaDeviceSynchronize();
+      if (e != cudaSuccess)
+            return fail(-EIO, "transpose failed: %s", cudaGetErrorString(e));
+      return 0;
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A) {
+      if (!A) {
+            fail(-EINVAL, "null CSR handle");
+            return nullptr;
+      }
+      if (A->NZ >= (1ll << 31) - 64) {
+            fail(-ENOTSUP, "transpose of handles with 2^31 or more entries is not supported (NZ=%lld)",
+                 A->NZ);
+            return nullptr;
+      }
+      if (ensure_device())
+            return nullptr;
+      int prev = 0;
+      if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(A->device) != cudaSuccess) {
+            fail(-EIO, "transpose: cannot select device %d", A->device);
+            return nullptr;
+      }
+      spmv_b200_csr *h = csr_alloc_shell(A->N, A->M, A->NZ, 0, 0);
+      if (h)
+            h = csr_finish(h, csr_transpose_fill(A, h), nullptr, 0, "transpose");
+      cudaSetDevice(prev);
+      return h;
+}
+
+// ------------------------------------------------------------- from COO --
 // CSR from n COO entries on the current device, all device work on `st`.  Steps:
 //   pack   bounds check, key = row << cb | col (rb row bits, cb column bits; 32-bit keys when
 //          rb + cb <= 32, else 64-bit), and whether the keys are sorted or repeat; 16 bytes read back;
@@ -1574,17 +1554,13 @@ static spmv_b200_csr *csr_from_coo_here(long long M, long long N, long long n, c
             return nullptr;
       }
 
-      spmv_b200_csr *h = csr_alloc_shell(M, N, nz_out, 0);
+      spmv_b200_csr *h = csr_alloc_shell(M, N, nz_out, 0, st);
       if (!h)
             return nullptr;
       int *count = nullptr;
       void *scratch = nullptr;
       size_t bytes = 0;
-      // csr_alloc_shell zeroes the arrays on the legacy default stream, which `st` need not wait for
-      e = cudaStreamSynchronize(0);
-      if (e == cudaSuccess)
-            e = h->wide ? scan_row_offsets(nullptr, bytes, count, (long long *)h->d_irp, M, st)
-                        : scan_row_offsets(nullptr, bytes, count, (int *)h->d_irp, M, st);
+      e = scan_row_offsets(nullptr, bytes, count, h, st);
       int rc = e == cudaSuccess ? 0 : fail(-EIO, "from_coo: CUB size query failed: %s", cudaGetErrorString(e));
       if (!rc)
             rc = tmp.alloc(&count, (M + 1) * sizeof(int), what) || tmp.alloc(&scratch, bytes, what);
@@ -1601,8 +1577,7 @@ static spmv_b200_csr *csr_from_coo_here(long long M, long long N, long long n, c
                   e = cudaGetLastError();
             }
             if (e == cudaSuccess) {
-                  e = h->wide ? scan_row_offsets(scratch, bytes, count, (long long *)h->d_irp, M, st)
-                              : scan_row_offsets(scratch, bytes, count, (int *)h->d_irp, M, st);
+                  e = scan_row_offsets(scratch, bytes, count, h, st);
                   ++g_counters.launches;
             }
             if (e == cudaSuccess)
@@ -1611,14 +1586,7 @@ static spmv_b200_csr *csr_from_coo_here(long long M, long long N, long long n, c
             if (e != cudaSuccess)
                   rc = fail(-EIO, "from_coo failed: %s", cudaGetErrorString(e));
       }
-      if (!rc)
-            rc = h->wide ? download_row_offsets<long long>(h, what) : download_row_offsets<int>(h, what);
-      if (rc || finish_create(h, nullptr, 0)) {
-            spmv_b200_csr_destroy(h);
-            return nullptr;
-      }
-      csr_measure_span(h);
-      return h;
+      return csr_finish(h, rc, nullptr, 0, what);
 }
 
 template <typename IdxT>
@@ -2352,13 +2320,11 @@ extern "C" spmv_b200_hll *spmv_b200_hll_from_csr(const spmv_b200_csr *A) {
             int *d_width = nullptr;
             ok = cudaMalloc(&d_width, (size_t)h->n_hacks * sizeof(int)) == cudaSuccess;
             if (ok) {
-                  const int grid = blocks_for(h->n_hacks * 32, 256);
-                  if (A->wide)
-                        hll_width_kernel<long long><<<grid, 256>>>((const long long *)A->d_irp, A->M,
-                                                                   h->n_hacks, d_width);
-                  else
-                        hll_width_kernel<int><<<grid, 256>>>((const int *)A->d_irp, A->M,
-                                                             h->n_hacks, d_width);
+                  with_offsets(A->wide, [&](auto t) {
+                        using OffT = typename decltype(t)::type;
+                        hll_width_kernel<OffT><<<blocks_for(h->n_hacks * 32, 256), 256>>>(
+                            (const OffT *)A->d_irp, A->M, h->n_hacks, d_width);
+                  });
                   ++g_counters.launches;
                   ok = cudaMemcpy(width.data(), d_width, (size_t)h->n_hacks * sizeof(int),
                                   cudaMemcpyDeviceToHost) == cudaSuccess;
@@ -2369,16 +2335,12 @@ extern "C" spmv_b200_hll *spmv_b200_hll_from_csr(const spmv_b200_csr *A) {
       }
       ok = ok && hll_alloc(h, width) == 0;
       if (ok && h->n_hacks > 0) {
-            const int grid = blocks_for(h->n_hacks * 32, 256);
-            if (A->wide)
-                  hll_fill_from_csr_kernel<long long><<<grid, 256>>>(
-                      (const long long *)A->d_irp, A->d_ja, A->d_as, A->M, h->n_hacks, h->d_hoff,
-                      h->d_ja, h->d_as, h->d_rowlen);
-            else
-                  hll_fill_from_csr_kernel<int><<<grid, 256>>>((const int *)A->d_irp, A->d_ja,
-                                                               A->d_as, A->M, h->n_hacks,
-                                                               h->d_hoff, h->d_ja, h->d_as,
-                                                               h->d_rowlen);
+            with_offsets(A->wide, [&](auto t) {
+                  using OffT = typename decltype(t)::type;
+                  hll_fill_from_csr_kernel<OffT><<<blocks_for(h->n_hacks * 32, 256), 256>>>(
+                      (const OffT *)A->d_irp, A->d_ja, A->d_as, A->M, h->n_hacks, h->d_hoff, h->d_ja,
+                      h->d_as, h->d_rowlen);
+            });
             ++g_counters.launches;
             cudaError_t e = cudaDeviceSynchronize();
             if (e != cudaSuccess) {
