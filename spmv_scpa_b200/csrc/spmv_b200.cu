@@ -9,6 +9,8 @@
 #include "internal.cuh"
 
 #include <cub/cub.cuh>
+#include <memory>
+#include <new>
 
 #include "coo_kernels.cuh"
 #include "csr_kernels.cuh"
@@ -77,6 +79,59 @@ int ensure_device() {
 namespace {
 void *g_flush_buf[kMaxDevices] = {nullptr};
 constexpr size_t kFlushBytes = 512ull << 20; // > 126 MB L2
+} // namespace
+
+// ============================================================ build helpers
+namespace {
+
+template <typename T> struct OffTag { using type = T; };
+
+// f(OffTag<OffT>{}) with OffT the row offset type of a handle: long long when `wide`, else int.
+template <typename F> auto with_offsets(bool wide, F &&f) {
+      return wide ? f(OffTag<long long>{}) : f(OffTag<int>{});
+}
+
+// Device temporaries of one build, freed on every way out.
+struct DeviceTemps {
+      std::vector<void *> ptrs;
+      long long bytes = 0; // requested so far, for the -ENOMEM message
+      ~DeviceTemps() { release_all(); }
+      template <typename T>
+      int alloc(T **out, size_t n_bytes, const char *what) {
+            bytes += (long long)n_bytes;
+            void *p = nullptr;
+            if (cudaMalloc(&p, std::max<size_t>(n_bytes, 1)) != cudaSuccess) {
+                  cudaGetLastError(); // clear the allocation error
+                  return fail(-ENOMEM, "%s: cudaMalloc of %lld bytes of temporaries failed", what, bytes);
+            }
+            ptrs.push_back(p);
+            *out = static_cast<T *>(p);
+            return 0;
+      }
+      // alloc() holding a copy of `h`, counted in the h2d bytes as upload() counts it
+      template <typename T>
+      int upload(T **d, const std::vector<T> &h, const char *what) {
+            const size_t n_bytes = h.size() * sizeof(T);
+            if (alloc(d, n_bytes, what))
+                  return -ENOMEM;
+            B200_CUDA(cudaMemcpy(*d, h.data(), n_bytes, cudaMemcpyHostToDevice));
+            g_counters.h2d += (long long)n_bytes;
+            return 0;
+      }
+      void release(const void *p) {
+            for (auto &q : ptrs)
+                  if (q == p) {
+                        cudaFree(q);
+                        q = nullptr;
+                  }
+      }
+      void release_all() {
+            for (void *p : ptrs)
+                  cudaFree(p);
+            ptrs.clear();
+      }
+};
+
 } // namespace
 
 // ================================================================ CSR plans
@@ -480,18 +535,14 @@ double measure_gather_span(const Src &src, long long M, long long N) {
       constexpr long long kBlock = 256;
       const int n = (int)std::min<long long>(kSamples, (M + kBlock - 1) / kBlock);
       const long long stride = std::max<long long>(kBlock, M / n / kBlock * kBlock);
+      DeviceTemps tmp;
       int *d_lo = nullptr, *d_hi = nullptr;
-      if (cudaMalloc(&d_lo, n * sizeof(int)) != cudaSuccess ||
-          cudaMalloc(&d_hi, n * sizeof(int)) != cudaSuccess) {
-            cudaFree(d_lo);
-            cudaGetLastError();
+      if (tmp.alloc(&d_lo, n * sizeof(int), "gather span") || tmp.alloc(&d_hi, n * sizeof(int), "gather span"))
             return 0.0;
-      }
       col_extent_kernel<<<n, 256>>>(src, M, kBlock, stride, n, d_lo, d_hi);
       std::vector<int> lo(n), hi(n);
       cudaMemcpy(lo.data(), d_lo, n * sizeof(int), cudaMemcpyDeviceToHost);
       cudaMemcpy(hi.data(), d_hi, n * sizeof(int), cudaMemcpyDeviceToHost);
-      cudaFree(d_lo), cudaFree(d_hi);
       if (cudaGetLastError() != cudaSuccess)
             return 0.0;
       std::vector<double> span;
@@ -573,7 +624,6 @@ void sell_plan_host(const std::vector<int> &counts, long long M, int K, int sigm
 template <typename Src>
 int sell_build(const Src &src, long long M, long long N, int K, int max_row, SellPlan &sp,
                std::vector<int> *long_rows) {
-      sp.state = -1;
       if (M <= 0 || M >= (1ll << 31) - 64)
             return 0;
       const int sigma = std::max(32, g_knobs.sell_sigma / 32 * 32);
@@ -584,13 +634,17 @@ int sell_build(const Src &src, long long M, long long N, int K, int max_row, Sel
             pb.pc[p] = (int)(N * p / K);
       sp.pc.assign(pb.pc, pb.pc + K + 1);
 
+      DeviceTemps tmp;
       int *d_counts = nullptr;
-      B200_CUDA(cudaMalloc(&d_counts, (size_t)K * M * sizeof(int)));
+      if (tmp.alloc(&d_counts, (size_t)K * M * sizeof(int), "SELL row counts"))
+            return -ENOMEM;
       sell_count_kernel<<<blocks_for(M, 256), 256>>>(src, M, pb, max_row, d_counts);
+      cudaError_t e = cudaGetLastError();
+      if (e != cudaSuccess)
+            return fail(-EIO, "SELL count kernel launch failed: %s", cudaGetErrorString(e));
       std::vector<int> counts((size_t)K * M);
-      cudaError_t e = cudaMemcpy(counts.data(), d_counts, counts.size() * sizeof(int),
-                                 cudaMemcpyDeviceToHost);
-      cudaFree(d_counts);
+      e = cudaMemcpy(counts.data(), d_counts, counts.size() * sizeof(int), cudaMemcpyDeviceToHost);
+      tmp.release_all();
       if (e != cudaSuccess)
             return fail(-EIO, "SELL row counts failed: %s", cudaGetErrorString(e));
       g_counters.launches += 1;
@@ -655,7 +709,6 @@ void sell_virtual_rows(const std::vector<long long> &irp, long long M, int chunk
 template <typename Src>
 int sell_build_vrows(const Src &src, const std::vector<long long> &irp, long long M, long long N,
                      int chunk, SellPlan &sp) {
-      sp.state = -1;
       if (M <= 0 || irp[M] + M >= (1ll << 31) - 64)
             return 0;
       const int sigma = std::max(32, g_knobs.sell_sigma / 32 * 32);
@@ -673,10 +726,12 @@ int sell_build_vrows(const Src &src, const std::vector<long long> &irp, long lon
       sp.slots = soff.back();
       sp.n_split_rows = (long long)split_row.size();
       sp.n_partials = split_first.back();
+      static const char *what = "SELL virtual rows";
+      DeviceTemps tmp;
       int *d_perm_v = nullptr, *d_vr_row = nullptr, *d_vr_j0 = nullptr;
-      int rc = upload(&d_perm_v, perm_v);
-      rc = rc ? rc : upload(&d_vr_row, vr_row);
-      rc = rc ? rc : upload(&d_vr_j0, vr_j0);
+      int rc = tmp.upload(&d_perm_v, perm_v, what);
+      rc = rc ? rc : tmp.upload(&d_vr_row, vr_row, what);
+      rc = rc ? rc : tmp.upload(&d_vr_j0, vr_j0, what);
       rc = rc ? rc : upload(&sp.d_perm, perm_dest);
       rc = rc ? rc : upload(&sp.d_soff, soff);
       if (!rc && sp.n_split_rows) {
@@ -688,17 +743,14 @@ int sell_build_vrows(const Src &src, const std::vector<long long> &irp, long lon
       if (!rc && (cudaMalloc(&sp.d_ja, ((size_t)sp.slots + 32) * sizeof(int)) != cudaSuccess ||
                   cudaMalloc(&sp.d_as, ((size_t)sp.slots + 32) * sizeof(double)) != cudaSuccess))
             rc = fail(-ENOMEM, "SELL slices: out of device memory");
-      if (!rc) {
-            sell_fill_vrow_kernel<<<blocks_for(S * 32, 256), 256>>>(src, S, sp.d_soff, d_perm_v, d_vr_row,
-                                                                    d_vr_j0, chunk, sp.d_ja, sp.d_as);
-            g_counters.launches += 1;
-            cudaError_t e = cudaDeviceSynchronize();
-            if (e != cudaSuccess)
-                  rc = fail(-EIO, "SELL fill kernel failed: %s", cudaGetErrorString(e));
-      }
-      cudaFree(d_perm_v), cudaFree(d_vr_row), cudaFree(d_vr_j0);
       if (rc)
             return rc;
+      sell_fill_vrow_kernel<<<blocks_for(S * 32, 256), 256>>>(src, S, sp.d_soff, d_perm_v, d_vr_row, d_vr_j0,
+                                                              chunk, sp.d_ja, sp.d_as);
+      g_counters.launches += 1;
+      cudaError_t e = cudaDeviceSynchronize();
+      if (e != cudaSuccess)
+            return fail(-EIO, "SELL fill kernel failed: %s", cudaGetErrorString(e));
       sp.state = 1;
       return 0;
 }
@@ -775,6 +827,13 @@ bool csr_wants_sell(spmv_b200_csr *h) {
       return sell_panels_for(h->N, h->gather_span) > 1;
 }
 
+// A plan not built (not applicable, or a step failed) holds no device memory and is not tried again.
+int sell_not_built(SellPlan &plan) {
+      free_sell(plan);
+      plan.state = -1;
+      return -1;
+}
+
 // `rhs` right-hand sides share one pass (SpMM): the x a panel must keep in the L2 is rhs times as large
 int csr_build_sell(spmv_b200_csr *h, SellPlan &plan, int rhs) {
       if (plan.state != 0)
@@ -785,26 +844,17 @@ int csr_build_sell(spmv_b200_csr *h, SellPlan &plan, int rhs) {
       const bool ragged = !h->segs.empty() && !h->segs[0].regular;
       const int K = ragged && g_knobs.sell_panels <= 0 ? 1 : sell_panels_for(h->N * rhs, h->gather_span);
       // virtual rows: ragged matrices, or any one-panel plan when SELL-P is forced by the knob
-      if ((ragged || g_knobs.sell == 1) && K == 1 && g_knobs.sell_panels <= 0 && g_knobs.sell_chunk > 0) {
-            int rc;
-            if (h->wide)
-                  rc = sell_build_vrows(CsrSrc<long long>{(const long long *)h->d_irp, h->d_ja, h->d_as},
-                                        h->h_irp, h->M, h->N, g_knobs.sell_chunk, plan);
-            else
-                  rc = sell_build_vrows(CsrSrc<int>{(const int *)h->d_irp, h->d_ja, h->d_as}, h->h_irp,
-                                        h->M, h->N, g_knobs.sell_chunk, plan);
-            return rc || plan.state != 1 ? -1 : 0;
-      }
-      std::vector<int> long_rows;
-      int rc;
-      if (h->wide)
-            rc = sell_build(CsrSrc<long long>{(const long long *)h->d_irp, h->d_ja, h->d_as}, h->M,
-                            h->N, K, g_knobs.sell_max_row, plan, &long_rows);
-      else
-            rc = sell_build(CsrSrc<int>{(const int *)h->d_irp, h->d_ja, h->d_as}, h->M, h->N, K,
-                            g_knobs.sell_max_row, plan, &long_rows);
+      const bool vrows =
+          (ragged || g_knobs.sell == 1) && K == 1 && g_knobs.sell_panels <= 0 && g_knobs.sell_chunk > 0;
+      std::vector<int> long_rows; // stays empty for virtual rows: no row is too long for them
+      const int rc = with_offsets(h->wide, [&](auto t) {
+            using OffT = typename decltype(t)::type;
+            const CsrSrc<OffT> src{(const OffT *)h->d_irp, h->d_ja, h->d_as};
+            return vrows ? sell_build_vrows(src, h->h_irp, h->M, h->N, g_knobs.sell_chunk, plan)
+                         : sell_build(src, h->M, h->N, K, g_knobs.sell_max_row, plan, &long_rows);
+      });
       if (rc || plan.state != 1)
-            return -1;
+            return sell_not_built(plan);
       // rows too long for a slice: a warp per row up to 2048 entries, a CTA per row up to 65 536,
       // split into chunks beyond (the bins of the direct path)
       std::vector<int> wrp, blk, spl;
@@ -816,11 +866,8 @@ int csr_build_sell(spmv_b200_csr *h, SellPlan &plan, int rhs) {
       plan.long_warp.n = (long long)wrp.size();
       plan.long_block.n = (long long)blk.size();
       if (upload(&plan.long_warp.d_rows, wrp) || upload(&plan.long_block.d_rows, blk) ||
-          build_split(h, spl, plan.long_split)) {
-            free_sell(plan);
-            plan.state = -1;
-            return -1;
-      }
+          build_split(h, spl, plan.long_split))
+            return sell_not_built(plan);
       return 0;
 }
 
@@ -1079,14 +1126,15 @@ static __global__ void col_minmax_kernel(const int *__restrict__ ja, long long n
 int csr_check_columns(const spmv_b200_csr *h) {
       if (h->NZ == 0)
             return 0;
+      DeviceTemps tmp;
       int *d = nullptr;
       const int init[2] = {0x7fffffff, -0x7fffffff - 1};
       int got[2];
-      B200_CUDA(cudaMalloc(&d, 2 * sizeof(int)));
+      if (tmp.alloc(&d, sizeof init, "column check"))
+            return -ENOMEM;
       B200_CUDA(cudaMemcpy(d, init, sizeof init, cudaMemcpyHostToDevice));
       col_minmax_kernel<<<(int)std::min<long long>(1184, (h->NZ + 255) / 256), 256>>>(h->d_ja, h->NZ, d);
       cudaError_t e = cudaMemcpy(got, d, sizeof got, cudaMemcpyDeviceToHost);
-      cudaFree(d);
       if (e != cudaSuccess)
             return fail(-EIO, "column check failed: %s", cudaGetErrorString(e));
       if (got[0] < 0 || got[1] >= h->N)
@@ -1123,47 +1171,6 @@ int hll_max_col(const spmv_b200_hll *h, long long hack0, long long hack1, int *o
 } // namespace b200
 
 // --------------------------------------------------------------- creation --
-namespace {
-
-template <typename T> struct OffTag { using type = T; };
-
-// f(OffTag<OffT>{}) with OffT the row offset type of a handle: long long when `wide`, else int.
-template <typename F> auto with_offsets(bool wide, F &&f) {
-      return wide ? f(OffTag<long long>{}) : f(OffTag<int>{});
-}
-
-// Device temporaries of one build, freed on every way out.
-struct DeviceTemps {
-      std::vector<void *> ptrs;
-      long long bytes = 0; // requested so far, for the -ENOMEM message
-      ~DeviceTemps() { release_all(); }
-      template <typename T>
-      int alloc(T **out, size_t n_bytes, const char *what) {
-            bytes += (long long)n_bytes;
-            void *p = nullptr;
-            if (cudaMalloc(&p, std::max<size_t>(n_bytes, 1)) != cudaSuccess) {
-                  cudaGetLastError(); // clear the allocation error
-                  return fail(-ENOMEM, "%s: cudaMalloc of %lld bytes of temporaries failed", what, bytes);
-            }
-            ptrs.push_back(p);
-            *out = static_cast<T *>(p);
-            return 0;
-      }
-      void release(const void *p) {
-            for (auto &q : ptrs)
-                  if (q == p) {
-                        cudaFree(q);
-                        q = nullptr;
-                  }
-      }
-      void release_all() {
-            for (void *p : ptrs)
-                  cudaFree(p);
-            ptrs.clear();
-      }
-};
-
-} // namespace
 
 static void csr_measure_span(spmv_b200_csr *h) {
       h->gather_span = with_offsets(h->wide, [&](auto t) {
@@ -2077,7 +2084,7 @@ int hll_ensure_sell(spmv_b200_hll *h) {
             return h->sell.state == 1 ? 0 : -1;
       const int K = sell_panels_for(h->N, h->gather_span);
       int rc = sell_build(hll_src(h), h->M, h->N, K, 0x7fffffff, h->sell, nullptr);
-      return rc || h->sell.state != 1 ? -1 : 0;
+      return rc || h->sell.state != 1 ? sell_not_built(h->sell) : 0;
 }
 
 } // namespace
@@ -2220,6 +2227,66 @@ int hll_run_range(spmv_b200_hll *h, int kernel, int wpb, long long hack0, long l
 
 } // namespace b200
 
+static spmv_b200_hll *hll_alloc_shell(long long M, long long N, long long NZ, long long n_hacks, int device) {
+      auto *h = new spmv_b200_hll();
+      h->M = M, h->N = N, h->NZ = NZ, h->n_hacks = n_hacks, h->device = device;
+      return h;
+}
+
+// Both HLL constructors return through here once the shell exists.  rc != 0: a step failed (fail()
+// has set the message), so the shell is destroyed.  Otherwise the fill is waited for (`what` names
+// it if it failed) and the handle takes `span` as its gather span, or measures it when `span` < 0.
+static spmv_b200_hll *hll_finish(spmv_b200_hll *h, int rc, double span, const char *what) {
+      const cudaError_t e = rc ? cudaSuccess : cudaDeviceSynchronize();
+      if (e != cudaSuccess)
+            rc = fail(-EIO, "%s failed: %s", what, cudaGetErrorString(e));
+      if (rc) {
+            spmv_b200_hll_destroy(h);
+            return nullptr;
+      }
+      h->gather_span = span >= 0 ? span : measure_gather_span(hll_src(h), h->M, h->N);
+      return h;
+}
+
+// Gather the per-hack host arrays into one staging copy (hack b from slot src_off[b]), ship it, and
+// let the GPU transpose / re-stride / patch the pads.
+static int hll_fill_from_host(spmv_b200_hll *h, const sparse_hll *H, const std::vector<long long> &src_off,
+                              int is_col_major) {
+      static const char *what = "HLL upload";
+      const long long src_slots = src_off.back();
+      // not std::vector: its zero fill would be one more pass over the matrix
+      std::unique_ptr<int[]> st_ja(new (std::nothrow) int[src_slots]);
+      std::unique_ptr<double[]> st_as(new (std::nothrow) double[src_slots]);
+      if (!st_ja || !st_as)
+            return fail(-ENOMEM, "host staging allocation failed (%lld slots)", src_slots);
+#pragma omp parallel for schedule(static, 256)
+      for (long long b = 0; b < h->n_hacks; ++b) {
+            const size_t n = (size_t)(src_off[b + 1] - src_off[b]);
+            memcpy(st_ja.get() + src_off[b], H->blocks[b].JA, n * sizeof(int));
+            memcpy(st_as.get() + src_off[b], H->blocks[b].AS, n * sizeof(double));
+      }
+      DeviceTemps tmp;
+      int *d_sja = nullptr;
+      double *d_sas = nullptr;
+      long long *d_soff = nullptr;
+      if (tmp.alloc(&d_sja, (size_t)src_slots * sizeof(int), what) ||
+          tmp.alloc(&d_sas, (size_t)src_slots * sizeof(double), what) ||
+          tmp.alloc(&d_soff, src_off.size() * sizeof(long long), what))
+            return -ENOMEM;
+      cudaError_t e = cudaMemcpy(d_sja, st_ja.get(), (size_t)src_slots * sizeof(int), cudaMemcpyHostToDevice);
+      if (e == cudaSuccess)
+            e = cudaMemcpy(d_sas, st_as.get(), (size_t)src_slots * sizeof(double), cudaMemcpyHostToDevice);
+      if (e == cudaSuccess)
+            e = cudaMemcpy(d_soff, src_off.data(), src_off.size() * sizeof(long long), cudaMemcpyHostToDevice);
+      if (e != cudaSuccess)
+            return fail(-EIO, "HLL upload failed: %s", cudaGetErrorString(e));
+      g_counters.h2d += src_slots * 12;
+      hll_fill_from_host_layout_kernel<<<blocks_for(h->n_hacks * 32, 256), 256>>>(
+          d_soff, d_sja, d_sas, is_col_major, h->M, h->n_hacks, h->d_hoff, h->d_ja, h->d_as, h->d_rowlen);
+      ++g_counters.launches;
+      return 0;
+}
+
 extern "C" spmv_b200_hll *spmv_b200_hll_create(const sparse_hll *H, int is_col_major) {
       if (ensure_device())
             return nullptr;
@@ -2231,74 +2298,19 @@ extern "C" spmv_b200_hll *spmv_b200_hll_create(const sparse_hll *H, int is_col_m
             fail(-EINVAL, "hack_size %d unsupported (library is built for 32)", H->hack_size);
             return nullptr;
       }
-      auto *h = new spmv_b200_hll();
-      cudaGetDevice(&h->device);
-      h->M = H->M, h->N = H->N, h->NZ = H->NZ, h->n_hacks = H->num_blocks;
+      int device = 0;
+      cudaGetDevice(&device);
+      spmv_b200_hll *h = hll_alloc_shell(H->M, H->N, H->NZ, H->num_blocks, device);
       std::vector<int> width((size_t)h->n_hacks);
       std::vector<long long> src_off((size_t)h->n_hacks + 1, 0);
       for (long long b = 0; b < h->n_hacks; ++b) {
             width[b] = H->blocks[b].max_NZ;
             src_off[b + 1] = src_off[b] + (long long)H->blocks[b].M * H->blocks[b].max_NZ;
       }
-      const long long src_slots = src_off[h->n_hacks];
-
-      // Gather the per-hack host arrays into one staging copy, ship it, and
-      // let the GPU transpose / re-stride / patch the pads.
-      int *st_ja = nullptr, *d_sja = nullptr;
-      double *st_as = nullptr, *d_sas = nullptr;
-      long long *d_soff = nullptr;
-      bool ok = hll_alloc(h, width) == 0;
-      if (ok && src_slots > 0) {
-            st_ja = (int *)malloc((size_t)src_slots * sizeof(int));
-            st_as = (double *)malloc((size_t)src_slots * sizeof(double));
-            ok = st_ja && st_as;
-            if (!ok)
-                  fail(-ENOMEM, "host staging allocation failed (%lld slots)", src_slots);
-      }
-      if (ok && src_slots > 0) {
-#pragma omp parallel for schedule(static, 256)
-            for (long long b = 0; b < h->n_hacks; ++b) {
-                  const size_t n = (size_t)(src_off[b + 1] - src_off[b]);
-                  memcpy(st_ja + src_off[b], H->blocks[b].JA, n * sizeof(int));
-                  memcpy(st_as + src_off[b], H->blocks[b].AS, n * sizeof(double));
-            }
-            ok = cudaMalloc(&d_sja, (size_t)src_slots * sizeof(int)) == cudaSuccess &&
-                 cudaMalloc(&d_sas, (size_t)src_slots * sizeof(double)) == cudaSuccess &&
-                 cudaMalloc(&d_soff, src_off.size() * sizeof(long long)) == cudaSuccess &&
-                 cudaMemcpy(d_sja, st_ja, (size_t)src_slots * sizeof(int),
-                            cudaMemcpyHostToDevice) == cudaSuccess &&
-                 cudaMemcpy(d_sas, st_as, (size_t)src_slots * sizeof(double),
-                            cudaMemcpyHostToDevice) == cudaSuccess &&
-                 cudaMemcpy(d_soff, src_off.data(), src_off.size() * sizeof(long long),
-                            cudaMemcpyHostToDevice) == cudaSuccess;
-            if (!ok)
-                  fail(-EIO, "HLL upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-            g_counters.h2d += src_slots * 12;
-      }
-      if (ok && h->n_hacks > 0) {
-            if (!d_soff) // every hack is empty: the kernel still writes the row lengths
-                  ok = cudaMalloc(&d_soff, src_off.size() * sizeof(long long)) == cudaSuccess &&
-                       cudaMemcpy(d_soff, src_off.data(), src_off.size() * sizeof(long long),
-                                  cudaMemcpyHostToDevice) == cudaSuccess;
-            if (ok)
-                  hll_fill_from_host_layout_kernel<<<blocks_for(h->n_hacks * 32, 256), 256>>>(
-                      d_soff, d_sja, d_sas, is_col_major, h->M, h->n_hacks, h->d_hoff, h->d_ja,
-                      h->d_as, h->d_rowlen);
-            ++g_counters.launches;
-            cudaError_t e = cudaDeviceSynchronize();
-            if (e != cudaSuccess) {
-                  ok = false;
-                  fail(-EIO, "HLL layout kernel failed: %s", cudaGetErrorString(e));
-            }
-      }
-      free(st_ja), free(st_as);
-      cudaFree(d_sja), cudaFree(d_sas), cudaFree(d_soff);
-      if (!ok) {
-            spmv_b200_hll_destroy(h);
-            return nullptr;
-      }
-      h->gather_span = measure_gather_span(hll_src(h), h->M, h->N);
-      return h;
+      int rc = hll_alloc(h, width);
+      if (!rc && h->n_hacks > 0)
+            rc = hll_fill_from_host(h, H, src_off, is_col_major);
+      return hll_finish(h, rc, -1.0, "HLL layout kernel");
 }
 
 extern "C" spmv_b200_hll *spmv_b200_hll_from_csr(const spmv_b200_csr *A) {
@@ -2308,33 +2320,30 @@ extern "C" spmv_b200_hll *spmv_b200_hll_from_csr(const spmv_b200_csr *A) {
             fail(-EINVAL, "null CSR handle");
             return nullptr;
       }
-      auto *h = new spmv_b200_hll();
-      h->device = A->device;
-      h->M = A->M, h->N = A->N, h->NZ = A->NZ;
-      h->n_hacks = (A->M + kHack - 1) / kHack;
+      spmv_b200_hll *h = hll_alloc_shell(A->M, A->N, A->NZ, (A->M + kHack - 1) / kHack, A->device);
       // hack widths (longest row of each hack) on the GPU; the host only needs them for the
       // prefix sum that sizes the buffers
       std::vector<int> width((size_t)h->n_hacks, 0);
-      bool ok = true;
+      int rc = 0;
       if (h->n_hacks > 0) {
+            DeviceTemps tmp;
             int *d_width = nullptr;
-            ok = cudaMalloc(&d_width, (size_t)h->n_hacks * sizeof(int)) == cudaSuccess;
-            if (ok) {
+            rc = tmp.alloc(&d_width, width.size() * sizeof(int), "hack widths");
+            if (!rc) {
                   with_offsets(A->wide, [&](auto t) {
                         using OffT = typename decltype(t)::type;
                         hll_width_kernel<OffT><<<blocks_for(h->n_hacks * 32, 256), 256>>>(
                             (const OffT *)A->d_irp, A->M, h->n_hacks, d_width);
                   });
                   ++g_counters.launches;
-                  ok = cudaMemcpy(width.data(), d_width, (size_t)h->n_hacks * sizeof(int),
-                                  cudaMemcpyDeviceToHost) == cudaSuccess;
+                  const cudaError_t e =
+                      cudaMemcpy(width.data(), d_width, width.size() * sizeof(int), cudaMemcpyDeviceToHost);
+                  if (e != cudaSuccess)
+                        rc = fail(-EIO, "hack width kernel failed: %s", cudaGetErrorString(e));
             }
-            cudaFree(d_width);
-            if (!ok)
-                  fail(-EIO, "hack width kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
       }
-      ok = ok && hll_alloc(h, width) == 0;
-      if (ok && h->n_hacks > 0) {
+      rc = rc ? rc : hll_alloc(h, width);
+      if (!rc && h->n_hacks > 0) {
             with_offsets(A->wide, [&](auto t) {
                   using OffT = typename decltype(t)::type;
                   hll_fill_from_csr_kernel<OffT><<<blocks_for(h->n_hacks * 32, 256), 256>>>(
@@ -2342,18 +2351,8 @@ extern "C" spmv_b200_hll *spmv_b200_hll_from_csr(const spmv_b200_csr *A) {
                       h->d_as, h->d_rowlen);
             });
             ++g_counters.launches;
-            cudaError_t e = cudaDeviceSynchronize();
-            if (e != cudaSuccess) {
-                  ok = false;
-                  fail(-EIO, "CSR->HLL kernel failed: %s", cudaGetErrorString(e));
-            }
       }
-      if (!ok) {
-            spmv_b200_hll_destroy(h);
-            return nullptr;
-      }
-      h->gather_span = A->gather_span;
-      return h;
+      return hll_finish(h, rc, A->gather_span, "CSR->HLL kernel");
 }
 
 extern "C" void spmv_b200_hll_destroy(spmv_b200_hll *h) {
