@@ -130,6 +130,24 @@ spmv_b200_csr *spmv_b200_csr_gen_stencil27(int nx, int ny, int nz, int z0,
  * failure; -ENOTSUP for 2^31 or more entries. */
 spmv_b200_csr *spmv_b200_csr_transpose(const spmv_b200_csr *A);
 
+/* C = A * B of two resident CSR handles, built on their device as a new resident CSR.
+ * Shape: C has A's M rows and B's N columns (N is n_local for a shard: a shard multiplies its
+ * local block); it needs A.N == B.M.  C has col_offset 0 and no cuts.
+ * Pattern: row i of C lists each column j once, in increasing column order, for every (i, j) with
+ * at least one product, even when the sum is zero; explicit zeros of the inputs still produce
+ * entries.  The inputs may have unsorted rows and repeated (row, col) entries.
+ * Values: the products of row i are taken in the order p over A's row i, then q over B's row
+ * ja_A[p], both in stored order; C[i][j] is the left-to-right sum of those that land in column j,
+ * starting from the first, each product a_p * b_q rounded to FP64 before it is added (no fused
+ * multiply-add).  So a lone -0.0 stays -0.0, NaN and Inf propagate, and the result is the same on
+ * every run.
+ * Synchronous, on A's device (the current device is restored); A and B are unchanged; destroy all
+ * three handles separately.  Row offsets of either input may be 32- or 64-bit, and the number of
+ * products may exceed 2^31.  NULL + last_error on failure: -EINVAL for a null handle, A.N != B.M
+ * or handles on different devices; -ENOTSUP when C would have 2^31 - 64 or more entries (found
+ * before C is allocated); -ENOMEM when the temporaries do not fit. */
+spmv_b200_csr *spmv_b200_csr_spgemm(const spmv_b200_csr *A, const spmv_b200_csr *B);
+
 #define SPMV_B200_COO_SUM_DUPLICATES 1
 /* Resident CSR from n entries (d_row[k], d_col[k], d_val[k]) in device memory of the current
  * device.  idx_bytes = 4 or 8 (both index arrays; torch indices are int64).  Row r of the result

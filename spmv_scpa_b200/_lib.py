@@ -97,6 +97,7 @@ _sig(b200, "spmv_b200_csr_create_ex", vp, c_i64, c_i64, c_i64, vp, C.c_int, c_ip
 _sig(b200, "spmv_b200_csr_gen_stencil27", vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_i64,
      c_i64, c_i64p, C.c_int)
 _sig(b200, "spmv_b200_csr_transpose", vp, vp)
+_sig(b200, "spmv_b200_csr_spgemm", vp, vp, vp)
 _sig(b200, "spmv_b200_csr_from_coo", vp, c_i64, c_i64, c_i64, vp, vp, C.c_int, vp, C.c_int, vp)
 _sig(b200, "spmv_b200_csr_rows", c_i64, vp)
 _sig(b200, "spmv_b200_csr_cols", c_i64, vp)

@@ -555,6 +555,18 @@ class CsrDevice:
         block.  Both handles are independent."""
         return CsrDevice(L.b200.spmv_b200_csr_transpose(self._h))
 
+    def matmul(self, B):
+        """C = A·B as a new resident CSR built on the GPU (spmv_b200_csr_spgemm): M rows, B.N
+        columns, each row's columns once in increasing order, explicit zeros kept.  C[i][j] is the
+        left-to-right sum, in FP64 without fused multiply-adds, of the products a_p·b_q landing in
+        column j, taken for p in A's row i and q in B's row ja_A[p], both in stored order.  A shard
+        multiplies its local block.  All three handles are independent."""
+        if not isinstance(B, CsrDevice):
+            raise TypeError(f"B must be a CsrDevice, got {type(B).__name__}")
+        if self.N != B.M:
+            raise ValueError(f"A has {self.N} columns but B has {B.M} rows")
+        return CsrDevice(L.b200.spmv_b200_csr_spgemm(self._h, B._h))
+
     def close(self):
         if self._h:
             L.b200.spmv_b200_csr_destroy(self._h)

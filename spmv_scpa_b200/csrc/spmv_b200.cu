@@ -17,6 +17,7 @@
 #include "gen_kernels.cuh"
 #include "hll_kernels.cuh"
 #include "sell_kernels.cuh"
+#include "spgemm_kernels.cuh"
 #include "transpose_kernels.cuh"
 
 using namespace b200;
@@ -1654,6 +1655,240 @@ extern "C" spmv_b200_csr *spmv_b200_csr_from_coo(int64_t M, int64_t N, int64_t n
       cudaStream_t st = static_cast<cudaStream_t>(stream);
       return idx_bytes == 4 ? csr_from_coo_idx<int>(M, N, n, d_row, d_col, d_val, sum, st)
                             : csr_from_coo_idx<long long>(M, N, n, d_row, d_col, d_val, sum, st);
+}
+
+// -------------------------------------------------------------- product --
+namespace {
+// Hash tables of the product (spgemm_kernels.cuh): a row's table has the least power of two slots
+// that is >= 2 min(P_i, B.N) and >= kSpgemmMinSlots, at most 2^31.  Tables of up to
+// kSpgemmSharedSlots slots are per warp in shared memory, one launch per size; larger ones are
+// regions of one global table.
+constexpr long long kSpgemmMinSlots = 32;
+constexpr long long kSpgemmSharedSlots = 4096;
+constexpr int kSpgemmSharedBins = 8; // 32, 64, ..., 4096 slots
+constexpr int kSpgemmGlobalWarps = 4;
+
+// Warps per block of a shared-table launch: 8192 slots per block (98 KB of keys, values and
+// staging at 4096 slots in the numeric pass), at most 8 warps.
+int spgemm_warps(long long slots) { return (int)std::min<long long>(8, std::max<long long>(1, 8192 / slots)); }
+
+long long spgemm_slots(long long P, long long N) {
+      const long long b = 2 * std::min(P, N);
+      long long s = kSpgemmMinSlots;
+      if (b > s)
+            s = 1ll << (64 - __builtin_clzll((unsigned long long)(b - 1)));
+      return std::min(s, 1ll << 31);
+}
+} // namespace
+
+// C = A * B on the current device (A's).  Steps, all on the legacy default stream:
+//   count     P_i for every row of A, read back (8 bytes per row) and binned on the host by table
+//             size; rows with P_i = 0 are empty in C and run nowhere;
+//   symbolic  entries per row of C and their 64-bit sum (read back, so that 2^31 - 64 or more
+//             entries fail before C is allocated);
+//   numeric   the rows of C, each in slot order, at C's row offsets (the scan of the counts) in two
+//             temporary arrays;
+//   sort      cub::DeviceSegmentedSort orders each row by column into C's arrays.
+// Temporary memory besides the new handle: 8 bytes per row of A (P) + 4 per row (+ 4) for the
+// counts + 4 per row with products (the binned rows) + 12 per global-table slot and 8 per row
+// that has one + 12 per entry of C (the unsorted rows), plus CUB's scratch.
+static spmv_b200_csr *csr_spgemm_here(const spmv_b200_csr *A, const spmv_b200_csr *B) {
+      static const char *what = "spgemm";
+      const long long M = A->M, lim = (1ll << 31) - 64;
+      DeviceTemps tmp;
+      long long *d_P = nullptr;
+      if (tmp.alloc(&d_P, M * sizeof(long long), what))
+            return nullptr;
+      cudaError_t e = cudaSuccess;
+      if (M > 0) {
+            const int grid = (int)std::min<long long>(blocks_for(M * 32, 256), 65535ll * 8);
+            with_offsets(A->wide, [&](auto ta) {
+                  with_offsets(B->wide, [&](auto tb) {
+                        using OffA = typename decltype(ta)::type;
+                        using OffB = typename decltype(tb)::type;
+                        spgemm_count_kernel<OffA, OffB>
+                            <<<grid, 256>>>((const OffA *)A->d_irp, A->d_ja, M, (const OffB *)B->d_irp, d_P);
+                  });
+            });
+            ++g_counters.launches;
+            e = cudaGetLastError();
+      }
+      std::vector<long long> P((size_t)M);
+      if (e == cudaSuccess)
+            e = cudaMemcpy(P.data(), d_P, M * sizeof(long long), cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess) {
+            fail(-EIO, "spgemm: product count failed: %s", cudaGetErrorString(e));
+            return nullptr;
+      }
+      g_counters.d2h += M * (long long)sizeof(long long);
+      tmp.release(d_P);
+
+      // bins: kSpgemmSharedBins shared-table sizes, then the global-table rows; a stable counting
+      // sort of the rows by bin, and the global rows' table regions
+      constexpr int kBins = kSpgemmSharedBins + 1;
+      auto bin_of = [&](long long p) {
+            const long long s = spgemm_slots(p, B->N);
+            return s > kSpgemmSharedSlots ? kSpgemmSharedBins : 63 - __builtin_clzll((unsigned long long)s) - 5;
+      };
+      long long start[kBins + 1] = {0};
+      for (long long r = 0; r < M; ++r)
+            if (P[r] > 0)
+                  ++start[bin_of(P[r]) + 1];
+      for (int b = 0; b < kBins; ++b)
+            start[b + 1] += start[b];
+      std::vector<int> rows((size_t)start[kBins]);
+      std::vector<long long> toff(1, 0);
+      long long fill[kBins];
+      std::copy(start, start + kBins, fill);
+      for (long long r = 0; r < M; ++r) {
+            if (P[r] <= 0)
+                  continue;
+            const int b = bin_of(P[r]);
+            rows[fill[b]++] = (int)r;
+            if (b == kSpgemmSharedBins)
+                  toff.push_back(toff.back() + spgemm_slots(P[r], B->N));
+      }
+      std::vector<long long>().swap(P);
+
+      int *d_rows = nullptr, *d_count = nullptr, *gkeys = nullptr;
+      long long *d_toff = nullptr;
+      double *gvals = nullptr;
+      unsigned long long *d_total = nullptr;
+      const long long gslots = toff.back();
+      if (tmp.upload(&d_rows, rows, what) || tmp.upload(&d_toff, toff, what) ||
+          tmp.alloc(&d_count, (M + 1) * sizeof(int), what) || tmp.alloc(&d_total, sizeof *d_total, what) ||
+          tmp.alloc(&gkeys, gslots * sizeof(int), what) || tmp.alloc(&gvals, gslots * sizeof(double), what))
+            return nullptr;
+      e = cudaMemsetAsync(d_count, 0, (M + 1) * sizeof(int));
+      if (e == cudaSuccess)
+            e = cudaMemsetAsync(d_total, 0, sizeof *d_total);
+
+      // one pass (symbolic or numeric) over every non-empty bin
+      auto pass = [&](bool numeric, const void *irp_c, bool wide_c, int *t_ja, double *t_as) {
+            cudaError_t pe = cudaSuccess;
+            for (int b = 0; b < kBins && pe == cudaSuccess; ++b) {
+                  const long long n = start[b + 1] - start[b];
+                  if (n == 0)
+                        continue;
+                  const bool shared = b < kSpgemmSharedBins;
+                  const long long slots = shared ? kSpgemmMinSlots << b : 0;
+                  const int wpb = shared ? spgemm_warps(slots) : kSpgemmGlobalWarps;
+                  const size_t smem = shared ? (size_t)wpb * (numeric ? slots * 12 + 256 : slots * 4)
+                                             : (numeric ? (size_t)wpb * 256 : 0);
+                  const int grid = (int)std::min<long long>(blocks_for(n * 32, wpb * 32), (long long)g_sm_count * 64);
+                  const SpgemmRows rs{d_rows + start[b], n, slots, d_toff, gkeys, gvals};
+                  with_offsets(A->wide, [&](auto ta) {
+                        with_offsets(B->wide, [&](auto tb) {
+                              using OffA = typename decltype(ta)::type;
+                              using OffB = typename decltype(tb)::type;
+                              auto go = [&](auto kernel, auto... args) {
+                                    pe = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                              (int)smem);
+                                    if (pe == cudaSuccess) {
+                                          kernel<<<grid, wpb * 32, smem>>>(args...);
+                                          pe = cudaGetLastError();
+                                    }
+                              };
+                              const OffA *ia = (const OffA *)A->d_irp;
+                              const OffB *ib = (const OffB *)B->d_irp;
+                              if (numeric && shared)
+                                    go(spgemm_numeric_kernel<SharedTable, OffA, OffB>, ia, A->d_ja, A->d_as, ib,
+                                       B->d_ja, B->d_as, rs, irp_c, wide_c, t_ja, t_as);
+                              else if (numeric)
+                                    go(spgemm_numeric_kernel<GlobalTable, OffA, OffB>, ia, A->d_ja, A->d_as, ib,
+                                       B->d_ja, B->d_as, rs, irp_c, wide_c, t_ja, t_as);
+                              else if (shared)
+                                    go(spgemm_symbolic_kernel<SharedTable, OffA, OffB>, ia, A->d_ja, ib, B->d_ja, rs,
+                                       d_count, d_total);
+                              else
+                                    go(spgemm_symbolic_kernel<GlobalTable, OffA, OffB>, ia, A->d_ja, ib, B->d_ja, rs,
+                                       d_count, d_total);
+                        });
+                  });
+                  ++g_counters.launches;
+            }
+            return pe;
+      };
+
+      unsigned long long total = 0;
+      if (e == cudaSuccess)
+            e = pass(false, nullptr, false, nullptr, nullptr);
+      if (e == cudaSuccess)
+            e = cudaMemcpy(&total, d_total, sizeof total, cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess) {
+            fail(-EIO, "spgemm: symbolic pass failed: %s", cudaGetErrorString(e));
+            return nullptr;
+      }
+      if ((long long)total >= lim) {
+            fail(-ENOTSUP, "spgemm: products with 2^31 - 64 or more entries are not supported (%llu entries)",
+                 total);
+            return nullptr;
+      }
+      const long long nz = (long long)total;
+
+      spmv_b200_csr *h = csr_alloc_shell(M, B->N, nz, 0, 0);
+      if (!h)
+            return nullptr;
+      int *t_ja = nullptr;
+      double *t_as = nullptr;
+      void *scratch = nullptr;
+      size_t scan_bytes = 0, sort_bytes = 0;
+      auto segsort = [&](void *s, size_t &bytes) {
+            return with_offsets(h->wide, [&](auto t) {
+                  using OffT = typename decltype(t)::type;
+                  const OffT *irp = (const OffT *)h->d_irp;
+                  return cub::DeviceSegmentedSort::SortPairs(s, bytes, t_ja, h->d_ja, t_as, h->d_as, (int)nz, (int)M,
+                                                             irp, irp + 1);
+            });
+      };
+      e = scan_row_offsets(nullptr, scan_bytes, d_count, h);
+      if (e == cudaSuccess && nz > 0)
+            e = segsort(nullptr, sort_bytes);
+      int rc = e == cudaSuccess ? 0 : fail(-EIO, "spgemm: CUB size query failed: %s", cudaGetErrorString(e));
+      if (!rc)
+            rc = tmp.alloc(&scratch, std::max(scan_bytes, sort_bytes), what) ||
+                 tmp.alloc(&t_ja, nz * sizeof(int), what) || tmp.alloc(&t_as, nz * sizeof(double), what);
+      if (!rc) {
+            e = scan_row_offsets(scratch, scan_bytes, d_count, h);
+            ++g_counters.launches;
+            if (e == cudaSuccess)
+                  e = pass(true, h->d_irp, h->wide, t_ja, t_as);
+            if (e == cudaSuccess && nz > 0) {
+                  e = segsort(scratch, sort_bytes);
+                  ++g_counters.launches;
+            }
+            if (e == cudaSuccess)
+                  e = cudaDeviceSynchronize();
+            tmp.release_all();
+            if (e != cudaSuccess)
+                  rc = fail(-EIO, "spgemm failed: %s", cudaGetErrorString(e));
+      }
+      return csr_finish(h, rc, nullptr, 0, what);
+}
+
+extern "C" spmv_b200_csr *spmv_b200_csr_spgemm(const spmv_b200_csr *A, const spmv_b200_csr *B) {
+      if (!A || !B) {
+            fail(-EINVAL, "spgemm: null CSR handle");
+            return nullptr;
+      }
+      if (A->N != B->M) {
+            fail(-EINVAL, "spgemm: A has %lld columns but B has %lld rows", A->N, B->M);
+            return nullptr;
+      }
+      if (A->device != B->device) {
+            fail(-EINVAL, "spgemm: A is on device %d, B on device %d", A->device, B->device);
+            return nullptr;
+      }
+      if (ensure_device())
+            return nullptr;
+      int prev = 0;
+      if (cudaGetDevice(&prev) != cudaSuccess || cudaSetDevice(A->device) != cudaSuccess) {
+            fail(-EIO, "spgemm: cannot select device %d", A->device);
+            return nullptr;
+      }
+      spmv_b200_csr *h = csr_spgemm_here(A, B);
+      cudaSetDevice(prev);
+      return h;
 }
 
 extern "C" void spmv_b200_csr_destroy(spmv_b200_csr *h) {
