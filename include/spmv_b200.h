@@ -173,6 +173,10 @@ int spmv_b200_csr_download(const spmv_b200_csr *h, int64_t *irp64, int *JA,
 /* Rows per adaptive bin: out[0..5] = {empty, sub-warp, warp, block, split,
  * tiles}.  Diagnostic. */
 int spmv_b200_csr_plan_info(const spmv_b200_csr *h, int64_t *out, int n_out);
+/* Column codes of the staged row-tile plans built so far (kernels 2 / 4): out[0..4) = {state
+ * (0 none built, 1 coded, -1 some plan keeps int32 columns: a tile has more than 256 distinct
+ * column offsets), coded tiles, largest dictionary of a tile, bytes of the code blocks}. */
+int spmv_b200_csr_codes_info(const spmv_b200_csr *h, int64_t *out, int n_out);
 
 /* y[0..M) = A * x on `stream` (asynchronous).  d_x has n_local entries. */
 int spmv_b200_csr_spmv(spmv_b200_csr *h, int kernel, int warps_per_block,
@@ -298,7 +302,9 @@ void spmv_b200_counters(int64_t *launches, int64_t *h2d_bytes,
 
 /* Experiment knobs used by bin/kbench sweeps and tests ("csr_stream_cfg", "hll_stream_cfg",
  * "force_wide", "pipeline", "pipe_chunks", "csr_pipe", "hll_pipe" (short rows / narrow hacks
- * through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit), "sell", "sell_panels",
+ * through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit), "csr_codes" (1, the
+ * default: row-tile stream plans stream one-byte column codes where every tile allows; 0: int32
+ * columns), "sell", "sell_panels",
  * "sell_sigma", "sell_panel_mb", "sell_max_row", "sell_chunk", "cache").
  * 0 or -EINVAL.  Knobs that change planning must be set before a handle is created. */
 int spmv_b200_set_knob(const char *key, int value);

@@ -144,6 +144,7 @@ _sig(b200, "spmv_b200_hll_spmv_fused", C.c_int, vp, C.c_int, C.c_int, vp, vp, C.
 _sig(b200, "spmv_b200_csr_spmv_host", C.c_int, vp, C.c_int, C.c_int, vp, vp, c_dp)
 _sig(b200, "spmv_b200_hll_spmv_host", C.c_int, vp, C.c_int, C.c_int, vp, vp, c_dp)
 _sig(b200, "spmv_b200_csr_sell_info", C.c_int, vp, C.c_int, c_i64p, C.c_int)
+_sig(b200, "spmv_b200_csr_codes_info", C.c_int, vp, c_i64p, C.c_int)
 _sig(b200, "spmv_b200_hll_sell_info", C.c_int, vp, C.c_int, c_i64p, C.c_int)
 _sig(b200, "spmv_b200_sell_plan", C.c_int, c_ip, c_i64, C.c_int, C.c_int, c_ip, c_i64p)
 _sig(b200, "spmv_b200_sell_plan_vrows", C.c_int, c_i64p, c_i64, C.c_int, C.c_int, c_i64p, c_ip, c_i64p)

@@ -509,6 +509,14 @@ class CsrDevice:
                 "chunk", "split_rows", "pieces")
         return dict(zip(keys, list(out)))
 
+    def codes_info(self):
+        """Column codes of the staged row-tile plans built so far (spmv_b200_csr_codes_info):
+        state (0 none built, 1 coded, -1 a plan keeps int32 columns), coded tiles, the largest
+        dictionary of a tile and the bytes of the code blocks."""
+        out = (C.c_int64 * 4)()
+        self._check(L.b200.spmv_b200_csr_codes_info(self._h, out, 4))
+        return dict(zip(("state", "tiles", "max_dict", "bytes"), list(out)))
+
     def sell_download(self):
         info = self.sell_info()
         assert info["state"] == 1, "no SELL-P plan on this handle"

@@ -220,29 +220,49 @@ __global__ void csr_combine_kernel(const int *__restrict__ split_row,
 // few contiguous sectors (ELL-like access on CSR).  For even row lengths the
 // walk through the row is rotated by the row's index so lanes start in
 // different shared-memory banks.
+//
+// Column codes (CODES = true, row-tile mode only): in place of the int32
+// index stream a tile brings one block, built once per plan by
+// stream_codes_kernel: a uint8 code per staged entry, in the positions of
+// the value stage, padded to 16 bytes, then the tile's dictionary of
+// distinct column offsets d = col - row (int32, ascending, at most
+// kCodeDict, padded to 16 bytes).  The column of an entry is row +
+// dict[code], exactly the stored index, so results do not change; a banded
+// or stencil tile streams 9 bytes per entry instead of 12.
 // ------------------------------------------------------------------------
-template <int THREADS, int LPR, int STAGES, int CAP, int PASSES, bool WS, bool SPLIT = false>
+constexpr int kCodeDict = 256; // distinct column offsets a coded tile may hold
+
+__host__ __device__ constexpr long long round16(long long n) { return (n + 15) & ~15ll; }
+
+template <int THREADS, int LPR, int STAGES, int CAP, int PASSES, bool WS, bool SPLIT = false,
+          bool CODES = false>
 struct StreamCfg {
+      static_assert(!(SPLIT && CODES), "column codes exist for the row-tile mode only");
       static constexpr int kConsumers = THREADS;
       static constexpr int kThreads = THREADS + (WS ? 32 : 0);
       static constexpr int kRowsPerPass = THREADS / LPR;
       static constexpr int kMaxRows = kRowsPerPass * PASSES;
-      static constexpr int kCap = CAP; // entries per stage (multiple of 4)
+      static constexpr int kCap = CAP; // entries per stage (multiple of 16)
+      // bytes of the index part of a stage: int32 columns, or a code block
+      static constexpr int kIdxBytes = CODES ? CAP + kCodeDict * 4 : CAP * 4;
       static constexpr int kQueue = CAP / 32 + 8; // rows longer than 32 entries per tile
       static constexpr int kIrpSlots = kMaxRows + 8; // staged row offsets per stage (SPLIT)
       template <typename OffT>
       static constexpr size_t smem() {
-            return (size_t)STAGES * CAP * 12 + 2 * STAGES * 8 + 16 +
+            return (size_t)STAGES * (CAP * 8 + kIdxBytes) + 2 * STAGES * 8 + 16 +
                    (SPLIT ? (size_t)(kQueue + 4) * 4 + 16 + (size_t)STAGES * kIrpSlots * sizeof(OffT) : 0);
       }
 };
 
 // All rows of one staged tile.  `gi` = row slot of this thread, `sub` = lane
-// within the row group.
-template <int LPR, int RPP, int PASSES, int EPI, typename OffT>
+// within the row group.  Columns come from `tja`, or with CODES from
+// row + tdict[tcode[...]].
+template <int LPR, int RPP, int PASSES, int EPI, bool CODES, typename OffT>
 __device__ __forceinline__ void stream_tile_rows(const OffT *__restrict__ irp,
                                                  const double *__restrict__ tas,
-                                                 const int *__restrict__ tja, int r0, int r1,
+                                                 const int *__restrict__ tja,
+                                                 const unsigned char *__restrict__ tcode,
+                                                 const int *__restrict__ tdict, int r0, int r1,
                                                  long long kbase, int gi, int sub, long long ks,
                                                  long long ke, const double *__restrict__ x,
                                                  double *__restrict__ y, uint64_t pol_x,
@@ -279,8 +299,14 @@ __device__ __forceinline__ void stream_tile_rows(const OffT *__restrict__ irp,
                               const int jj = j + u * LPR;
                               const bool ok = jj < to;
                               okm[u] = ok;
-                              c[u] = ok ? tja[base + jj] : 0;
+                              // (codes: the byte now, its dictionary entry in a second sweep)
+                              c[u] = ok ? (CODES ? (int)tcode[base + jj] : tja[base + jj]) : 0;
                               a[u] = ok ? tas[base + jj] : 0.0;
+                        }
+                        if (CODES) {
+#pragma unroll
+                              for (int u = 0; u < U; ++u)
+                                    c[u] = row + tdict[c[u]];
                         }
 #pragma unroll
                         for (int u = 0; u < U; ++u)
@@ -397,21 +423,25 @@ __device__ __forceinline__ void stream_tile_products(const OffT *s_irp, double *
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 
+// code_off / codes: the code blocks of the tiles (CODES only; tile t's block is
+// codes[code_off[t], code_off[t+1])).
 template <int THREADS, int LPR, int STAGES, int CAP, int PASSES, bool WS, bool SPLIT, int EPI,
-          typename OffT>
+          bool CODES, typename OffT>
 __global__ void __launch_bounds__(THREADS + (WS ? 32 : 0))
     csr_stream_kernel(const OffT *__restrict__ irp, const int *__restrict__ ja,
                       const double *__restrict__ as, const int *__restrict__ tile_row,
-                      const long long *__restrict__ tile_k, int tile0, int n_tiles,
+                      const long long *__restrict__ tile_k, const long long *__restrict__ code_off,
+                      const unsigned char *__restrict__ codes, int tile0, int n_tiles,
                       const double *__restrict__ x, double *__restrict__ y, EpiArgs epi) {
+      using Cfg = StreamCfg<THREADS, LPR, STAGES, CAP, PASSES, WS, SPLIT, CODES>;
       extern __shared__ __align__(128) unsigned char smem_raw[];
       double *s_as = reinterpret_cast<double *>(smem_raw);
-      int *s_ja = reinterpret_cast<int *>(smem_raw + (size_t)STAGES * CAP * 8);
-      uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw + (size_t)STAGES * CAP * 12);
+      // index part of the stages: int32 columns, or code blocks
+      unsigned char *s_idx = smem_raw + (size_t)STAGES * CAP * 8;
+      uint64_t *full = reinterpret_cast<uint64_t *>(s_idx + (size_t)STAGES * Cfg::kIdxBytes);
       uint64_t *empty = full + STAGES;
       int *s_queue_n = reinterpret_cast<int *>(empty + STAGES + 1);
       int *s_queue = s_queue_n + 4;
-      using Cfg = StreamCfg<THREADS, LPR, STAGES, CAP, PASSES, WS, SPLIT>;
       // staged row offsets (entry-split mode only), 16-byte aligned
       OffT *s_irp = reinterpret_cast<OffT *>(
           (reinterpret_cast<uintptr_t>(s_queue + Cfg::kQueue) + 15) & ~uintptr_t(15));
@@ -457,12 +487,19 @@ __global__ void __launch_bounds__(THREADS + (WS ? 32 : 0))
                   const int n = (tile_row[t + 1] + 1 - r0a + IRP_ALIGN - 1) & ~(IRP_ALIGN - 1);
                   irp_bytes = (uint32_t)n * (uint32_t)sizeof(OffT);
             }
-            mbar_expect_tx(&full[stage], (uint32_t)(cnt * 12) + irp_bytes);
+            long long idx_off = k0 * 4, idx_bytes = cnt * 4;
+            const unsigned char *idx_src = reinterpret_cast<const unsigned char *>(ja);
+            if (CODES) {
+                  idx_off = code_off[t];
+                  idx_bytes = code_off[t + 1] - idx_off;
+                  idx_src = codes;
+            }
+            mbar_expect_tx(&full[stage], (uint32_t)(cnt * 8 + idx_bytes) + irp_bytes);
             if (cnt > 0) {
                   bulk_g2s(s_as + (size_t)stage * CAP, as + k0, (uint32_t)(cnt * 8), &full[stage],
                            pol_s);
-                  bulk_g2s(s_ja + (size_t)stage * CAP, ja + k0, (uint32_t)(cnt * 4), &full[stage],
-                           pol_s);
+                  bulk_g2s(s_idx + (size_t)stage * Cfg::kIdxBytes, idx_src + idx_off,
+                           (uint32_t)idx_bytes, &full[stage], pol_s);
             }
             if (SPLIT)
                   bulk_g2s(s_irp + (size_t)stage * Cfg::kIrpSlots, irp + r0a, irp_bytes,
@@ -513,15 +550,20 @@ __global__ void __launch_bounds__(THREADS + (WS ? 32 : 0))
                   if (staged) {
                         stream_tile_products<THREADS, PASSES, CAP, EPI, OffT>(
                             s_irp + (size_t)stage * Cfg::kIrpSlots, s_as + (size_t)stage * CAP,
-                            s_ja + (size_t)stage * CAP, r0, r1, r0 & ~(IRP_ALIGN - 1), kbase, cnt,
+                            reinterpret_cast<const int *>(s_idx + (size_t)stage * Cfg::kIdxBytes),
+                            r0, r1, r0 & ~(IRP_ALIGN - 1), kbase, cnt,
                             tid, x, y, pol_x, epi, dot_acc, s_queue, s_queue_n + (n_split & 1),
                             s_queue_n + ((n_split + 1) & 1));
                         ++n_split;
                   }
             } else if (staged) {
-                  stream_tile_rows<LPR, RPP, PASSES, EPI, OffT>(
-                      irp, s_as + (size_t)stage * CAP, s_ja + (size_t)stage * CAP, r0, r1, kbase,
-                      gi, sub, ks, ke, x, y, pol_x, epi, dot_acc);
+                  const unsigned char *t_idx = s_idx + (size_t)stage * Cfg::kIdxBytes;
+                  // the dictionary follows the codes of the tile's staged entries
+                  const long long cnt = ((tile_k[t + 1] + 3) & ~3ll) - kbase;
+                  stream_tile_rows<LPR, RPP, PASSES, EPI, CODES, OffT>(
+                      irp, s_as + (size_t)stage * CAP, reinterpret_cast<const int *>(t_idx), t_idx,
+                      reinterpret_cast<const int *>(t_idx + round16(cnt)), r0, r1, kbase, gi, sub,
+                      ks, ke, x, y, pol_x, epi, dot_acc);
             }
             if (WS) {
                   __syncwarp();
@@ -537,6 +579,106 @@ __global__ void __launch_bounds__(THREADS + (WS ? 32 : 0))
             }
       }
       epi_finish_warp<EPI>(epi, dot_acc, (long long)blockIdx.x * CWARPS + (tid >> 5));
+}
+
+// Code blocks of the staged tiles (layout above), one CTA of 256 threads per tile.  The tile's
+// distinct offsets d = ja[k] - row go into a shared-memory hash set; a code is the rank of d among
+// them, so the blocks depend on the matrix only, not on the order the set was filled in.
+//   codes == nullptr  count pass: n_dict[t] = distinct offsets (kCodeDict + 1: too many) and
+//                     bytes[t] = size of the block (0 for a tile holding one row beyond `cap`)
+//   otherwise         fill pass: write block t at codes + code_off[t], every byte of it (entries
+//                     staged with the tile that belong to its neighbours, and padding: code 0)
+constexpr int kCodeHash = 1024; // hash slots: > 2 * kCodeDict
+template <typename OffT>
+__global__ void __launch_bounds__(256)
+    stream_codes_kernel(const OffT *__restrict__ irp, const int *__restrict__ ja,
+                        const int *__restrict__ tile_row, const long long *__restrict__ tile_k,
+                        int cap, int *__restrict__ n_dict, long long *__restrict__ bytes,
+                        const long long *__restrict__ code_off, unsigned char *__restrict__ codes) {
+      constexpr int kEmpty = -0x7fffffff - 1; // no offset: col >= 0 and row < 2^31 give d > -2^31
+      __shared__ int s_key[kCodeHash];
+      __shared__ unsigned char s_rank[kCodeHash];
+      __shared__ short s_slot[kCodeDict]; // occupied slots, in claim order
+      __shared__ int s_n, s_over;
+      const int t = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+      const long long k0 = tile_k[t] & ~3ll, k1 = (tile_k[t + 1] + 3) & ~3ll;
+      if (k1 - k0 > cap) { // one long row: the long-row kernels take it, no block
+            if (!codes && tid == 0)
+                  n_dict[t] = 0, bytes[t] = 0;
+            return;
+      }
+      for (int i = tid; i < kCodeHash; i += 256)
+            s_key[i] = kEmpty;
+      if (tid == 0)
+            s_n = 0, s_over = 0;
+      __syncthreads();
+      auto hash = [](int d) { return (int)(((unsigned)d * 2654435761u) >> 22); }; // 10 bits
+      const int r0 = tile_row[t], r1 = tile_row[t + 1];
+      for (int row = r0 + warp; row < r1; row += 8) {
+            const long long e = (long long)irp[row + 1];
+            for (long long k = (long long)irp[row] + lane; k < e; k += 32) {
+                  // past kCodeDict offsets the answer is known: stop before the table fills (at
+                  // most one more claim per thread follows, 257 + 256 < kCodeHash)
+                  if (*(volatile int *)&s_n > kCodeDict)
+                        break;
+                  const int d = ja[k] - row;
+                  int h = hash(d), i = 0;
+                  for (; i < kCodeHash; ++i, h = (h + 1) & (kCodeHash - 1)) {
+                        int v = *(volatile int *)&s_key[h];
+                        if (v == kEmpty) {
+                              v = atomicCAS(&s_key[h], kEmpty, d);
+                              if (v == kEmpty) {
+                                    const int n = atomicAdd(&s_n, 1);
+                                    if (n < kCodeDict)
+                                          s_slot[n] = (short)h;
+                                    break;
+                              }
+                        }
+                        if (v == d)
+                              break;
+                  }
+                  if (i == kCodeHash)
+                        s_over = 1; // the table is full: far more than kCodeDict offsets
+            }
+      }
+      __syncthreads();
+      const int n = s_over ? kCodeDict + 1 : min(s_n, kCodeDict + 1);
+      const long long code_bytes = round16(k1 - k0);
+      if (!codes) {
+            if (tid == 0)
+                  n_dict[t] = n, bytes[t] = code_bytes + round16(4ll * n);
+            return;
+      }
+      if (n > kCodeDict)
+            return; // the plan is not coded: the host never asks for this
+      unsigned char *blk = codes + code_off[t];
+      int *dict = reinterpret_cast<int *>(blk + code_bytes);
+      for (int i = tid; i < n; i += 256) {
+            const int v = s_key[s_slot[i]];
+            int r = 0;
+            for (int j = 0; j < n; ++j)
+                  r += s_key[s_slot[j]] < v;
+            s_rank[s_slot[i]] = (unsigned char)r;
+            dict[r] = v;
+      }
+      for (int i = n + tid; i < (int)(round16(4ll * n) / 4); i += 256)
+            dict[i] = 0;
+      // staged positions outside the tile's own entries
+      const int lead = (int)(tile_k[t] - k0), tail = (int)(tile_k[t + 1] - k0);
+      for (int p = tid; p < (int)code_bytes; p += 256)
+            if (p < lead || p >= tail)
+                  blk[p] = 0;
+      __syncthreads();
+      for (int row = r0 + warp; row < r1; row += 8) {
+            const long long e = (long long)irp[row + 1];
+            for (long long k = (long long)irp[row] + lane; k < e; k += 32) {
+                  const int d = ja[k] - row;
+                  int h = hash(d);
+                  while (s_key[h] != d)
+                        h = (h + 1) & (kCodeHash - 1);
+                  blk[k - k0] = s_rank[h];
+            }
+      }
 }
 
 // ------------------------------------------------------------------------

@@ -33,6 +33,7 @@ extern Counters g_counters;
 struct Knobs {
       int csr_stream_cfg = -1; // -1: pick from warps_per_block and the row-length profile
       int csr_pipe = -1;       // short regular CSR rows through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit
+      int csr_codes = 1;       // row-tile stream plans stream column codes where they apply; 0: int32 columns
       int hll_pipe = -1;       // narrow hacks through per-warp bulk-copy rings: -1 auto, 0 off, 1 whenever they fit
       int hll_stream_cfg = -1;
       int force_wide = 0;      // use 64-bit row offsets even when NZ < 2^31 (tests)
@@ -108,6 +109,13 @@ struct StreamPlan {
       RowList long_lists[kNumKinds]; // rows that do not fit a stage, by kind (5..7)
       SplitPlan split;
       bool built = false;
+      // column codes of the row-tile configurations (csr_kernels.cuh, stream_codes_kernel):
+      // tile t's block is d_codes[d_code_off[t], d_code_off[t+1])
+      int codes_state = 0; // 0 not tried, 1 built, -1 not applicable (a tile has too many offsets)
+      long long *d_code_off = nullptr;
+      unsigned char *d_codes = nullptr;
+      long long code_bytes = 0;
+      int max_dict = 0; // largest dictionary of a tile
 };
 
 struct Segment {

@@ -10,6 +10,7 @@
 
 #include <cub/cub.cuh>
 #include <memory>
+#include <type_traits>
 #include <new>
 
 #include "coo_kernels.cuh"
@@ -160,6 +161,8 @@ void free_segment(Segment &sg) {
             free_list(l);
       free_split(sg.split);
       for (auto &kv : sg.stream) {
+            cudaFree(kv.second.d_code_off);
+            cudaFree(kv.second.d_codes);
             cudaFree(kv.second.d_tile_row);
             cudaFree(kv.second.d_tile_k);
             for (auto &l : kv.second.long_lists)
@@ -282,6 +285,74 @@ static int build_stream(spmv_b200_csr *h, Segment &sg, int max_rows, int cap, St
       rc = rc ? rc : build_split(h, longs[kNumKinds - 1], sp.split);
       sp.built = rc == 0;
       return rc;
+}
+
+// Column codes of a row-tile plan (stream_codes_kernel), all or nothing: codes_state = 1 when
+// every staged tile has at most kCodeDict distinct column offsets, else -1 and the plan keeps
+// its int32 columns.  The codes only save bytes, so when device memory for them or for the build
+// runs short the plan also keeps its int32 columns (-1, no error).  Every buffer stays in the
+// temporaries guard until the build has succeeded, so no way out leaks one.  Synchronous on the
+// legacy stream, so never inside a graph capture (plans are built on a handle's first launches).
+template <typename OffT>
+static int build_codes(spmv_b200_csr *h, int cap, StreamPlan &sp) {
+      sp.codes_state = -1; // until the blocks exist
+      const int T = sp.n_tiles;
+      if (T <= 0)
+            return 0;
+      DeviceTemps tmp;
+      // quiet allocation: running short is not an error here
+      auto grab = [&](auto **out, size_t n_bytes) {
+            void *p = nullptr;
+            if (cudaMalloc(&p, std::max<size_t>(n_bytes, 1)) != cudaSuccess) {
+                  cudaGetLastError(); // clear the allocation error
+                  return false;
+            }
+            tmp.ptrs.push_back(p);
+            *out = static_cast<std::remove_pointer_t<decltype(out)>>(p);
+            return true;
+      };
+      int *d_nd = nullptr, *d_max = nullptr;
+      long long *d_bytes = nullptr, *d_code_off = nullptr;
+      unsigned char *d_codes = nullptr;
+      void *d_scratch = nullptr;
+      size_t scan_b = 0, max_b = 0;
+      B200_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_b, d_bytes, d_code_off, T + 1));
+      B200_CUDA(cub::DeviceReduce::Max(nullptr, max_b, d_nd, d_max, T));
+      if (!grab(&d_nd, (size_t)T * sizeof(int)) || !grab(&d_max, sizeof(int)) ||
+          !grab(&d_bytes, (size_t)(T + 1) * sizeof(long long)) ||
+          !grab(&d_scratch, std::max(scan_b, max_b)) ||
+          !grab(&d_code_off, (size_t)(T + 1) * sizeof(long long)))
+            return 0;
+      const OffT *irp = static_cast<const OffT *>(h->d_irp);
+      int max_nd = 0;
+      long long total = 0;
+      cudaError_t e = cudaMemset(d_bytes + T, 0, sizeof(long long));
+      if (e == cudaSuccess) {
+            stream_codes_kernel<OffT><<<T, 256>>>(irp, h->d_ja, sp.d_tile_row, sp.d_tile_k, cap,
+                                                   d_nd, d_bytes, nullptr, nullptr);
+            e = cub::DeviceScan::ExclusiveSum(d_scratch, scan_b, d_bytes, d_code_off, T + 1);
+      }
+      if (e == cudaSuccess)
+            e = cub::DeviceReduce::Max(d_scratch, max_b, d_nd, d_max, T);
+      if (e == cudaSuccess)
+            e = cudaMemcpy(&max_nd, d_max, sizeof(int), cudaMemcpyDeviceToHost);
+      if (e == cudaSuccess)
+            e = cudaMemcpy(&total, d_code_off + T, sizeof(long long), cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess)
+            return fail(-EIO, "column codes: count pass failed: %s", cudaGetErrorString(e));
+      if (max_nd > kCodeDict || !grab(&d_codes, (size_t)total))
+            return 0;
+      stream_codes_kernel<OffT><<<T, 256>>>(irp, h->d_ja, sp.d_tile_row, sp.d_tile_k, cap, d_nd,
+                                             d_bytes, d_code_off, d_codes);
+      e = cudaStreamSynchronize(nullptr);
+      if (e == cudaSuccess)
+            e = cudaGetLastError();
+      if (e != cudaSuccess)
+            return fail(-EIO, "column codes: fill pass failed: %s", cudaGetErrorString(e));
+      tmp.ptrs.pop_back(), tmp.ptrs.pop_back(); // d_codes and d_code_off belong to the plan now
+      sp.d_code_off = d_code_off, sp.d_codes = d_codes;
+      sp.code_bytes = total, sp.max_dict = max_nd, sp.codes_state = 1;
+      return 0;
 }
 
 static int finish_create(spmv_b200_csr *h, const long long *cuts, int n_cuts) {
@@ -421,9 +492,10 @@ void run_adaptive(const CsrArgs &a, const Segment &sg) {
 
 struct StreamShape {
       int id, threads, lpr, stages, cap, passes;
+      bool split;
 };
 constexpr StreamShape kStreamShapes[] = {
-#define X(id, t, l, s, c, p, sp) {id, t, l, s, c, p},
+#define X(id, t, l, s, c, p, sp) {id, t, l, s, c, p, sp},
     STREAM_CONFIGS(X)
 #undef X
 };
@@ -447,7 +519,9 @@ int stream_occupancy(Kern kern, int threads, size_t smem, int device, int *occ_c
       return 0;
 }
 
-// One launch of the staged kernel over the tiles of `sp`.  *grid_out = CTAs launched.
+// One launch of the staged kernel over the tiles of `sp`, streaming column codes when the plan
+// has them (row-tile configurations only) and the csr_codes knob is on.  *grid_out = CTAs
+// launched.
 template <typename OffT>
 int launch_stream_cfg(int cfg, const CsrArgs &a, const StreamPlan &sp, int *grid_out) {
       if (grid_out)
@@ -455,11 +529,12 @@ int launch_stream_cfg(int cfg, const CsrArgs &a, const StreamPlan &sp, int *grid
       if (sp.n_tiles <= 0)
             return 0;
       const OffT *irp = static_cast<const OffT *>(a.h->d_irp);
+      const bool coded = sp.codes_state == 1 && g_knobs.csr_codes != 0;
       switch (cfg) {
-#define LAUNCH_ONE(E, T, L, S, C, P, SP)                                                           \
+#define LAUNCH_ONE(E, T, L, S, C, P, SP, CODES)                                                    \
       {                                                                                            \
-            auto kern = csr_stream_kernel<T, L, S, C, P, true, SP, E, OffT>;                       \
-            using Cfg = StreamCfg<T, L, S, C, P, true, SP>;                                        \
+            auto kern = csr_stream_kernel<T, L, S, C, P, true, SP, E, CODES, OffT>;                \
+            using Cfg = StreamCfg<T, L, S, C, P, true, SP, CODES>;                                 \
             constexpr size_t smem = Cfg::template smem<OffT>();                                    \
             static int occ_by_dev[kMaxDevices] = {0}; /* the attribute is per device */            \
             int rc = stream_occupancy(kern, Cfg::kThreads, smem, a.h->device, occ_by_dev);         \
@@ -468,22 +543,30 @@ int launch_stream_cfg(int cfg, const CsrArgs &a, const StreamPlan &sp, int *grid
             const int grid =                                                                       \
                 std::min(sp.n_tiles, occ_by_dev[a.h->device % kMaxDevices] * g_sm_count);          \
             kern<<<grid, Cfg::kThreads, smem, a.st>>>(irp, a.h->d_ja, a.h->d_as, sp.d_tile_row,    \
-                                                      sp.d_tile_k, 0, sp.n_tiles, a.x, a.y,        \
-                                                      a.epi);                                      \
+                                                      sp.d_tile_k, sp.d_code_off, sp.d_codes, 0,   \
+                                                      sp.n_tiles, a.x, a.y, a.epi);                \
             if (grid_out)                                                                          \
                   *grid_out = grid;                                                                \
+      }
+#define LAUNCH_CODED(E, T, L, S, C, P, SP)                                                         \
+      {                                                                                            \
+            if (coded && !SP) /* entry-split plans have no codes */                                \
+                  LAUNCH_ONE(E, T, L, S, C, P, SP, !SP)                                            \
+            else                                                                                   \
+                  LAUNCH_ONE(E, T, L, S, C, P, SP, false)                                          \
       }
 #define X(id, T, L, S, C, P, SP)                                                                   \
       case id:                                                                                     \
             if (a.epi_mode == EPI_PUSH)                                                            \
-                  LAUNCH_ONE(EPI_PUSH, T, L, S, C, P, SP)                                          \
+                  LAUNCH_CODED(EPI_PUSH, T, L, S, C, P, SP)                                        \
             else if (a.epi_mode == EPI_FUSED)                                                      \
-                  LAUNCH_ONE(EPI_FUSED, T, L, S, C, P, SP)                                         \
+                  LAUNCH_CODED(EPI_FUSED, T, L, S, C, P, SP)                                       \
             else                                                                                   \
-                  LAUNCH_ONE(EPI_PLAIN, T, L, S, C, P, SP)                                         \
+                  LAUNCH_CODED(EPI_PLAIN, T, L, S, C, P, SP)                                       \
             break;
             STREAM_CONFIGS(X)
 #undef X
+#undef LAUNCH_CODED
 #undef LAUNCH_ONE
       default:
             return fail(-EINVAL, "unknown stream configuration %d", cfg);
@@ -953,9 +1036,14 @@ static int run_kernel(spmv_b200_csr *h, int kernel, int wpb, Segment &sg, const 
                                                   : 0.0;
             const int cfg = stream_cfg_for(wpb, mean_len, sg.regular);
             StreamPlan &sp = sg.stream[cfg];
+            const StreamShape &s = *stream_shape(cfg);
             if (!sp.built) {
-                  const StreamShape &s = *stream_shape(cfg);
                   int rc = build_stream(h, sg, s.threads / s.lpr * s.passes, s.cap, sp);
+                  if (rc)
+                        return rc;
+            }
+            if (!s.split && g_knobs.csr_codes != 0 && sp.codes_state == 0) {
+                  int rc = build_codes<OffT>(h, s.cap, sp);
                   if (rc)
                         return rc;
             }
@@ -1940,6 +2028,28 @@ extern "C" int spmv_b200_csr_plan_info(const spmv_b200_csr *h, int64_t *out, int
       return 0;
 }
 
+extern "C" int spmv_b200_csr_codes_info(const spmv_b200_csr *h, int64_t *out, int n_out) {
+      if (!h || !out)
+            return fail(-EINVAL, "null argument");
+      int64_t v[4] = {0, 0, 0, 0}; // state, tiles, largest dictionary, block bytes
+      for (const auto &sg : h->segs)
+            for (const auto &kv : sg.stream) {
+                  const StreamPlan &sp = kv.second;
+                  if (sp.codes_state == -1)
+                        v[0] = -1;
+                  else if (sp.codes_state == 1 && v[0] == 0)
+                        v[0] = 1;
+                  if (sp.codes_state == 1) {
+                        v[1] += sp.n_tiles;
+                        v[2] = std::max<int64_t>(v[2], sp.max_dict);
+                        v[3] += sp.code_bytes;
+                  }
+            }
+      for (int i = 0; i < n_out && i < 4; ++i)
+            out[i] = v[i];
+      return 0;
+}
+
 extern "C" int spmv_b200_csr_sell_info(spmv_b200_csr *h, int build, int64_t *out, int n_out) {
       if (!h || !out)
             return fail(-EINVAL, "null argument");
@@ -2805,6 +2915,7 @@ extern "C" int spmv_b200_set_knob(const char *key, int value) {
       } table[] = {{"csr_stream_cfg", &g_knobs.csr_stream_cfg},
                    {"hll_pipe", &g_knobs.hll_pipe},
                    {"csr_pipe", &g_knobs.csr_pipe},
+                   {"csr_codes", &g_knobs.csr_codes},
                    {"hll_stream_cfg", &g_knobs.hll_stream_cfg},
                    {"force_wide", &g_knobs.force_wide},
                    {"pipeline", &g_knobs.pipeline},
